@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MPN hot path (BASELINE.json metric: MPN inference directed edges/sec; p50 latency per S02-shape graph).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-extras] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one synthetic graph that is already resident in HBM, through the public call
 (`MOTMPNet.forward(data)` with `data.edge_attr = None`): graph tables from the int64 `edge_index` (K0), edge features (K1, with
@@ -683,6 +683,25 @@ def big_graph_step(m, dev, world, rank, sharded_cls, n_nodes=32768, L=4, steps=3
 
 
 # ------------------------------------------------------------------------------------------------- GPU arm
+DUMP_EDGES = 1 << 20        # per-edge outputs sampled for --dump-outputs: ~33 MB in all instead of ~470 MB at E = 14.7 M
+
+
+def dump_outputs(path, res):
+    """--dump-outputs: what one step handed its caller, as DIR/<name>.npy (float32; edge ids float64).  Per-edge arrays are taken
+    at the same DUMP_EDGES edges on every run (a seeded sample, sorted, stored as edge_ids.npy) so that two builds compare edge
+    for edge; h is stored whole."""
+    import numpy as np
+    logits = res["classified_edges"]
+    E = logits[0].shape[0]
+    ids = torch.randperm(E, generator=torch.Generator().manual_seed(0))[:DUMP_EDGES].sort().values
+    idx = ids.to(logits[0].device)
+    arrays = {"edge_ids": ids.double(), "classified_edges": torch.stack([l[idx] for l in logits]), "h": res["h"],
+              "pred": res["pred"][idx].float(), "prob1": res["prob1"][idx], "edge_attr": res["edge_attr"][idx]}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy())
+
+
 def step_timeline(lib, step_fn, flush, barrier, dev, world, reps=5):
     """Where inside ONE step the time goes (mpn_profile_timeline: CUDA events at the phase boundaries of the step's forward call;
     each entry = ms since the forward began, median over ``reps`` steps, max over ranks).  Measured after the timed region: the
@@ -741,17 +760,19 @@ def run_ours(args):
     cam_host = (torch.arange(n_nodes) * CAMS // n_nodes).numpy()
 
     def step(x, ei):
+        """One timed step -> the arrays its caller receives (logits per classified step, node embeddings, decisions, edge features)."""
         if world == 1:
             g = m.TrackletGraph(ei, n_nodes, validate="deferred")              # K0 (the edge-list check is read at the end)
             batch.x, batch.edge_index, batch.mpn_graph, batch.edge_attr = x, ei, g, None
-            net(batch)                                                         # K1 + K1b..K4 (+ fused decisions) in one call
+            out, h = net(batch)                                                # K1 + K1b..K4 (+ fused decisions) in one call
             g.validate()                                                       # raises on an unsorted / out-of-range edge list
-            return net.last_pred
+            return {"classified_edges": out["classified_edges"], "h": h, "pred": net.last_pred, "prob1": net.last_prob1,
+                    "edge_attr": batch.edge_attr}
         n0, n1 = blocks[rank]
         g = m.TrackletGraph(ei, n_nodes, row_offset=n0, n_rows=n1 - n0, validate="deferred")
         out, h, pred, prob1 = sharded.forward(x, ei, None, blocks, fuse_decisions=True, graph=g)     # edge features inside the call
         g.validate()
-        return pred
+        return {"classified_edges": out["classified_edges"], "h": h, "pred": pred, "prob1": prob1, "edge_attr": sharded.last_edge_attr}
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
 
@@ -766,7 +787,7 @@ def run_ours(args):
         parity = parity_gate(m, net, x, ei, dev)
     else:
         # the sharded decisions against the unsharded forward of the same graph run on every rank's own GPU
-        pred_sh = step(x, ei).clone()
+        pred_sh = step(x, ei)["pred"].clone()
         bfull = Batch()
         bfull.x, bfull.num_nodes, bfull.edge_attr = x, n_nodes, None
         bfull.mpn_graph = gfull = m.TrackletGraph.from_cameras(cam_host, dev)
@@ -794,11 +815,12 @@ def run_ours(args):
     launches0 = lib.mpn_kernel_launches()
     total_ms = 0.0
     for i in range(args.steps):
+        last = None                                                            # the previous step's outputs are not kept alive
         flush.fill_(i & 0xFF)                                                  # L2 flush between timed iterations
         barrier()
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        step(x, ei)
+        last = step(x, ei)
         b.record()
         barrier()
         ms = torch.tensor([a.elapsed_time(b)], dtype=torch.float64, device=dev)
@@ -807,6 +829,9 @@ def run_ours(args):
         total_ms += float(ms.item())
     launches = lib.mpn_kernel_launches() - launches0
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last = None
     ms_per_step = total_ms / args.steps
     value = E_total / (ms_per_step * 1e-3)
     timeline = step_timeline(lib, lambda: step(x, ei), flush, barrier, dev, world)
@@ -1048,7 +1073,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip the other BASELINE configs (extra / c5_strong blocks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (rank 0; "
+                                                           "per-edge arrays at a fixed sample of edges)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the timed GPU path; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

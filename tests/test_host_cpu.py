@@ -281,3 +281,29 @@ def test_unpack_decisions_and_block_cover_host_logic():
     assert not sh._blocks_cover([(0, 5), (5, 9)], 2, 10)          # does not reach the last node
     assert not sh._blocks_cover([(0, 5), (5, 5), (5, 9)], 3, 9)   # empty block
     assert not sh._blocks_cover([(0, 9)], 2, 9)                   # one block per rank
+
+
+def test_bench_dump_outputs_sample_and_format(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 / float64 .npy files; per-edge arrays at the same seeded, sorted edge sample every run."""
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, "DUMP_EDGES", 64)
+    gen = torch.Generator().manual_seed(2)
+    E = 1000
+    res = {"classified_edges": [torch.randn(E, 2, generator=gen) for _ in range(2)], "h": torch.randn(30, 32, generator=gen),
+           "pred": (torch.rand(E, generator=gen) < 0.5).to(torch.uint8), "prob1": torch.rand(E, generator=gen),
+           "edge_attr": torch.randn(E, 2, generator=gen)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), res)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["classified_edges.npy", "edge_attr.npy", "edge_ids.npy", "h.npy", "pred.npy", "prob1.npy"]
+    got = {n[:-4]: np.load(tmp_path / "a" / n) for n in names}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    ids = got["edge_ids"].astype(np.int64)
+    assert ids.size == 64 and np.all(np.diff(ids) > 0) and ids[-1] < E
+    assert np.array_equal(got["classified_edges"], torch.stack(res["classified_edges"]).numpy()[:, ids])
+    assert np.array_equal(got["pred"], res["pred"].numpy()[ids].astype(np.float32))
+    assert np.array_equal(got["prob1"], res["prob1"].numpy()[ids]) and np.array_equal(got["h"], res["h"].numpy())
+    assert np.array_equal(got["edge_attr"], res["edge_attr"].numpy()[ids])
+    for n in names:
+        assert (tmp_path / "a" / n).read_bytes() == (tmp_path / "b" / n).read_bytes()
