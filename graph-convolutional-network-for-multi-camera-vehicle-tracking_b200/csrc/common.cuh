@@ -127,6 +127,21 @@ __device__ __forceinline__ void block_sum_doubles(double (&v)[K], double* smem /
   __syncthreads();
 }
 
+// Block-wide sum of K columns held one per lane (lane k < K of every warp holds column k); result in out[0..K-1].
+// Deterministic: fixed order over warps.
+template <int K, int THREADS>
+__device__ __forceinline__ void block_sum_lane_columns(double v, double* smem /* [THREADS/32][K] */, double* out) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (lane < K) smem[warp * K + lane] = v;
+  __syncthreads();
+  if (threadIdx.x < K) {
+    double s = 0.0;
+    for (int w = 0; w < THREADS / 32; ++w) s += smem[w * K + threadIdx.x];
+    out[threadIdx.x] = s;
+  }
+  __syncthreads();
+}
+
 // streaming (read-once) loads: bypass L1 allocation
 __device__ __forceinline__ float4 ldg_stream4(const float4* p) {
   float4 r;

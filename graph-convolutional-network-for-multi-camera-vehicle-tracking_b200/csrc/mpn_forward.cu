@@ -42,6 +42,12 @@ constexpr int SUMS = MPN_SUMS_DOUBLES;     // 96 doubles per partial row
 constexpr int SWEEP_THREADS = 256;
 constexpr int SWEEP_BLOCKS_PER_SM = 4;
 constexpr int SWEEP_GRID = kNumSMs * SWEEP_BLOCKS_PER_SM;
+// The node-moment sweep over stored y (SB) is capped at 80 registers (__launch_bounds__ minimum of 3 blocks; no spills), so 3
+// blocks = 24 warps fit on an SM and its grid is exactly one resident wave: a second, partial wave would start late and finish
+// late.  The sweep is bound by the bytes each SM has in flight; 24 warps instead of 16 at the same loads per lane is the gain.
+// (The variant that recomputes y spills at 80 registers and keeps 2 blocks per SM and SWEEP_GRID.)
+constexpr int SWEEP_RESIDENT_BLOCKS = 3;
+constexpr int SWEEP_RESIDENT_GRID = kNumSMs * SWEEP_RESIDENT_BLOCKS;
 constexpr float BN_EPS = 1e-5f;
 
 struct EdgeConsts {           // staged in shared memory by every sweep
@@ -114,24 +120,25 @@ __device__ __forceinline__ TaskRange task_range(const mpn_graph& g, int t) {
 
 // Task ranges two strides ahead: task_range() is a chain of dependent loads (task_row -> rowptr/taskptr), ~2 L2 round trips that
 // a warp would otherwise pay at the start of every task.  Stage A fetches the row of task t + 2*stride, stage B the range of task
-// t + stride from the row fetched one iteration earlier; the current task never waits.
+// t + stride from the row fetched one iteration earlier; the current task never waits.  stride < 0 walks the tasks backwards.
+__device__ __forceinline__ bool task_in(int t, int n_tasks) { return (unsigned)t < (unsigned)n_tasks; }
 struct TaskPrefetch {
   TaskRange cur, nxt;
   int row_n;                                         // row of task t + stride (stage A result of the previous iteration)
   __device__ __forceinline__ void start(const mpn_graph& g, int t, int stride, int n_tasks) {
-    if (t < n_tasks) cur = task_range(g, t);
-    row_n = (t + stride < n_tasks) ? g.task_row[t + stride] : 0;
+    if (task_in(t, n_tasks)) cur = task_range(g, t);
+    row_n = task_in(t + stride, n_tasks) ? g.task_row[t + stride] : 0;
   }
   // call at the top of the iteration for task t; afterwards `cur` is valid; call rotate() at the bottom
   __device__ __forceinline__ int issue(const mpn_graph& g, int t, int stride, int n_tasks) {
-    if (t + stride < n_tasks) {
+    if (task_in(t + stride, n_tasks)) {
       const int tn = t + stride;
       nxt.row = row_n;
       const int rb = g.rowptr[row_n];
       nxt.beg = rb + (tn - g.taskptr[row_n]) * g.chunk;
       nxt.end = min(nxt.beg + g.chunk, g.rowptr[row_n + 1]);
     }
-    return (t + 2 * stride < n_tasks) ? g.task_row[t + 2 * stride] : 0;
+    return task_in(t + 2 * stride, n_tasks) ? g.task_row[t + 2 * stride] : 0;
   }
   __device__ __forceinline__ void rotate(int row_nn) { cur = nxt; row_n = row_nn; }
 };
@@ -147,6 +154,7 @@ struct FinArgs {
   int stage;
   const double* partials;
   int n_partials;
+  int row_stride;             // rows from one partial row read by the fold to the next (1; FOLD_GROUP for the group rows)
   const double* partials2;
   int n_partials2;
   double* sums;
@@ -164,6 +172,46 @@ struct FinArgs {
                               // step-1 weights), 2 on and y stored (switch to the split weights after the first edge update)
 };
 
+__device__ __forceinline__ int fin_ncols(int stage) { return (stage == MPN_STAGE_NODE) ? 74 : 8; }   // live partial columns
+
+// Fixed-order fold of n_rows partial rows (row r at rows + r * row_stride * SUMS); thread k < ncols returns column k's total, the
+// others 0.  Every thread of the block calls it.  It runs in the serial tail of a sweep: a thread owns a PAIR of adjacent live
+// columns (one 16-byte L2 load per partial row) and every `groups`-th row, four loads in flight; the row groups are then added
+// through shared memory in group order.  Fixed pattern => bit-reproducible.
+__device__ __forceinline__ double fold_rows(const double* rows, int n_rows, int row_stride, int ncols) {
+  __shared__ double red[2048];
+  const int k = threadIdx.x;
+  const size_t rs = (size_t)row_stride * SUMS;
+  const int pairs = ncols >> 1;
+  int groups = (int)blockDim.x / pairs;
+  if (groups * ncols > 2048) groups = 2048 / ncols;
+  if (k < groups * pairs) {
+    const int cp = k % pairs, gi = k / pairs;
+    const double* base = rows + 2 * cp;
+    double2 a0 = make_double2(0.0, 0.0), a1 = a0, a2 = a0, a3 = a0;
+    int p = gi;
+    for (; p + 3 * groups < n_rows; p += 4 * groups) {
+      const double2 v0 = __ldcg(reinterpret_cast<const double2*>(base + (size_t)p * rs));
+      const double2 v1 = __ldcg(reinterpret_cast<const double2*>(base + (size_t)(p + groups) * rs));
+      const double2 v2 = __ldcg(reinterpret_cast<const double2*>(base + (size_t)(p + 2 * groups) * rs));
+      const double2 v3 = __ldcg(reinterpret_cast<const double2*>(base + (size_t)(p + 3 * groups) * rs));
+      a0.x += v0.x; a0.y += v0.y; a1.x += v1.x; a1.y += v1.y; a2.x += v2.x; a2.y += v2.y; a3.x += v3.x; a3.y += v3.y;
+    }
+    for (; p < n_rows; p += groups) {
+      const double2 v = __ldcg(reinterpret_cast<const double2*>(base + (size_t)p * rs));
+      a0.x += v.x; a0.y += v.y;
+    }
+    red[gi * ncols + 2 * cp] = (a0.x + a1.x) + (a2.x + a3.x);
+    red[gi * ncols + 2 * cp + 1] = (a0.y + a1.y) + (a2.y + a3.y);
+  }
+  __syncthreads();
+  double t = 0.0;
+  if (k < ncols)
+    for (int gi = 0; gi < groups; ++gi) t += red[gi * ncols + k];
+  __syncthreads();                                   // red is free again
+  return t;
+}
+
 __device__ __forceinline__ void finalize_body(const FinArgs& f, int do_reduce, int do_consts) {
   const int stage = f.stage;
   double* sums = f.sums;
@@ -171,39 +219,8 @@ __device__ __forceinline__ void finalize_body(const FinArgs& f, int do_reduce, i
   const float* small = f.small;
   const int k = threadIdx.x;
   if (do_reduce) {
-    // The reduction is the serial tail of the sweep's last block: it has to be short.  A thread owns a PAIR of adjacent live columns
-    // (one 16-byte L2 load per partial row) and every `groups`-th row, four loads in flight; the row groups are then added through
-    // shared memory in group order.  Fixed pattern => bit-reproducible.  Live columns: 8 (ENC / EDGE stages), 74 (NODE stage).
-    __shared__ double red[2048];
-    const int ncols = (stage == MPN_STAGE_NODE) ? 74 : 8;
-    const int pairs = ncols >> 1;
-    int groups = (int)blockDim.x / pairs;
-    if (groups * ncols > 2048) groups = 2048 / ncols;
-    const int n_rows = f.n_partials;
-    if (k < groups * pairs) {
-      const int cp = k % pairs, gi = k / pairs;
-      const double* base = f.partials + 2 * cp;
-      double2 a0 = make_double2(0.0, 0.0), a1 = a0, a2 = a0, a3 = a0;
-      int p = gi;
-      for (; p + 3 * groups < n_rows; p += 4 * groups) {
-        const double2 v0 = __ldcg(reinterpret_cast<const double2*>(base + (size_t)p * SUMS));
-        const double2 v1 = __ldcg(reinterpret_cast<const double2*>(base + (size_t)(p + groups) * SUMS));
-        const double2 v2 = __ldcg(reinterpret_cast<const double2*>(base + (size_t)(p + 2 * groups) * SUMS));
-        const double2 v3 = __ldcg(reinterpret_cast<const double2*>(base + (size_t)(p + 3 * groups) * SUMS));
-        a0.x += v0.x; a0.y += v0.y; a1.x += v1.x; a1.y += v1.y; a2.x += v2.x; a2.y += v2.y; a3.x += v3.x; a3.y += v3.y;
-      }
-      for (; p < n_rows; p += groups) {
-        const double2 v = __ldcg(reinterpret_cast<const double2*>(base + (size_t)p * SUMS));
-        a0.x += v.x; a0.y += v.y;
-      }
-      red[gi * ncols + 2 * cp] = (a0.x + a1.x) + (a2.x + a3.x);
-      red[gi * ncols + 2 * cp + 1] = (a0.y + a1.y) + (a2.y + a3.y);
-    }
-    __syncthreads();
+    double t = fold_rows(f.partials, f.n_partials, f.row_stride, fin_ncols(stage));
     if (k < SUMS) {
-      double t = 0.0;
-      if (k < ncols)
-        for (int gi = 0; gi < groups; ++gi) t += red[gi * ncols + k];
       if (stage == MPN_STAGE_ENC0 && f.fixed != nullptr && k < 5)
         t += (double)(long long)__ldcg(f.fixed + k) * (1.0 / 1099511627776.0);
       sums[k] = t;
@@ -344,18 +361,39 @@ __global__ void peer_wait_h_kernel(const PeerArgs P, unsigned long long seq) {
   if (blockIdx.x == 0 && threadIdx.x < P.world) wait_flag(P.flags[P.rank] + KPEERS + threadIdx.x, seq);     // own memory
 }
 
-// called by every block at the end of a sweep kernel, after its partial row has been written
+// Called by every block at the end of a sweep kernel, after its partial row has been written.  Two-level ticket: the last block of
+// each group of FOLD_GROUP consecutive blocks folds the group's rows into the group's first row, and the last of those folds the
+// group rows and the constants.  One block folding all 444-592 rows was a serial tail of ~18 us for the 74 live columns of the
+// node BatchNorm; two short folds take a few L2 round trips each.  Counters: [0] groups done, [1 + g] blocks of group g done.
+constexpr int FOLD_GROUP = 16;
+constexpr int FIN_COUNTERS = 1 + (SWEEP_GRID + FOLD_GROUP - 1) / FOLD_GROUP;
 __device__ __forceinline__ void finalize_in_last_block(const FinArgs& f) {
   if (f.counter == nullptr) return;
   __shared__ unsigned int s_ticket;
+  const int grp = blockIdx.x / FOLD_GROUP, n_groups = (gridDim.x + FOLD_GROUP - 1) / FOLD_GROUP;
+  const int grp_blocks = min(FOLD_GROUP, (int)gridDim.x - grp * FOLD_GROUP);
   __threadfence();                                   // publish this block's partials
+  __syncthreads();
+  if (threadIdx.x == 0) s_ticket = atomicAdd(f.counter + 1 + grp, 1u);
+  __syncthreads();
+  if (s_ticket != (unsigned)grp_blocks - 1) return;
+  __threadfence();
+  double* grp_row = const_cast<double*>(f.partials) + (size_t)grp * FOLD_GROUP * SUMS;
+  const int ncols = fin_ncols(f.stage);
+  const double t = fold_rows(grp_row, grp_blocks, 1, ncols);
+  if (threadIdx.x < ncols) grp_row[threadIdx.x] = t;
+  if (threadIdx.x == 0) f.counter[1 + grp] = 0u;     // ready for the next sweep
+  __threadfence();                                   // publish the group row
   __syncthreads();
   if (threadIdx.x == 0) s_ticket = atomicAdd(f.counter, 1u);
   __syncthreads();
-  if (s_ticket != gridDim.x - 1) return;
+  if (s_ticket != (unsigned)n_groups - 1) return;
   __threadfence();
-  if (f.peers != nullptr) finalize_peer_body(f, *f.peers, f.seq);
-  else finalize_body(f, 1, 1);
+  FinArgs g = f;
+  g.n_partials = n_groups;
+  g.row_stride = FOLD_GROUP;
+  if (g.peers != nullptr) finalize_peer_body(g, *g.peers, g.seq);
+  else finalize_body(g, 1, 1);
   if (threadIdx.x == 0) *f.counter = 0u;             // ready for the next sweep
 }
 
@@ -464,6 +502,8 @@ __device__ __forceinline__ void load_edges(EdgeLoad<U>& L, const mpn_graph& g, i
 //   SRC 0: e_in = encoder(edge_attr[e])            (step 1)
 //   SRC 1: e_in = relu(BN3_prev(ybuf[e]))          (step >= 2; ybuf updated in place)
 //   RE_E (reattach_initial_edges, steps >= 2): e_in = [e0 | e] with e0 = encoder(edge_attr[e]) recomputed: y += We0 . e0
+// A warp walks its tasks from the last to the first: the sweep before it (ENC1 over edge_attr, or the apply sweep of the previous
+// step) ends at the high edges, which are then still in L2; the node-moment sweep after it walks forwards for the same reason.
 template <int SRC, bool WRITE_Y, bool BATCHED, bool RE_E = false>
 __global__ void __launch_bounds__(SWEEP_THREADS, 2) edge_moments_kernel(const mpn_graph g, const float2* __restrict__ edge_attr,
                                                                      const float4* __restrict__ Ps, const float4* __restrict__ Pd,
@@ -481,10 +521,11 @@ __global__ void __launch_bounds__(SWEEP_THREADS, 2) edge_moments_kernel(const mp
   const int n_tasks = *g.n_tasks;
   double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   int cur_gid = -1;
+  const int t_last = gwarp + max(n_tasks - 1 - gwarp, 0) / nwarps * nwarps;
   TaskPrefetch tp;
-  tp.start(g, gwarp, nwarps, n_tasks);
-  for (int t = gwarp; t < n_tasks; t += nwarps) {
-    const int row_nn = tp.issue(g, t, nwarps, n_tasks);
+  tp.start(g, t_last, -nwarps, n_tasks);
+  for (int t = t_last; task_in(t, n_tasks); t -= nwarps) {
+    const int row_nn = tp.issue(g, t, -nwarps, n_tasks);
     const TaskRange tr = tp.cur;
     if (BATCHED) {
       const int gid = g.node_gid[tr.row];
@@ -554,9 +595,11 @@ __device__ __forceinline__ void eprime_of(const EdgeConsts& sc, const float4 ps,
   bn3_relu(sc, y, ep);
 }
 
-// SB: per-task S1 = sum e' (for the closed-form node-BN moments), global T2 = sum e' e'^T
+// SB: per-task S1 = sum e' (for the closed-form node-BN moments), global T2 = sum e' e'^T.
+// A warp walks its tasks from the first to the last: the edge update before it (SA) walks them backwards, so the y lines it wrote
+// last, still in L2, are the first ones read here.
 template <int YSRC, bool BATCHED>
-__global__ void __launch_bounds__(SWEEP_THREADS, 2) node_moments_sweep_kernel(const mpn_graph g, const float2* __restrict__ edge_attr,
+__global__ void __launch_bounds__(SWEEP_THREADS, YSRC == 1 ? SWEEP_RESIDENT_BLOCKS : 2) node_moments_sweep_kernel(const mpn_graph g, const float2* __restrict__ edge_attr,
                                                                            const float4* __restrict__ Ps, const float4* __restrict__ Pd,
                                                                            const float4* __restrict__ ybuf, const float* __restrict__ consts,
                                                                            float4* __restrict__ s1_task, double* __restrict__ partials,
@@ -573,7 +616,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS, 2) node_moments_sweep_kernel(co
   const int gwarp = (blockIdx.x * SWEEP_THREADS + threadIdx.x) >> 5;
   const int nwarps = (gridDim.x * SWEEP_THREADS) >> 5;
   const int n_tasks = *g.n_tasks;
-  double t2[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+  double t2 = 0.0;                                         // lane i < 10: running sum of T2 entry i over this warp's tasks
   // per-node part of the closed-form node-BN moments, taken per task (it is linear in the task's edge count and S1):
   //   m1[c] += n_t A[row,c] + w_c.S1_t ;  m2[c] += n_t A[row,c]^2 + 2 A[row,c] (w_c.S1_t)      (w_c = W_node[c, 32:36]; lane = c)
   double m1 = 0.0, m2 = 0.0;
@@ -619,13 +662,10 @@ __global__ void __launch_bounds__(SWEEP_THREADS, 2) node_moments_sweep_kernel(co
       m2 += (double)(a_row * fmaf(nt, a_row, 2.0f * qd));
     }
 #pragma unroll
-    for (int i = 0; i < 10; ++i) {
-      if (BATCHED) {
-        const double v = warp_sum((double)q[i]);
-        if (lane == 0) partials[(size_t)t * TASK_PART + i] = v;
-      } else {
-        t2[i] += (double)q[i];                              // <= chunk/32 fp32 terms per lane, then fp64
-      }
+    for (int i = 0; i < 10; ++i) {                          // <= chunk/32 fp32 terms per lane, folded across the warp in fp64
+      const double v = warp_sum((double)q[i]);
+      if (BATCHED) { if (lane == 0) partials[(size_t)t * TASK_PART + i] = v; }
+      else if (lane == i) t2 += v;
     }
     tp.rotate(row_nn);
   }
@@ -633,7 +673,7 @@ __global__ void __launch_bounds__(SWEEP_THREADS, 2) node_moments_sweep_kernel(co
     const int warp = threadIdx.x >> 5;
     red_m[warp][lane] = m1;
     red_m[warp][32 + lane] = m2;
-    block_sum_doubles<10, SWEEP_THREADS>(t2, red, partials + (size_t)blockIdx.x * SUMS + 64);   // (has the barriers)
+    block_sum_lane_columns<10, SWEEP_THREADS>(t2, red, partials + (size_t)blockIdx.x * SUMS + 64);   // (has the barriers)
     if (threadIdx.x < 64) {
       double sm = 0.0;
       for (int wv = 0; wv < SWEEP_THREADS / 32; ++wv) sm += red_m[wv][threadIdx.x];
@@ -1293,7 +1333,7 @@ __global__ void __launch_bounds__(128) graph_finalize_kernel(int stage, const mp
   __syncthreads();
   FinArgs f;
   f.stage = stage;
-  f.partials = nullptr; f.n_partials = 0; f.partials2 = nullptr; f.n_partials2 = 0;
+  f.partials = nullptr; f.n_partials = 0; f.row_stride = 1; f.partials2 = nullptr; f.n_partials2 = 0;
   f.sums = sums;
   f.consts = consts_all + (size_t)gi * FC_TOTAL;
   f.small = small;
@@ -1706,7 +1746,7 @@ static int plan_layout(mpn_fwd_plan& p, void* ws, size_t ws_bytes, size_t* need)
   p.sums = a.take<double>(G * SUMS);
   p.partials = a.take<double>((size_t)SWEEP_GRID * SUMS);      // partials | fin_counter | fix_sums are adjacent: one memset clears
   p.partials2 = nullptr;                                       // them (clear_moment_state); the per-node moment part lives in the
-  p.fin_counter = a.take<unsigned int>(1);                     // sweep's own partial rows
+  p.fin_counter = a.take<unsigned int>(FIN_COUNTERS);          // sweep's own partial rows
   p.fix_sums = a.take<unsigned long long>(8);
   p.peers_dev = a.take<PeerArgs>(1);
   p.n_total_dev = a.take<double>(1);
@@ -1788,6 +1828,7 @@ static FinArgs make_fin(const mpn_fwd_plan* p, int stage, bool fused) {
   f.stage = stage;
   f.partials = p->partials;
   f.n_partials = SWEEP_GRID;
+  f.row_stride = 1;
   f.partials2 = p->partials;             // the node-BN sweep writes its per-node part into the same partial rows
   f.n_partials2 = SWEEP_GRID;
   f.sums = p->sums;
@@ -1803,6 +1844,16 @@ static FinArgs make_fin(const mpn_fwd_plan* p, int stage, bool fused) {
   if (fused && p->seq_m_active) { f.peers = p->peers_dev; f.seq = ++const_cast<mpn_fwd_plan*>(p)->seq_m; }
   f.re_e = p->w.reattach_edges ? (stores_y(*p) ? 2 : 1) : 0;
   return f;
+}
+
+// FinArgs of a moment sweep launched on grid <= SWEEP_GRID blocks: the fold reads that many partial rows.  A separate reduce
+// (phase API) adds SWEEP_GRID rows, and the rows beyond this grid still hold the previous stage's partial sums: they are cleared.
+static int sweep_fin(const mpn_fwd_plan* p, int stage, bool fused, int grid, cudaStream_t st, FinArgs& f) {
+  f = make_fin(p, stage, fused);
+  f.n_partials = f.n_partials2 = grid;
+  if (!fused && grid < SWEEP_GRID)
+    MPN_CUDA_OK(cudaMemsetAsync(p->partials + (size_t)grid * SUMS, 0, sizeof(double) * (size_t)(SWEEP_GRID - grid) * SUMS, st));
+  return MPN_OK;
 }
 
 // 3xFP16 planes for encoder layer l: cached weight planes present, K a multiple of 8 (TMA row stride), not disabled
@@ -1954,7 +2005,7 @@ int mpn_plan_sweep(mpn_fwd_plan* p, int32_t step, int32_t stage, const float* ed
         }
         break;
       case MPN_STAGE_NODE:
-        if (stored) mpn::launch(node_moments_sweep_kernel<1, true>, SWEEP_GRID, SWEEP_THREADS, 0, st, g, ea, Ps4, Pd4, yb, p->consts, (float4*)p->s1_task, tp, p->A, p->w.small, make_fin(p, stage, false));
+        if (stored) mpn::launch(node_moments_sweep_kernel<1, true>, SWEEP_RESIDENT_GRID, SWEEP_THREADS, 0, st, g, ea, Ps4, Pd4, yb, p->consts, (float4*)p->s1_task, tp, p->A, p->w.small, make_fin(p, stage, false));
         else mpn::launch(node_moments_sweep_kernel<0, true>, SWEEP_GRID, SWEEP_THREADS, 0, st, g, ea, Ps4, Pd4, nullptr, p->consts, (float4*)p->s1_task, tp, p->A, p->w.small, make_fin(p, stage, false));
         break;
       case MPN_STAGE_APPLY: {
@@ -1990,10 +2041,8 @@ int mpn_plan_sweep(mpn_fwd_plan* p, int32_t step, int32_t stage, const float* ed
       if ((((uintptr_t)ea) & 15) == 0 && g.n_edges >= 2) {
         const long long n_pairs = g.n_edges >> 1;
         const int pgrid = (int)min((long long)kNumSMs * 2, (long long)div_up(n_pairs, SWEEP_THREADS));
-        FinArgs pf = make_fin(p, stage, fused);
-        pf.n_partials = pf.n_partials2 = pgrid;             // rows beyond this grid still hold the previous stage's partial sums:
-        if (!fused && pgrid < SWEEP_GRID)                   // a separate reduce (phase API) adds SWEEP_GRID rows -> clear them
-          MPN_CUDA_OK(cudaMemsetAsync(p->partials + (size_t)pgrid * SUMS, 0, sizeof(double) * (size_t)(SWEEP_GRID - pgrid) * SUMS, st));
+        FinArgs pf;
+        MPN_TRY(sweep_fin(p, stage, fused, pgrid, st, pf));
         mpn::launch(enc_moments1_packed_kernel, pgrid, SWEEP_THREADS, 0, st, (const float4*)ea, n_pairs, ea, g.n_edges, p->consts, p->w.small,
                     p->partials, pf);
       } else {
@@ -2010,10 +2059,13 @@ int mpn_plan_sweep(mpn_fwd_plan* p, int32_t step, int32_t stage, const float* ed
         else mpn::launch(edge_moments_kernel<1, true, false>, SWEEP_GRID, SWEEP_THREADS, 0, st, g, ea, Ps4, Pd4, yb, p->consts, p->partials, make_fin(p, stage, fused));
       }
       break;
-    case MPN_STAGE_NODE:
-      if (stored) mpn::launch(node_moments_sweep_kernel<1, false>, SWEEP_GRID, SWEEP_THREADS, 0, st, g, ea, Ps4, Pd4, yb, p->consts, (float4*)p->s1_task, p->partials, p->A, p->w.small, make_fin(p, stage, fused));
-      else mpn::launch(node_moments_sweep_kernel<0, false>, SWEEP_GRID, SWEEP_THREADS, 0, st, g, ea, Ps4, Pd4, nullptr, p->consts, (float4*)p->s1_task, p->partials, p->A, p->w.small, make_fin(p, stage, fused));
+    case MPN_STAGE_NODE: {
+      FinArgs nf;
+      MPN_TRY(sweep_fin(p, stage, fused, stored ? SWEEP_RESIDENT_GRID : SWEEP_GRID, st, nf));
+      if (stored) mpn::launch(node_moments_sweep_kernel<1, false>, SWEEP_RESIDENT_GRID, SWEEP_THREADS, 0, st, g, ea, Ps4, Pd4, yb, p->consts, (float4*)p->s1_task, p->partials, p->A, p->w.small, nf);
+      else mpn::launch(node_moments_sweep_kernel<0, false>, SWEEP_GRID, SWEEP_THREADS, 0, st, g, ea, Ps4, Pd4, nullptr, p->consts, (float4*)p->s1_task, p->partials, p->A, p->w.small, nf);
       break;
+    }
     case MPN_STAGE_APPLY: {
       const bool classify = logits_out != nullptr;
       float2* lg = (float2*)logits_out;
@@ -2281,7 +2333,7 @@ static int forward_sharded_impl(const mpn_graph* g, const mpn_weights* w, const 
   unsigned long long& seq_m = p->seq_m;
   unsigned long long seq_h = peers->seq_h, seq_c = peers->seq_c;
   if (cudaMemcpyAsync(p->peers_dev, &P, sizeof(PeerArgs), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-      cudaMemsetAsync(p->fin_counter, 0, sizeof(unsigned int), st) != cudaSuccess) {
+      cudaMemsetAsync(p->fin_counter, 0, sizeof(unsigned int) * FIN_COUNTERS, st) != cudaSuccess) {
     set_error("peer table upload failed");
     mpn_plan_destroy(p);
     return MPN_ERR_CUDA;
