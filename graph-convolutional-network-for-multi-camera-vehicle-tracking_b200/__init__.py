@@ -4,6 +4,7 @@ Public surface (same names as the reference where one exists):
     MOTMPNet                     models/mpn.py:144
     edge_features                inference.py:453-456
     post_processing              inference.py:70
+    post_processing_batched      post_processing for every graph of a batch in one call (new; see INTEGRATION.md)
     pruning, splitting, remove_edges_single_direction, compute_SCC_and_Clusters      utils.py
     ShardedMPN                   row-block sharded forward across the GPUs of one box (new; see DESIGN.md)
     GraphStream                  a stream of host-resident graphs: PCIe copies of neighbouring graphs overlap the kernels (new)
@@ -27,10 +28,10 @@ from .mpn import MOTMPNet
 from .pipeline import GraphStream, ShardedGraphStream, unpack_decisions
 from .sharded import (CudaPhases, CudaPostOps, ShardedMPN, partition_rows, shard_edges, sharded_forward,
                       sharded_post_processing)
-from .postprocess import (compute_SCC_and_Clusters, post_processing, pruning, remove_edges_single_direction,
-                          split_stats, splitting)
+from .postprocess import (compute_SCC_and_Clusters, post_processing, post_processing_batched, pruning,
+                          remove_edges_single_direction, split_stats, splitting)
 
-__all__ = ["MOTMPNet", "edge_features", "post_processing", "pruning", "splitting", "remove_edges_single_direction",
+__all__ = ["MOTMPNet", "edge_features", "post_processing", "post_processing_batched", "pruning", "splitting", "remove_edges_single_direction",
            "compute_SCC_and_Clusters", "split_stats", "TrackletGraph", "graph_for", "ShardedMPN", "CudaPhases", "sharded_forward", "partition_rows",
            "shard_edges", "GraphStream", "ShardedGraphStream", "unpack_decisions", "sharded_post_processing", "CudaPostOps", "_lib", "evaluation", "compute_P_R_F", "clustering_scores", "relabel_detections", "tracking_table",
            "save_mtmc", "edge_labels", "normalize_columns", "pack_reid_features", "pack_reid_features_from_pickles",

@@ -132,6 +132,8 @@ _PROTOS = {
     "mpn_scc_labels": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p, C.c_size_t, C.c_void_p]),
     "mpn_post_processing": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                       C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpn_post_processing_batched": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "mpn_active_edges": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64),
                                    C.c_void_p, C.c_size_t, C.c_void_p]),
     "mpn_compact_workspace_bytes": (C.c_size_t, [C.POINTER(MpnGraph)]),
@@ -141,6 +143,8 @@ _PROTOS = {
     "mpn_clear_inactive": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "mpn_labels_reference": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p, C.c_size_t,
                                       C.c_void_p]),
+    "mpn_labels_reference_batched": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                              C.c_void_p]),
     "mpn_labels_reference_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.POINTER(C.c_int32)]),
     "mpn_split_exact_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
                                       C.c_void_p]),

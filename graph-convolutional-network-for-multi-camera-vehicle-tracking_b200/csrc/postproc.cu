@@ -7,8 +7,11 @@
 // packed (prob bits, edge id) 64-bit atomicMin (ties -> lowest edge id, as torch.argmin over ascending
 // candidates, utils.py:288-289), components use min-id union-find.
 #include <algorithm>
+#include <atomic>
 #include <chrono>
 #include <cstdlib>
+#include <string>
+#include <thread>
 #include <unordered_map>
 #include <vector>
 
@@ -36,6 +39,9 @@ struct PostCtx {
   int tie_cap;
   float* a_prob;                                                 // SPLIT: probabilities in active-list order
   uint8_t *sel, *tiedb;                                          // SPLIT: entry selected for the host; value carried by >= 2 active edges
+  // batched graphs only (n_graphs > 1)
+  int *a_gptr, *gflag, *groots;                                  // first active-list entry per graph [G+1]; per-graph flag, root count [G]
+  unsigned long long *hash64, *tie_keys64;                       // SPLIT sets keyed by (graph id, probability bits)
   size_t total;
   // host
   int n_active;
@@ -76,6 +82,16 @@ static void post_layout(PostCtx& c, void* ws, size_t ws_bytes) {
   c.sel = a.take<uint8_t>(E);
   c.tiedb = a.take<uint8_t>(E);
   c.counters = a.take<int>(16);
+  c.a_gptr = c.gflag = c.groots = nullptr;
+  c.hash64 = c.tie_keys64 = nullptr;
+  if (c.g.n_graphs > 1) {                                        // appended: the single-graph layout is unchanged
+    const size_t G = (size_t)c.g.n_graphs;
+    c.a_gptr = a.take<int>(G + 1);
+    c.gflag = a.take<int>(G);
+    c.groots = a.take<int>(G);
+    c.hash64 = a.take<unsigned long long>(c.hash_cap);
+    c.tie_keys64 = a.take<unsigned long long>(c.tie_cap);
+  }
   c.total = a.off;
 }
 
@@ -248,6 +264,27 @@ __global__ void prune_pick_kernel(int A, const int* __restrict__ a_eid, const in
   }
   if (viol) *any_violation = 1;
 }
+// batched graphs: the bound of a node is num_cameras[its graph] - 1 (an edge's endpoints lie in one graph)
+__global__ void prune_pick_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src,
+                                          const int* __restrict__ a_dst, const uint8_t* __restrict__ act, const float* __restrict__ prob,
+                                          int pstride, const int* __restrict__ gid, const int* __restrict__ ncam,
+                                          const int* __restrict__ fo, const int* __restrict__ fi, unsigned long long* __restrict__ mo,
+                                          unsigned long long* __restrict__ mi, int* __restrict__ any_violation) {
+  bool viol = false;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
+    const int e = a_eid[i];
+    if (!act[e]) continue;
+    const int u = a_src[i], v = a_dst[i];
+    const int limit = ncam[gid[u]] - 1;
+    const bool bo = fo[u] > limit, bi = fi[v] > limit;
+    if (!(bo || bi)) continue;
+    viol = true;
+    const unsigned long long key = ((unsigned long long)__float_as_uint(prob[(size_t)e * pstride]) << 32) | (unsigned int)e;
+    if (bo) atomicMin(&mo[u], key);
+    if (bi) atomicMin(&mi[v], key);
+  }
+  if (viol) *any_violation = 1;
+}
 __global__ void prune_remove_kernel(int N, const unsigned long long* __restrict__ mo, const unsigned long long* __restrict__ mi,
                                     uint8_t* __restrict__ act) {
   for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) {
@@ -267,8 +304,11 @@ __global__ void prune_reset_kernel(int N, int* __restrict__ fo, int* __restrict_
 // Rounds are enqueued PRUNE_BATCH at a time with one flag word each and the host reads the flags once per batch: a round without
 // a violating node removes nothing, so the rounds enqueued past the fixed point are no-ops (the violation flags of a batch are a
 // prefix of ones).  One host round trip per 8 rounds instead of one per round (the smoke graph needs 87 rounds).
+// BATCH: per-graph bounds num_cameras_dev[node_gid[n]]; a graph that has converged sees no-op rounds while the others go on.
 constexpr int PRUNE_BATCH = 8;
-static int prune_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride, int num_cameras, int* changed, int* rounds) {
+template <bool BATCH = false>
+static int prune_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride, int num_cameras, int* changed, int* rounds,
+                       const int* num_cameras_dev = nullptr) {
   const int A = c.n_active, N = c.g.n_nodes;
   *changed = 0;
   *rounds = 0;
@@ -281,8 +321,12 @@ static int prune_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride,
       MPN_LAUNCH_OK();
       flow_count_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.fo, c.fi);
       MPN_LAUNCH_OK();
-      prune_pick_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, prob, pstride, num_cameras - 1, c.fo,
-                                                        c.fi, c.mo, c.mi, flags + r);
+      if constexpr (BATCH)
+        prune_pick_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, prob, pstride, c.g.node_gid,
+                                                                  num_cameras_dev, c.fo, c.fi, c.mo, c.mi, flags + r);
+      else
+        prune_pick_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, prob, pstride, num_cameras - 1, c.fo,
+                                                          c.fi, c.mo, c.mi, flags + r);
       MPN_LAUNCH_OK();
       prune_remove_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.mo, c.mi, act);
       MPN_LAUNCH_OK();
@@ -916,6 +960,382 @@ static int split_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride,
   return MPN_OK;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Batched graphs (n_graphs > 1): G block-diagonal graphs, nodes of a graph contiguous, edges (row, col)-sorted, so the active
+// entries of graph g are the contiguous slice [a_gptr[g], a_gptr[g+1]) of the active list.  CUT, the union-find SCC and the
+// canonical labels are graph-local as they stand (the reverse edge and every SCC lie inside one graph); what the kernels below add
+// is the per-graph camera bound and, for SPLITTING, sets keyed by (graph id, probability bits): the reference removes every edge
+// of ITS graph whose probability equals the dropped minimum (utils.py:96-98), so a value shared by two different graphs must
+// neither couple them nor count as a tie.
+// ------------------------------------------------------------------------------------------------
+constexpr unsigned long long HASH64_EMPTY = ~0ull;         // never a key: graph ids are < 2^31
+__device__ __forceinline__ unsigned long long graph_value_key(int g, unsigned int bits) {
+  return ((unsigned long long)(unsigned int)g << 32) | bits;
+}
+__device__ __forceinline__ unsigned int hash_u64(unsigned long long k) {
+  return hash_u32((unsigned int)k ^ hash_u32((unsigned int)(k >> 32) + 0x9e3779b9u));
+}
+__device__ __forceinline__ void set64_insert(unsigned long long* __restrict__ t, int cap, unsigned long long key) {
+  unsigned int slot = hash_u64(key) & (cap - 1);
+  for (;;) {
+    const unsigned long long old = atomicCAS(&t[slot], HASH64_EMPTY, key);
+    if (old == HASH64_EMPTY || old == key) return;
+    slot = (slot + 1) & (cap - 1);
+  }
+}
+__device__ __forceinline__ int set64_find(const unsigned long long* __restrict__ t, int cap, unsigned long long key) {
+  unsigned int slot = hash_u64(key) & (cap - 1);
+  for (;;) {
+    const unsigned long long v = t[slot];
+    if (v == key) return (int)slot;
+    if (v == HASH64_EMPTY) return -1;
+    slot = (slot + 1) & (cap - 1);
+  }
+}
+
+// a_gptr[g] = first active-list entry at or after the first edge of graph g (a_eid ascends); a_gptr[G] = A
+__global__ void active_graph_ptr_kernel(int G, const int* __restrict__ rowptr, const int* __restrict__ nptr, const int* __restrict__ a_eid,
+                                        int A, int* __restrict__ a_gptr) {
+  for (int g = blockIdx.x * blockDim.x + threadIdx.x; g <= G; g += gridDim.x * blockDim.x) {
+    const int e0 = rowptr[nptr[g]];
+    int lo = 0, hi = A;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (a_eid[mid] < e0) lo = mid + 1; else hi = mid;
+    }
+    a_gptr[g] = lo;
+  }
+}
+// canonical graph-local labels (smallest node id of the SCC minus the graph's first node) and the number of SCCs per graph
+__global__ void graph_labels_kernel(int N, const int* __restrict__ label, const int* __restrict__ gid, const int* __restrict__ nptr,
+                                    int* __restrict__ local, int* __restrict__ roots) {
+  for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) {
+    const int g = gid[n], l = label[n];
+    if (local) local[n] = l - nptr[g];
+    if (l == n) atomicAdd(&roots[g], 1);
+  }
+}
+// skip (optional): graphs whose clusters are left out (they go through the reference order on the host)
+__global__ void mark_dirty_nodes_batched_kernel(int N, const int* __restrict__ label, const int* __restrict__ size, const int* __restrict__ gid,
+                                                const int* __restrict__ ncam, const int* __restrict__ skip, int* __restrict__ list,
+                                                int* __restrict__ count) {
+  for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) {
+    const int g = gid[n];
+    if ((skip == nullptr || !skip[g]) && size[label[n]] > ncam[g]) list[atomicAdd(count, 1)] = n;
+  }
+}
+__global__ void mark_dirty_edges_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src,
+                                                const int* __restrict__ a_dst, const uint8_t* __restrict__ act, const int* __restrict__ label,
+                                                const int* __restrict__ size, const int* __restrict__ gid, const int* __restrict__ ncam,
+                                                const int* __restrict__ skip, int* __restrict__ list, int* __restrict__ count) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
+    if (!act[a_eid[i]]) continue;
+    const int g = gid[a_src[i]];
+    if (skip != nullptr && skip[g]) continue;
+    const int limit = ncam[g];
+    if (size[label[a_src[i]]] > limit || size[label[a_dst[i]]] > limit) list[atomicAdd(count, 1)] = i;
+  }
+}
+__global__ void split_min_list_batched_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ a_eid,
+                                              const int* __restrict__ a_src, const int* __restrict__ a_dst, const uint8_t* __restrict__ act,
+                                              const float* __restrict__ prob, int pstride, const int* __restrict__ label,
+                                              const int* __restrict__ size, const int* __restrict__ gid, const int* __restrict__ ncam,
+                                              unsigned int* __restrict__ mbits) {
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
+    const int i = list[k];
+    const int e = a_eid[i];
+    if (!act[e]) continue;
+    const int lu = label[a_src[i]], lv = label[a_dst[i]];
+    const int limit = ncam[gid[a_src[i]]];
+    const unsigned int pb = __float_as_uint(prob[(size_t)e * pstride]);
+    if (size[lu] > limit) atomicMin(&mbits[lu], pb);
+    if (lv != lu && size[lv] > limit) atomicMin(&mbits[lv], pb);
+  }
+}
+__global__ void split_collect_list_batched_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ label,
+                                                  const int* __restrict__ size, const int* __restrict__ gid, const int* __restrict__ ncam,
+                                                  const unsigned int* __restrict__ mbits, unsigned long long* __restrict__ hash, int cap,
+                                                  int* __restrict__ n_big) {
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
+    const int n = list[k];
+    if (label[n] != n || size[n] <= ncam[gid[n]]) continue;
+    atomicAdd(n_big, 1);
+    const unsigned int bits = mbits[n];
+    if (bits == HASH_EMPTY) continue;
+    set64_insert(hash, cap, graph_value_key(gid[n], bits));
+  }
+}
+// every active edge of a graph whose probability equals one of that graph's dropped minima (utils.py:96-98)
+__global__ void split_remove_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ gid,
+                                            uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
+                                            const unsigned long long* __restrict__ hash, int cap) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
+    const int e = a_eid[i];
+    if (!act[e]) continue;
+    if (set64_find(hash, cap, graph_value_key(gid[a_src[i]], __float_as_uint(prob[(size_t)e * pstride]))) >= 0) act[e] = 0;
+  }
+}
+// ties per graph: the values of the dirty edges, how many active edges of the SAME graph carry each, the graphs that have one
+__global__ void tie_insert_batched_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ a_eid, const int* __restrict__ a_src,
+                                          const int* __restrict__ gid, const uint8_t* __restrict__ act, const float* __restrict__ prob,
+                                          int pstride, unsigned long long* __restrict__ keys, int cap) {
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
+    const int i = list[k];
+    const int e = a_eid[i];
+    if (!act[e]) continue;
+    set64_insert(keys, cap, graph_value_key(gid[a_src[i]], __float_as_uint(prob[(size_t)e * pstride])));
+  }
+}
+__global__ void tie_count_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ gid,
+                                         const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
+                                         const unsigned long long* __restrict__ keys, int* __restrict__ counts, int cap) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
+    const int e = a_eid[i];
+    if (!act[e]) continue;
+    const int slot = set64_find(keys, cap, graph_value_key(gid[a_src[i]], __float_as_uint(prob[(size_t)e * pstride])));
+    if (slot >= 0) atomicAdd(&counts[slot], 1);
+  }
+}
+__global__ void flag_wcc_ties_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ gid,
+                                             const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
+                                             const unsigned long long* __restrict__ keys, const int* __restrict__ counts, int cap,
+                                             const int* __restrict__ wcc, int* __restrict__ flag, uint8_t* __restrict__ tiedb,
+                                             int* __restrict__ gtied, int* __restrict__ n_tied_edges) {
+  int tied = 0;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
+    const int e = a_eid[i];
+    uint8_t t = 0;
+    if (act[e]) {
+      const int g = gid[a_src[i]];
+      const int slot = set64_find(keys, cap, graph_value_key(g, __float_as_uint(prob[(size_t)e * pstride])));
+      if (slot >= 0 && counts[slot] >= 2) { flag[wcc[a_src[i]]] = 1; gtied[g] = 1; ++tied; t = 1; }
+    }
+    tiedb[i] = t;
+  }
+  tied = __reduce_add_sync(0xffffffffu, tied);
+  if ((threadIdx.x & 31) == 0 && tied) atomicAdd(n_tied_edges, tied);
+}
+__global__ void flag_graphs_of_nodes_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ gid, int* __restrict__ gflag) {
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) gflag[gid[list[k]]] = 1;
+}
+
+static int copy_graph_ptr(const PostCtx& c, std::vector<int>& nptr) {
+  nptr.resize((size_t)c.g.n_graphs + 1);
+  MPN_CUDA_OK(cudaMemcpyAsync(nptr.data(), c.g.graph_nptr, sizeof(int) * nptr.size(), cudaMemcpyDeviceToHost, c.st));
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  return MPN_OK;
+}
+
+// The reference order on the host for the graphs flagged in c.gflag (a probability tie among the values one of their oversized
+// clusters can drop): one split_exact_host_impl call per graph on its own slice of the active list, with graph-local node ids,
+// its own node count and camera bound — exactly the call a single-graph post-processing of that graph makes, so the engine's
+// numbering and its re-read of the integer label (utils.py:112) are the graph's own.  Graphs are independent: they run on a few
+// host threads, each writing its own slice, and the result depends neither on the thread count nor on the order of the seeds.
+static int split_host_graphs(PostCtx& c, uint8_t* act, const float* prob, int pstride, const std::vector<int>& ncam,
+                             const std::vector<int>& nptr, const std::vector<int>& host_graph, int Dn, bool have_ties,
+                             long long* steps, long long* off_lowest) {
+  const int A = c.n_active, G = c.g.n_graphs;
+  gather_select_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, act, prob, pstride, c.wcc, c.wccflag, c.a_prob, c.sel);
+  MPN_LAUNCH_OK();
+  active_graph_ptr_kernel<<<list_grid(G + 1), 256, 0, c.st>>>(G, c.g.rowptr, c.g.graph_nptr, c.a_eid, A, c.a_gptr);
+  MPN_LAUNCH_OK();
+  std::vector<int> agp((size_t)G + 1), seeds(Dn);
+  MPN_CUDA_OK(cudaMemcpyAsync(agp.data(), c.a_gptr, sizeof(int) * (G + 1), cudaMemcpyDeviceToHost, c.st));
+  MPN_CUDA_OK(cudaMemcpyAsync(seeds.data(), c.dirty_nodes, sizeof(int) * Dn, cudaMemcpyDeviceToHost, c.st));
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  // runs of consecutive host-order graphs = contiguous ranges of the active list, packed back to back in pinned staging
+  struct Run { int g0, g1; long long a0, a1, h0; };
+  std::vector<Run> runs;
+  long long staged = 0;
+  for (int g = 0; g < G; ++g) {
+    if (!host_graph[g]) continue;
+    if (!runs.empty() && runs.back().g1 == g) { runs.back().g1 = g + 1; runs.back().a1 = agp[g + 1]; continue; }
+    runs.push_back(Run{g, g + 1, agp[g], agp[g + 1], 0});
+  }
+  for (Run& r : runs) { r.h0 = staged; staged += r.a1 - r.a0; }
+  const size_t S16 = ((size_t)staged + 15) & ~(size_t)15;
+  char* pin = (char*)g_split_pin.get(15 * S16 + 64);
+  MPN_REQUIRE(pin != nullptr, "split: out of pinned host memory (%zu bytes)", 15 * S16 + 64);
+  int* hs = (int*)pin;
+  int* hd = (int*)(pin + 4 * S16);
+  float* hp = (float*)(pin + 8 * S16);
+  uint8_t* hsel = (uint8_t*)(pin + 12 * S16);
+  uint8_t* htied = hsel + S16;
+  uint8_t* keep = htied + S16;
+  for (const Run& r : runs) {
+    const size_t n = (size_t)(r.a1 - r.a0);
+    if (n == 0) continue;
+    MPN_CUDA_OK(cudaMemcpyAsync(hs + r.h0, c.a_src + r.a0, sizeof(int) * n, cudaMemcpyDeviceToHost, c.st));
+    MPN_CUDA_OK(cudaMemcpyAsync(hd + r.h0, c.a_dst + r.a0, sizeof(int) * n, cudaMemcpyDeviceToHost, c.st));
+    MPN_CUDA_OK(cudaMemcpyAsync(hp + r.h0, c.a_prob + r.a0, sizeof(float) * n, cudaMemcpyDeviceToHost, c.st));
+    MPN_CUDA_OK(cudaMemcpyAsync(hsel + r.h0, c.sel + r.a0, n, cudaMemcpyDeviceToHost, c.st));
+    if (have_ties) MPN_CUDA_OK(cudaMemcpyAsync(htied + r.h0, c.tiedb + r.a0, n, cudaMemcpyDeviceToHost, c.st));
+  }
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  // per host-order graph: where its slice sits in the staging, its seeds in graph-local ids
+  std::vector<int> graphs;
+  std::vector<long long> h_of((size_t)G, -1);
+  for (const Run& r : runs)
+    for (int g = r.g0; g < r.g1; ++g) { graphs.push_back(g); h_of[g] = r.h0 + (agp[g] - r.a0); }
+  std::vector<std::vector<int>> gseeds((size_t)G);
+  for (int v : seeds) {
+    const int g = (int)(std::upper_bound(nptr.begin(), nptr.end(), v) - nptr.begin()) - 1;
+    if (host_graph[g]) gseeds[g].push_back(v - nptr[g]);
+  }
+  std::vector<int64_t> gst(4 * (size_t)G, 0);
+  std::vector<int> rc((size_t)G, MPN_OK);
+  std::vector<std::string> err((size_t)G);
+  std::atomic<size_t> next{0};
+  auto worker = [&] {
+    std::vector<int> ls, ld;
+    for (size_t k = next++; k < graphs.size(); k = next++) {
+      const int g = graphs[k];
+      const long long h = h_of[g], m = agp[g + 1] - agp[g];
+      const int n0 = nptr[g];
+      long long n_sel = 0;
+      ls.resize(m); ld.resize(m);
+      for (long long i = 0; i < m; ++i) { ls[i] = hs[h + i] - n0; ld[i] = hd[h + i] - n0; n_sel += hsel[h + i]; }
+      if (n_sel == 0) { memset(keep + h, 1, (size_t)m); continue; }
+      rc[g] = split_exact_host_impl(ls.data(), ld.data(), hp + h, m, nptr[g + 1] - n0, ncam[g], keep + h, &gst[4 * (size_t)g],
+                                    have_ties ? htied + h : nullptr, gseeds[g].data(), (long long)gseeds[g].size(), hsel + h);
+      if (rc[g] != MPN_OK) err[g] = mpn_last_error();
+    }
+  };
+  const int n_threads = (int)std::min<size_t>(graphs.size(), std::max(1u, std::min(8u, std::thread::hardware_concurrency())));
+  if (n_threads <= 1) {
+    worker();
+  } else {
+    std::vector<std::thread> pool;
+    for (int t = 0; t < n_threads; ++t) pool.emplace_back(worker);
+    for (std::thread& t : pool) t.join();
+  }
+  for (int g : graphs)
+    if (rc[g] != MPN_OK) { set_error("split (graph %d of the batch): %s", g, err[g].c_str()); return rc[g]; }
+  *steps = *off_lowest = 0;
+  for (int g : graphs) { *steps += gst[4 * (size_t)g]; *off_lowest += gst[4 * (size_t)g + 1]; }
+  // write back: keep = 1 everywhere but in the slices the engine decided
+  MPN_CUDA_OK(cudaMemsetAsync(c.sel, 1, (size_t)A, c.st));
+  for (const Run& r : runs)
+    if (r.a1 > r.a0) MPN_CUDA_OK(cudaMemcpyAsync(c.sel + r.a0, keep + r.h0, (size_t)(r.a1 - r.a0), cudaMemcpyHostToDevice, c.st));
+  apply_keep_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.sel, act);
+  MPN_LAUNCH_OK();
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));        // the staging buffer is reused by the next call
+  return MPN_OK;
+}
+
+// SPLITTING of every graph of the batch.  The mode is chosen per graph: a graph with a tie among the values its oversized clusters
+// can drop (or every graph with an oversized cluster, when the tie table does not fit) goes through the reference order on the
+// host; the others drop their minima in parallel rounds on the device, restricted to their own dirty lists.  Graphs are
+// independent, so both modes run on one batch and the result is exact.
+static int split_stage_batched(PostCtx& c, uint8_t* act, const float* prob, int pstride, const int* ncam_dev,
+                               const std::vector<int>& ncam, const std::vector<int>& nptr) {
+  const int A = c.n_active, N = c.g.n_nodes, G = c.g.n_graphs;
+  const int* gid = c.g.node_gid;
+  g_split_stats[0] = g_split_stats[1] = g_split_stats[2] = g_split_stats[3] = 0;
+  if (A == 0) return MPN_OK;
+  MPN_TRY(scc_stage(c, act, nullptr));
+  MPN_CUDA_OK(cudaMemsetAsync(c.size, 0, sizeof(int) * N, c.st));
+  MPN_CUDA_OK(cudaMemsetAsync(c.counters + 5, 0, 4 * sizeof(int), c.st));
+  comp_size_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size);
+  MPN_LAUNCH_OK();
+  mark_dirty_nodes_batched_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size, gid, ncam_dev, nullptr, c.dirty_nodes, c.counters + 5);
+  MPN_LAUNCH_OK();
+  mark_dirty_edges_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.label, c.size, gid, ncam_dev, nullptr,
+                                                                  c.dirty_edges, c.counters + 6);
+  MPN_LAUNCH_OK();
+  int h[2] = {0, 0};
+  MPN_CUDA_OK(cudaMemcpyAsync(h, c.counters + 5, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.st));
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  int Dn = h[0], De = h[1];
+  if (Dn == 0) return MPN_OK;
+  // ---- which graphs have a tie among the values their oversized clusters can drop?
+  iota_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.wcc);
+  MPN_LAUNCH_OK();
+  union_all_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.wcc);
+  MPN_LAUNCH_OK();
+  flatten_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.wcc, nullptr);
+  MPN_LAUNCH_OK();
+  MPN_CUDA_OK(cudaMemsetAsync(c.wccflag, 0, sizeof(int) * N, c.st));
+  MPN_CUDA_OK(cudaMemsetAsync(c.gflag, 0, sizeof(int) * G, c.st));
+  const bool table_fits = (long long)De * 5 <= (long long)c.tie_cap * 3;       // load factor <= 0.6
+  int n_tied = 0;
+  if (table_fits) {
+    MPN_CUDA_OK(cudaMemsetAsync(c.tie_keys64, 0xFF, sizeof(unsigned long long) * c.tie_cap, c.st));
+    MPN_CUDA_OK(cudaMemsetAsync(c.tie_counts, 0, sizeof(int) * c.tie_cap, c.st));
+    if (De > 0) {
+      tie_insert_batched_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, gid, act, prob, pstride, c.tie_keys64,
+                                                                 c.tie_cap);
+      MPN_LAUNCH_OK();
+    }
+    tie_count_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, gid, act, prob, pstride, c.tie_keys64, c.tie_counts,
+                                                             c.tie_cap);
+    MPN_LAUNCH_OK();
+    flag_wcc_ties_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, gid, act, prob, pstride, c.tie_keys64, c.tie_counts,
+                                                                 c.tie_cap, c.wcc, c.wccflag, c.tiedb, c.gflag, c.counters + 7);
+    MPN_LAUNCH_OK();
+    flag_wcc_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.wcc, c.wccflag);
+    MPN_LAUNCH_OK();
+  } else {
+    MPN_CUDA_OK(cudaMemsetAsync(c.wccflag, 0x01, sizeof(int) * N, c.st));   // every component of the host-order graphs
+    flag_graphs_of_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, gid, c.gflag);
+    MPN_LAUNCH_OK();
+  }
+  std::vector<int> host_graph((size_t)G);
+  MPN_CUDA_OK(cudaMemcpyAsync(host_graph.data(), c.gflag, sizeof(int) * G, cudaMemcpyDeviceToHost, c.st));
+  MPN_CUDA_OK(cudaMemcpyAsync(&n_tied, c.counters + 7, sizeof(int), cudaMemcpyDeviceToHost, c.st));
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  long long n_host = 0, host_steps = 0, host_off_lowest = 0;
+  for (int g = 0; g < G; ++g) n_host += host_graph[g] != 0;
+  g_split_stats[0] = table_fits ? n_tied : -1;
+  if (n_host > 0) {
+    MPN_TRY(split_host_graphs(c, act, prob, pstride, ncam, nptr, host_graph, Dn, table_fits, &host_steps, &host_off_lowest));
+    // the device rounds below only see the other graphs
+    MPN_CUDA_OK(cudaMemsetAsync(c.counters + 5, 0, 2 * sizeof(int), c.st));
+    mark_dirty_nodes_batched_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size, gid, ncam_dev, c.gflag, c.dirty_nodes, c.counters + 5);
+    MPN_LAUNCH_OK();
+    mark_dirty_edges_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.label, c.size, gid, ncam_dev, c.gflag,
+                                                                    c.dirty_edges, c.counters + 6);
+    MPN_LAUNCH_OK();
+    MPN_CUDA_OK(cudaMemcpyAsync(h, c.counters + 5, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.st));
+    MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+    Dn = h[0];
+    De = h[1];
+  }
+  // ---- no tie inside any of the remaining graphs: every oversized cluster drops its minimum in the same round
+  int rounds = 0;
+  while (Dn > 0) {
+    reset_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, c.mbits, 4);
+    MPN_LAUNCH_OK();
+    MPN_CUDA_OK(cudaMemsetAsync(c.hash64, 0xFF, sizeof(unsigned long long) * c.hash_cap, c.st));
+    MPN_CUDA_OK(cudaMemsetAsync(c.counters + 4, 0, sizeof(int), c.st));
+    if (De > 0) {
+      split_min_list_batched_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, c.a_dst, act, prob, pstride,
+                                                                     c.label, c.size, gid, ncam_dev, c.mbits);
+      MPN_LAUNCH_OK();
+    }
+    split_collect_list_batched_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, gid, ncam_dev, c.mbits, c.hash64,
+                                                                       c.hash_cap, c.counters + 4);
+    MPN_LAUNCH_OK();
+    int n_big = 0;
+    MPN_CUDA_OK(cudaMemcpyAsync(&n_big, c.counters + 4, sizeof(int), cudaMemcpyDeviceToHost, c.st));
+    MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+    if (n_big == 0) break;
+    ++rounds;
+    if (rounds > A + 1) { set_error("split did not converge"); return MPN_ERR_INVALID; }
+    split_remove_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, gid, act, prob, pstride, c.hash64, c.hash_cap);
+    MPN_LAUNCH_OK();
+    MPN_TRY(scc_dirty(c, act, Dn, De));
+    reset_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, c.mbits, 2);
+    MPN_LAUNCH_OK();
+    comp_size_list_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size);
+    MPN_LAUNCH_OK();
+  }
+  g_split_stats[1] = rounds + host_steps;
+  g_split_stats[2] = host_off_lowest;
+  g_split_stats[3] = n_host;
+  return MPN_OK;
+}
+
 static int post_begin(PostCtx& c, const mpn_graph* g, const uint8_t* act, void* ws, size_t ws_bytes, void* stream) {
   MPN_REQUIRE(g && ws, "post: NULL argument");
   MPN_REQUIRE(act || g->n_edges == 0, "post: NULL activity flags");
@@ -1041,7 +1461,14 @@ __global__ void select_flagged_kernel(int A, const int* __restrict__ a_eid, cons
 void scc_emission_keys_host(const int* src, const int* dst, long long m, int n_nodes, std::vector<int>& node_out,
                             std::vector<long long>& key_out, std::vector<int>& idx_out, std::vector<int>& size_out);   // split_exact.cu
 
-static int labels_reference_parallel(PostCtx& c, const uint8_t* act, long long* labels_out, int* n_comp_out) {
+// per SCC (root = smallest node id) of the active digraph: size, first-appearance key and index within the emitting DFS;
+// label[n] = root of n, fa[n] = first-appearance key of n (0xFFFFFFFF: no active edge)
+struct RefKeys {
+  std::vector<int> label;
+  std::vector<unsigned int> fa, size, idx;
+  std::vector<unsigned long long> key;
+};
+static int reference_keys(PostCtx& c, const uint8_t* act, RefKeys& k) {
   const int A = c.n_active, N = c.g.n_nodes;
   MPN_TRY(scc_stage(c, act, nullptr));
   unsigned int* fa = reinterpret_cast<unsigned int*>(c.fo);
@@ -1054,8 +1481,10 @@ static int labels_reference_parallel(PostCtx& c, const uint8_t* act, long long* 
     inter_scc_flag_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.label, nullptr, nullptr, c.counters + 7);
     MPN_LAUNCH_OK();
   }
-  std::vector<int> h_label(N);
-  std::vector<unsigned int> h_fa(N);
+  std::vector<int>& h_label = k.label;
+  std::vector<unsigned int>& h_fa = k.fa;
+  h_label.resize(N);
+  h_fa.resize(N);
   MPN_CUDA_OK(cudaMemcpyAsync(h_label.data(), c.label, sizeof(int) * N, cudaMemcpyDeviceToHost, c.st));
   MPN_CUDA_OK(cudaMemcpyAsync(h_fa.data(), fa, sizeof(unsigned int) * N, cudaMemcpyDeviceToHost, c.st));
   MPN_CUDA_OK(cudaMemcpyAsync(&n_inter, c.counters + 7, sizeof(int), cudaMemcpyDeviceToHost, c.st));
@@ -1091,10 +1520,11 @@ static int labels_reference_parallel(PostCtx& c, const uint8_t* act, long long* 
       if (hsel[i]) { pos.push_back(i); ss.push_back(hs[i]); dd.push_back(hd[i]); }
     scc_emission_keys_host(ss.data(), dd.data(), (long long)ss.size(), N, cx_node, cx_key, cx_idx, cx_size);
   }
-  // per SCC (root = smallest node id): size, key, index; then the rank
-  struct Rep { unsigned int size; unsigned int idx; unsigned long long key; int root; };
-  std::vector<unsigned int> size(N, 0u), idx(N, 0u);
-  std::vector<unsigned long long> key(N, ~0ull);
+  std::vector<unsigned int>&size = k.size, &idx = k.idx;
+  std::vector<unsigned long long>& key = k.key;
+  size.assign(N, 0u);
+  idx.assign(N, 0u);
+  key.assign(N, ~0ull);
   for (int n = 0; n < N; ++n) {
     if (h_fa[n] == 0xFFFFFFFFu) continue;
     const int r = h_label[n];
@@ -1108,46 +1538,110 @@ static int labels_reference_parallel(PostCtx& c, const uint8_t* act, long long* 
     idx[r] = (unsigned int)cx_idx[v];
     if ((unsigned int)cx_size[v] != size[r]) { set_error("reference numbering: component sizes disagree (device %u, host %d)", size[r], cx_size[v]); return MPN_ERR_INVALID; }
   }
-  // rank of a component = its position in the order (size, key, idx).  Keys are positions in the active list (< 2A + 2): one
-  // bucket pass puts the components in (key, idx) order — several components share a key only when one DFS source of the
-  // sequential generator emitted them, those few are sorted by idx — and a stable counting sort by size finishes the order.
-  std::vector<Rep> reps;
-  {
-    const size_t n_keys = 2 * (size_t)A + 2;
-    std::vector<int> head(n_keys, -1), nxt((size_t)N, -1);
-    unsigned int max_size = 0;
-    size_t n_reps = 0;
-    for (int r = N - 1; r >= 0; --r) {
-      if (size[r] == 0) continue;
-      if (key[r] >= n_keys) { set_error("reference numbering: first-appearance key out of range"); return MPN_ERR_INVALID; }
-      nxt[r] = head[key[r]];
-      head[key[r]] = r;
-      max_size = std::max(max_size, size[r]);
-      ++n_reps;
-    }
-    std::vector<int> by_key;
-    by_key.reserve(n_reps);
-    std::vector<int> same;
-    for (size_t k = 0; k < n_keys; ++k) {
-      int r = head[k];
-      if (r < 0) continue;
-      if (nxt[r] < 0) { by_key.push_back(r); continue; }
-      same.clear();
-      for (; r >= 0; r = nxt[r]) same.push_back(r);
-      std::sort(same.begin(), same.end(), [&](int a, int b) { return idx[a] < idx[b]; });
-      by_key.insert(by_key.end(), same.begin(), same.end());
-    }
-    std::vector<size_t> first((size_t)max_size + 2, 0);
-    for (int r : by_key) ++first[size[r] + 1];
-    for (size_t z = 1; z < first.size(); ++z) first[z] += first[z - 1];
-    reps.resize(n_reps);
-    for (int r : by_key) reps[first[size[r]]++] = Rep{size[r], idx[r], key[r], r};
+  return MPN_OK;
+}
+
+// The roots of the SCCs with an active edge in (key, idx) order, then stably by size.  Keys are positions in the active list
+// (< 2A + 2): one bucket pass puts the components in (key, idx) order — several components share a key only when one DFS source
+// of the sequential generator emitted them, those few are sorted by idx — and a stable counting sort by size finishes the order.
+static int roots_in_reference_order(const RefKeys& k, int A, std::vector<int>& order) {
+  const int N = (int)k.label.size();
+  const size_t n_keys = 2 * (size_t)A + 2;
+  std::vector<int> head(n_keys, -1), nxt((size_t)N, -1);
+  unsigned int max_size = 0;
+  size_t n_reps = 0;
+  for (int r = N - 1; r >= 0; --r) {
+    if (k.size[r] == 0) continue;
+    if (k.key[r] >= n_keys) { set_error("reference numbering: first-appearance key out of range"); return MPN_ERR_INVALID; }
+    nxt[r] = head[k.key[r]];
+    head[k.key[r]] = r;
+    max_size = std::max(max_size, k.size[r]);
+    ++n_reps;
   }
+  std::vector<int> by_key;
+  by_key.reserve(n_reps);
+  std::vector<int> same;
+  for (size_t q = 0; q < n_keys; ++q) {
+    int r = head[q];
+    if (r < 0) continue;
+    if (nxt[r] < 0) { by_key.push_back(r); continue; }
+    same.clear();
+    for (; r >= 0; r = nxt[r]) same.push_back(r);
+    std::sort(same.begin(), same.end(), [&](int a, int b) { return k.idx[a] < k.idx[b]; });
+    by_key.insert(by_key.end(), same.begin(), same.end());
+  }
+  std::vector<size_t> first((size_t)max_size + 2, 0);
+  for (int r : by_key) ++first[k.size[r] + 1];
+  for (size_t z = 1; z < first.size(); ++z) first[z] += first[z - 1];
+  order.resize(n_reps);
+  for (int r : by_key) order[first[k.size[r]]++] = r;
+  return MPN_OK;
+}
+
+static int labels_reference_parallel(PostCtx& c, const uint8_t* act, long long* labels_out, int* n_comp_out) {
+  const int N = c.g.n_nodes;
+  RefKeys k;
+  MPN_TRY(reference_keys(c, act, k));
+  std::vector<int> order;
+  MPN_TRY(roots_in_reference_order(k, c.n_active, order));
   std::vector<int> rank(N, -1);
-  for (size_t i = 0; i < reps.size(); ++i) rank[reps[i].root] = (int)i;
-  long long next = (long long)reps.size();
-  for (int n = 0; n < N; ++n) labels_out[n] = (h_fa[n] != 0xFFFFFFFFu) ? rank[h_label[n]] : next++;
+  for (size_t i = 0; i < order.size(); ++i) rank[order[i]] = (int)i;
+  long long next = (long long)order.size();
+  for (int n = 0; n < N; ++n) labels_out[n] = (k.fa[n] != 0xFFFFFFFFu) ? rank[k.label[n]] : next++;
   if (n_comp_out) *n_comp_out = (int)next;
+  return MPN_OK;
+}
+
+// Batched graphs: each graph numbered from 0 on its own.  A DFS never leaves its graph and the active list holds the graphs one
+// after the other, so a component's (key, idx) orders it within its graph exactly as the single-graph numbering does (keys shifted
+// by the graph's first active entry); the order (size, key, idx) then becomes (graph, size, key, idx) — a stable pass by graph
+// over the single-graph order — and the nodes without an active edge follow their own graph's components, in node order.
+static int labels_reference_batched(PostCtx& c, const uint8_t* act, const std::vector<int>& nptr, long long* labels_out,
+                                    int* n_comp_out) {
+  const int N = c.g.n_nodes, G = c.g.n_graphs;
+  RefKeys k;
+  MPN_TRY(reference_keys(c, act, k));
+  std::vector<int> order;
+  MPN_TRY(roots_in_reference_order(k, c.n_active, order));
+  std::vector<int> gid((size_t)N);
+  for (int g = 0; g < G; ++g)
+    for (int n = nptr[g]; n < nptr[g + 1]; ++n) gid[n] = g;
+  std::vector<int> start((size_t)G + 1, 0);             // components with an active edge per graph -> first position
+  for (int r : order) ++start[gid[r] + 1];
+  for (int g = 0; g < G; ++g) start[g + 1] += start[g];
+  std::vector<int> rank(N, -1);
+  {
+    std::vector<int> fill(start.begin(), start.end() - 1);
+    for (int r : order) { const int g = gid[r]; rank[r] = fill[g]++ - start[g]; }
+  }
+  for (int g = 0; g < G; ++g) {
+    long long next = start[g + 1] - start[g];
+    for (int n = nptr[g]; n < nptr[g + 1]; ++n) labels_out[n] = (k.fa[n] != 0xFFFFFFFFu) ? rank[k.label[n]] : next++;
+    n_comp_out[g] = (int)next;
+  }
+  return MPN_OK;
+}
+
+// inference.post_processing (inference.py:70-169) on one graph: CUT, PRUNE, CUT, SPLIT, then the SCC labels
+static int post_processing_one_graph(PostCtx& c, uint8_t* act, const float* prob1, int pstride, int num_cameras, int flags, int32_t* labels,
+                                     int32_t* n_components, int32_t* prune_changed) {
+  int ch = 0, r = 0;
+  if ((flags & MPN_POST_CUT) && c.n_active) {
+    cut_kernel<<<list_grid(c.n_active), 256, 0, c.st>>>(c.n_active, c.a_eid, c.a_rev, act);
+    MPN_LAUNCH_OK();
+  }
+  if (flags & MPN_POST_PRUNE) MPN_TRY(prune_stage(c, act, prob1, pstride, num_cameras, &ch, &r));
+  if ((flags & MPN_POST_CUT) && c.n_active) {
+    cut_kernel<<<list_grid(c.n_active), 256, 0, c.st>>>(c.n_active, c.a_eid, c.a_rev, act);
+    MPN_LAUNCH_OK();
+  }
+  if (flags & MPN_POST_SPLIT) MPN_TRY(split_stage(c, act, prob1, pstride, num_cameras, &r));
+  int nc = 0;
+  MPN_TRY(scc_stage(c, act, &nc));
+  if (labels) MPN_CUDA_OK(cudaMemcpyAsync(labels, c.label, sizeof(int) * c.g.n_nodes, cudaMemcpyDeviceToDevice, c.st));
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  if (n_components) *n_components = nc;
+  if (prune_changed) *prune_changed = ch;
   return MPN_OK;
 }
 
@@ -1242,23 +1736,40 @@ int mpn_post_processing(const mpn_graph* g, uint8_t* act, const float* prob1, in
   PostCtx c;
   MPN_REQUIRE(prob1 && pstride >= 1 && num_cameras >= 1, "post_processing: bad arguments");
   MPN_TRY(post_begin(c, g, act, ws, ws_bytes, stream));
+  return post_processing_one_graph(c, act, prob1, pstride, num_cameras, flags, labels, n_components, prune_changed);
+}
+
+int mpn_post_processing_batched(const mpn_graph* g, uint8_t* act, const float* prob1, int32_t pstride, const int32_t* num_cameras_dev,
+                                int32_t flags, int32_t* labels, int32_t* n_components, void* ws, size_t ws_bytes, void* stream) {
+  PostCtx c;
+  MPN_REQUIRE(prob1 && pstride >= 1 && num_cameras_dev && n_components, "post_processing_batched: bad arguments");
+  MPN_TRY(post_begin(c, g, act, ws, ws_bytes, stream));
+  const int G = std::max(1, g->n_graphs);
+  std::vector<int> ncam((size_t)G);
+  MPN_CUDA_OK(cudaMemcpyAsync(ncam.data(), num_cameras_dev, sizeof(int) * G, cudaMemcpyDeviceToHost, c.st));
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  for (int k = 0; k < G; ++k) MPN_REQUIRE(ncam[k] >= 1, "post_processing_batched: num_cameras[%d] = %d < 1", k, ncam[k]);
+  if (g->n_graphs <= 1) return post_processing_one_graph(c, act, prob1, pstride, ncam[0], flags, labels, n_components, nullptr);
+  MPN_REQUIRE(g->node_gid && g->graph_nptr, "post_processing_batched: batched graph without node_gid / graph_nptr");
+  std::vector<int> nptr;
+  MPN_TRY(copy_graph_ptr(c, nptr));
   int ch = 0, r = 0;
   if ((flags & MPN_POST_CUT) && c.n_active) {
     cut_kernel<<<list_grid(c.n_active), 256, 0, c.st>>>(c.n_active, c.a_eid, c.a_rev, act);
     MPN_LAUNCH_OK();
   }
-  if (flags & MPN_POST_PRUNE) MPN_TRY(prune_stage(c, act, prob1, pstride, num_cameras, &ch, &r));
+  if (flags & MPN_POST_PRUNE) MPN_TRY(prune_stage<true>(c, act, prob1, pstride, 0, &ch, &r, num_cameras_dev));
   if ((flags & MPN_POST_CUT) && c.n_active) {
     cut_kernel<<<list_grid(c.n_active), 256, 0, c.st>>>(c.n_active, c.a_eid, c.a_rev, act);
     MPN_LAUNCH_OK();
   }
-  if (flags & MPN_POST_SPLIT) MPN_TRY(split_stage(c, act, prob1, pstride, num_cameras, &r));
-  int nc = 0;
-  MPN_TRY(scc_stage(c, act, &nc));
-  if (labels) MPN_CUDA_OK(cudaMemcpyAsync(labels, c.label, sizeof(int) * g->n_nodes, cudaMemcpyDeviceToDevice, c.st));
+  if (flags & MPN_POST_SPLIT) MPN_TRY(split_stage_batched(c, act, prob1, pstride, num_cameras_dev, ncam, nptr));
+  MPN_TRY(scc_stage(c, act, nullptr));
+  MPN_CUDA_OK(cudaMemsetAsync(c.groots, 0, sizeof(int) * G, c.st));
+  graph_labels_kernel<<<list_grid(c.g.n_nodes), 256, 0, c.st>>>(c.g.n_nodes, c.label, c.g.node_gid, c.g.graph_nptr, labels, c.groots);
+  MPN_LAUNCH_OK();
+  MPN_CUDA_OK(cudaMemcpyAsync(n_components, c.groots, sizeof(int) * G, cudaMemcpyDeviceToHost, c.st));
   MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  if (n_components) *n_components = nc;
-  if (prune_changed) *prune_changed = ch;
   return MPN_OK;
 }
 
@@ -1346,6 +1857,19 @@ int mpn_labels_reference(const mpn_graph* g, const uint8_t* act, int64_t* labels
   MPN_TRY(labels_reference_parallel(c, act, (long long*)labels_out_host, &nc));
   if (n_components) *n_components = nc;
   return MPN_OK;
+}
+
+int mpn_labels_reference_batched(const mpn_graph* g, const uint8_t* act, int64_t* labels_out_host, int32_t* n_components_host, void* ws,
+                                 size_t ws_bytes, void* stream) {
+  PostCtx c;
+  MPN_REQUIRE(labels_out_host && n_components_host, "labels_reference_batched: NULL output");
+  MPN_TRY(post_begin(c, g, act, ws, ws_bytes, stream));
+  MPN_REQUIRE((long long)c.n_active < (1ll << 30), "labels_reference_batched: more than 2^30 active edges");
+  if (g->n_graphs <= 1) return labels_reference_parallel(c, act, (long long*)labels_out_host, n_components_host);
+  MPN_REQUIRE(g->graph_nptr, "labels_reference_batched: batched graph without graph_nptr");
+  std::vector<int> nptr;
+  MPN_TRY(copy_graph_ptr(c, nptr));
+  return labels_reference_batched(c, act, nptr, (long long*)labels_out_host, n_components_host);
 }
 
 int mpn_labels_reference_host(const int32_t* src, const int32_t* dst, int64_t n_active, int32_t n_nodes, int64_t* labels_out,

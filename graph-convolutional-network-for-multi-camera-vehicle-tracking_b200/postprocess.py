@@ -60,21 +60,27 @@ class _Post:
             act = out
         return act.to(like.dtype)
 
+    def caller_order_active(self):
+        """(src, dst) int64 device tensors of the active edges in the CALLER's edge order (graphs with a ``perm``)."""
+        g = self.g
+        orig = torch.empty_like(self.act)
+        orig[g.perm] = self.act
+        idx = torch.nonzero(orig, as_tuple=False).reshape(-1)
+        ei = g._keepalive                                      # sorted copy
+        inv = torch.empty_like(g.perm)
+        inv[g.perm] = torch.arange(g.perm.numel(), device=self.dev)
+        sel = inv[idx]
+        return ei[0, sel], ei[1, sel]
+
     def labels_reference(self):
         """ID_pred exactly as compute_SCC_and_Clusters numbers it (utils.py:30-52): int64 CPU tensor."""
         g = self.g
         act = self.act
         if g.perm is not None:
             # the reference scans active edges in the CALLER's edge order: compact in that order
-            orig = torch.empty_like(act)
-            orig[g.perm] = act
-            idx = torch.nonzero(orig, as_tuple=False).reshape(-1)
-            ei = g._keepalive                                  # sorted copy
-            inv = torch.empty_like(g.perm)
-            inv[g.perm] = torch.arange(g.perm.numel(), device=self.dev)
-            sel = inv[idx]
-            s_h, d_h = ei[0, sel].to(torch.int32).cpu(), ei[1, sel].to(torch.int32).cpu()
-            n = int(idx.numel())
+            s, d = self.caller_order_active()
+            s_h, d_h = s.to(torch.int32).cpu(), d.to(torch.int32).cpu()
+            n = int(s.numel())
         else:
             # sorted graphs: partition + first-appearance keys on the device, the rank over the components on the host
             labels = torch.empty(g.n_nodes, dtype=torch.int64)
@@ -88,6 +94,36 @@ class _Post:
         _lib.check(self.lib.mpn_labels_reference_host(s_h.data_ptr(), d_h.data_ptr(), n, g.n_nodes, labels.data_ptr(),
                                                       C.byref(ncomp)))
         return labels, int(ncomp.value)
+
+    def labels_reference_batched(self):
+        """The reference numbering of each graph of a batch, each numbered from 0: (int64 CPU [N], int64 CPU [G] counts)."""
+        g = self.g
+        if g.n_graphs <= 1:
+            labels, n = self.labels_reference()
+            return labels, torch.tensor([n], dtype=torch.int64)
+        labels = torch.empty(g.n_nodes, dtype=torch.int64)
+        counts = torch.empty(g.n_graphs, dtype=torch.int32)
+        if g.perm is None:
+            with torch.cuda.device(self.dev):
+                _lib.check(self.lib.mpn_labels_reference_batched(g.ref, self.act.data_ptr(), labels.data_ptr(), counts.data_ptr(),
+                                                                 self.ws.data_ptr(), self.ws.numel(), self.stream))
+            return labels, counts.long()
+        # unsorted batch: each graph's active edges in the caller's order, numbered on the host graph by graph
+        s, d = self.caller_order_active()
+        gid = g.node_gid[s].long()
+        order = torch.sort(gid, stable=True).indices
+        n0 = g.graph_nptr.long()[gid[order]]
+        s_h = (s[order] - n0).to(torch.int32).cpu()
+        d_h = (d[order] - n0).to(torch.int32).cpu()
+        e_ptr = [0] + torch.bincount(gid, minlength=g.n_graphs).cumsum(0).tolist()
+        nptr = g.graph_nptr.tolist()
+        nc = C.c_int32(0)
+        for k in range(g.n_graphs):
+            e0, e1 = e_ptr[k], e_ptr[k + 1]
+            _lib.check(self.lib.mpn_labels_reference_host(s_h[e0:].data_ptr(), d_h[e0:].data_ptr(), e1 - e0, nptr[k + 1] - nptr[k],
+                                                          labels[nptr[k]:].data_ptr(), C.byref(nc)))
+            counts[k] = nc.value
+        return labels, counts.long()
 
     def labels_canonical(self):
         lab = torch.empty(self.g.n_nodes, dtype=torch.int32, device=self.dev)
@@ -153,12 +189,14 @@ def splitting(ID_pred, predictions, preds_prob, edge_list, data_batch, predicted
 
 
 def split_stats():
-    """SPLITTING of this thread's last ``splitting`` / ``post_processing`` call (mpn_split_last_stats): dict with the number of active
-    edges that carried a tied probability value, rounds / dropped values, off-lowest steps and the mode that ran."""
+    """SPLITTING of this thread's last ``splitting`` / ``post_processing`` / ``post_processing_batched`` call (mpn_split_last_stats):
+    dict with the number of active edges that carried a tied probability value, rounds / dropped values, off-lowest steps, the mode
+    that ran and ``host_order_graphs``, the number of graphs that took the reference order on the host (0 or 1 for one graph).
+    After a batched call the counts are summed over the graphs."""
     out = (C.c_int64 * 4)()
     _lib.lib().mpn_split_last_stats(C.cast(out, C.c_void_p))
     return {"tied_edges": int(out[0]), "rounds": int(out[1]), "off_lowest_steps": int(out[2]),
-            "mode": "reference_order_host" if out[3] else "device_rounds"}
+            "mode": "reference_order_host" if out[3] else "device_rounds", "host_order_graphs": int(out[3])}
 
 
 def post_processing(num_cameras, ID_pred, predicted_active_edges, predictions, edge_list, CONFIG, data, preds_prob,
@@ -200,3 +238,81 @@ def post_processing(num_cameras, ID_pred, predicted_active_edges, predictions, e
     if verbose:
         print('# CC = ' + str(n))
     return ID, new_pred
+
+
+def _graph_count(data):
+    """Number of graphs the batch carries, read without touching the device: a cached ``data.mpn_graph`` or ``data.ptr``."""
+    pre = getattr(data, "mpn_graph", None)
+    if pre is not None:
+        return int(pre.n_graphs)
+    ptr = getattr(data, "ptr", None)
+    return 1 if ptr is None else int(ptr.numel()) - 1
+
+
+def _cameras_per_graph(num_cameras, n_graphs):
+    """``num_cameras`` as a list of n_graphs ints >= 1: one int for every graph, or one per graph (sequence / 1-D array / tensor)."""
+    if isinstance(num_cameras, torch.Tensor):
+        if num_cameras.dim() > 1:
+            raise ValueError("num_cameras must be an int or a 1-D sequence with one entry per graph")
+        vals = num_cameras.detach().cpu().reshape(-1).tolist() if num_cameras.dim() == 1 else [num_cameras.item()] * n_graphs
+    elif isinstance(num_cameras, (int, np.integer)) and not isinstance(num_cameras, bool):
+        vals = [int(num_cameras)] * n_graphs
+    else:
+        try:
+            vals = np.asarray(num_cameras).reshape(-1).tolist() if np.ndim(num_cameras) == 1 else None
+        except (TypeError, ValueError):
+            vals = None
+        if vals is None:
+            raise ValueError("num_cameras must be an int or a 1-D sequence with one entry per graph")
+    if len(vals) != n_graphs:
+        raise ValueError("num_cameras has %d entries for a batch of %d graphs" % (len(vals), n_graphs))
+    out = []
+    for v in vals:
+        try:
+            ok = not isinstance(v, bool) and float(v).is_integer() and 1 <= v < 2 ** 31
+        except (TypeError, ValueError):
+            ok = False
+        if not ok:
+            raise ValueError("every num_cameras entry must be an integer >= 1, got %r" % (v,))
+        out.append(int(v))
+    return out
+
+
+def post_processing_batched(num_cameras, predictions, CONFIG, data, preds_prob, numbering='reference', verbose=False):
+    """``post_processing`` for every graph of a batch in one call (new; the reference loops over graphs, inference.py:475-497).
+
+    ``data`` carries the batch as the batched forward takes it: ``data.ptr`` (G+1 node offsets) or a cached ``data.mpn_graph``;
+    ``predictions`` [E] (uint8 / int64) and ``preds_prob`` ([E,2] softmax or [E] prob1) as ``post_processing`` takes them, e.g.
+    ``MOTMPNet.last_pred`` / ``last_prob1`` of a batched forward with ``fuse_decisions=True``.  ``num_cameras``: an int for every
+    graph or one int >= 1 per graph.  ``CONFIG`` is fixed up in place as in ``post_processing``.
+
+    Returns (ID_pred int64 CPU [N], predictions (a new device tensor, the caller's dtype and shape), n_components int64 CPU [G]).
+    For every graph g the slices ``ID_pred[ptr[g]:ptr[g+1]]`` (numbered from 0) and ``predictions`` of its edges equal what
+    ``post_processing(num_cameras[g], ...)`` returns for that graph alone; with all three flags off, ID_pred holds each graph's SCC
+    labels of the active edges.  ``split_stats()`` sums over the graphs and reports ``host_order_graphs``.
+    """
+    if numbering not in ('reference', 'canonical'):
+        raise ValueError("numbering must be 'reference' or 'canonical'")
+    n_graphs = _graph_count(data)
+    cams = _cameras_per_graph(num_cameras, n_graphs)
+    for k in ('CUTTING', 'PRUNING', 'SPLITTING'):
+        CONFIG[k] = _as_bool(CONFIG[k])                       # same in-place fix-up as inference.py:75-91
+    flags = (_lib.POST_CUT if CONFIG['CUTTING'] else 0) | (_lib.POST_PRUNE if CONFIG['PRUNING'] else 0) | \
+            (_lib.POST_SPLIT if CONFIG['SPLITTING'] else 0)
+    p = _Post(data, predictions, preds_prob)
+    if p.g.n_graphs != n_graphs:
+        raise ValueError("data.ptr describes %d graphs, its cached graph tables %d" % (n_graphs, p.g.n_graphs))
+    ncam = torch.tensor(cams, dtype=torch.int32).to(p.dev)
+    lab = torch.empty(p.g.n_nodes, dtype=torch.int32, device=p.dev)
+    ncomp = torch.empty(max(1, n_graphs), dtype=torch.int32)
+    with torch.cuda.device(p.dev):
+        _lib.check(p.lib.mpn_post_processing_batched(p.g.ref, p.act.data_ptr(), p.prob_ptr, p.prob_stride, ncam.data_ptr(), flags,
+                                                     lab.data_ptr(), ncomp.data_ptr(), p.ws.data_ptr(), p.ws.numel(), p.stream))
+    new_pred = p.predictions(predictions).reshape(predictions.shape)
+    if numbering == 'reference':
+        ID, n = p.labels_reference_batched()
+    else:
+        ID, n = lab.cpu().long(), ncomp.long()
+    if verbose:
+        print('# CC = ' + ' '.join(str(v) for v in n.tolist()))
+    return ID, new_pred, n

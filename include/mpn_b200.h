@@ -362,13 +362,27 @@ int mpn_split(const mpn_graph* g, uint8_t* act_dev, const float* prob1_dev, int3
 /* SPLITTING of the calling thread's last mpn_split / mpn_post_processing: out[0] = active edges carrying a probability value
  * that is tied with an edge touching an oversized cluster (-1: not counted, every active edge went to the host),
  * out[1] = rounds (device) or dropped values (host order), out[2] = host-order steps taken on a label other than the lowest
- * oversized one (utils.py:112), out[3] = 0 device rounds | 1 reference order on the host. */
+ * oversized one (utils.py:112), out[3] = 0 device rounds | 1 reference order on the host.  After mpn_post_processing_batched:
+ * out[0] and out[2] summed over the graphs, out[1] = device rounds + the dropped values of the host-order graphs, out[3] = the
+ * number of graphs that took the reference order on the host. */
 void mpn_split_last_stats(int64_t out_host[4]);
 int mpn_scc_labels(const mpn_graph* g, const uint8_t* act_dev, int32_t* labels_dev, int32_t* n_components_host,
                    void* workspace_dev, size_t workspace_bytes, void* stream);
 int mpn_post_processing(const mpn_graph* g, uint8_t* act_dev, const float* prob1_dev, int32_t prob_stride,
                         int32_t num_cameras, int32_t flags, int32_t* labels_dev, int32_t* n_components_host,
                         int32_t* prune_changed_host, void* workspace_dev, size_t workspace_bytes, void* stream);
+/* inference.post_processing (inference.py:70-169, utils.py:30-52, 54-123, 125-142, 144-339) for EACH graph of a batched graph
+ * (n_graphs > 1, node_gid / graph_nptr set) in one call, with the result a single-graph mpn_post_processing gives on every graph
+ * alone.  num_cameras_dev: dev int32 [n_graphs], the camera count of each graph (PRUNE bounds degrees by num_cameras[g] - 1,
+ * SPLIT cluster sizes by num_cameras[g]).  SPLITTING removes the edges of THE SAME graph whose probability equals a dropped
+ * minimum (utils.py:96-98): its sets are keyed by (graph, value), and the mode (device rounds / reference order on the host) is
+ * chosen per graph; mpn_split_last_stats then sums the counts over the graphs and out[3] is the number of graphs that took the
+ * reference order.  labels_dev (optional): dev int32 [n_nodes], canonical graph-local labels (smallest node id of the SCC minus
+ * the graph's first node); n_components_host: HOST int32 [n_graphs].  n_graphs <= 1: same as mpn_post_processing with
+ * num_cameras_dev[0].  The workspace is mpn_post_workspace_bytes(g) (larger for n_graphs > 1).  Synchronises. */
+int mpn_post_processing_batched(const mpn_graph* g, uint8_t* act_dev, const float* prob1_dev, int32_t prob_stride,
+                                const int32_t* num_cameras_dev, int32_t flags, int32_t* labels_dev, int32_t* n_components_host,
+                                void* workspace_dev, size_t workspace_bytes, void* stream);
 /* Active edges in edge order as (src, dst) int32 pairs, for the reference label numbering.
  * n_active_host receives the count; src_out/dst_out dev [capacity].  Synchronises. */
 int mpn_active_edges(const mpn_graph* g, const uint8_t* act_dev, int32_t* src_out_dev, int32_t* dst_out_dev,
@@ -399,6 +413,11 @@ int mpn_clear_inactive(uint8_t* act_dev, const int32_t* eid_dev, const uint8_t* 
  * labels_out_host: HOST int64 [n_nodes].  Synchronises. */
 int mpn_labels_reference(const mpn_graph* g, const uint8_t* act_dev, int64_t* labels_out_host, int32_t* n_components_host,
                          void* workspace_dev, size_t workspace_bytes, void* stream);
+/* The same numbering (utils.py:30-52) for each graph of a batched (row, col)-sorted graph: labels_out_host HOST int64 [n_nodes]
+ * numbered from 0 within every graph, exactly as mpn_labels_reference numbers that graph alone; n_components_host HOST int32
+ * [n_graphs].  n_graphs <= 1: same as mpn_labels_reference.  Synchronises. */
+int mpn_labels_reference_batched(const mpn_graph* g, const uint8_t* act_dev, int64_t* labels_out_host, int32_t* n_components_host,
+                                 void* workspace_dev, size_t workspace_bytes, void* stream);
 int mpn_labels_reference_host(const int32_t* src_host, const int32_t* dst_host, int64_t n_active, int32_t n_nodes,
                               int64_t* labels_out_host, int32_t* n_components_host);
 /* Host-side SPLITTING in the reference's own order (utils.py:54-123): one oversized cluster at a time — the lowest label of the
