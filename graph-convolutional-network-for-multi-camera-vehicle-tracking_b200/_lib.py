@@ -87,6 +87,9 @@ _PROTOS = {
     "mpn_cross_camera_edges": (C.c_int64, [C.c_void_p, C.c_int32]),
     "mpn_cross_camera_block_edges": (C.c_int64, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32]),
     "mpn_graph_build_cross_camera": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
+    "mpn_cross_camera_batched_layout": (C.c_int64, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
+    "mpn_graph_build_cross_camera_batched": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                                       C.c_void_p, C.c_void_p]),
     "mpn_profile_gram": (C.c_int, [C.c_int]),
     "mpn_profile_gram_ms": (C.c_float, []),
     "mpn_shared_gram_mode": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
@@ -160,6 +163,8 @@ _PROTOS = {
     "mpn_edge_labels": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_void_p, C.c_void_p]),
     "mpn_normalize_columns_workspace_bytes": (C.c_size_t, [C.c_int32]),
     "mpn_normalize_columns": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpn_normalize_columns_batched": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                                C.c_size_t, C.c_void_p]),
     "mpn_gemm_nt_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32, C.c_int]),
     "mpn_gram_nt": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t,
                               C.c_void_p]),

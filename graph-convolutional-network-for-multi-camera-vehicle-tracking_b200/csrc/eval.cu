@@ -323,6 +323,7 @@ int mpn_write_mtmc_txt_host(const char* path, const int64_t* table_host, int64_t
 //                           an O(E*N) Python comprehension in the reference), float32, graph edge order
 //   mpn_normalize_columns   F.normalize(node_embeds, p=2, dim=0) (inference.py:403-404): every FEATURE COLUMN is scaled to unit
 //                           L2 norm over the nodes, eps 1e-12.  Sum of squares in fp64, then one scaling pass.
+//   mpn_normalize_columns_batched   the same for every graph of a batch on its own (inference.py:403-404 per graph), one kernel.
 // ================================================================================================
 namespace mpn {
 
@@ -372,6 +373,37 @@ __global__ void colnorm_apply_kernel(const float* __restrict__ x, long long tota
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) out[i] = x[i] / norm[i % D];
 }
 
+
+// mpn_normalize_columns_batched: F.normalize(dim=0) of every graph of a batch alone.  One CTA per (graph, slab of sw columns);
+// thread (ry, cx) sums the squares of column cx over the graph's rows ry, ry + 256/sw, ... in fp64, then the 256/sw partials are
+// added in order (deterministic).  Pass 2 re-reads the slab, which is still in L2 (300 rows x 32 columns = 38 KB at S02 size), and
+// writes it scaled.  A CTA writes only the slab it has finished summing, so out may alias x (no __restrict__).
+__global__ void __launch_bounds__(256) colnorm_graph_kernel(const float* x, int D, const int* __restrict__ graph_nptr, int sw,
+                                                            float* out) {
+  __shared__ double part[256];
+  __shared__ float nrm[32];
+  const int cx = threadIdx.x % sw, ry = threadIdx.x / sw, nry = 256 / sw;
+  const int col = blockIdx.y * sw + cx;
+  const int r0 = graph_nptr[blockIdx.x], r1 = graph_nptr[blockIdx.x + 1];
+  double s = 0.0;
+  if (col < D) {
+#pragma unroll 4
+    for (int r = r0 + ry; r < r1; r += nry) { const double v = x[(size_t)r * D + col]; s += v * v; }
+  }
+  part[threadIdx.x] = s;
+  __syncthreads();
+  if (ry == 0) {
+    for (int i = 1; i < nry; ++i) s += part[i * sw + cx];
+    nrm[cx] = fmaxf((float)sqrt(s), 1e-12f);                       // F.normalize: v / max(||v||_2, eps)
+  }
+  __syncthreads();
+  if (col < D) {
+    const float q = nrm[cx];
+#pragma unroll 4
+    for (int r = r0 + ry; r < r1; r += nry) out[(size_t)r * D + col] = x[(size_t)r * D + col] / q;
+  }
+}
+
 }  // namespace mpn
 
 extern "C" {
@@ -401,6 +433,21 @@ int mpn_normalize_columns(const float* x_dev, int32_t n, int32_t D, float* out_d
   MPN_LAUNCH_OK();
   const long long total = (long long)n * D;
   colnorm_apply_kernel<<<grid_for(total), 256, 0, st>>>(x_dev, total, D, norm, out_dev);
+  MPN_LAUNCH_OK();
+  return MPN_OK;
+}
+
+int mpn_normalize_columns_batched(const float* x_dev, int32_t n, int32_t D, const int32_t* graph_nptr_dev, int32_t n_graphs,
+                                  float* out_dev, void* ws, size_t ws_bytes, void* stream) {
+  if (n_graphs <= 1) return mpn_normalize_columns(x_dev, n, D, out_dev, ws, ws_bytes, stream);
+  MPN_REQUIRE(n > 0 && D > 0, "normalize_columns_batched: bad argument");
+  MPN_REQUIRE(x_dev && out_dev && graph_nptr_dev, "normalize_columns_batched: NULL argument");
+  MPN_REQUIRE(div_up(D, 8) <= 65535, "normalize_columns_batched: D must be <= 524280");
+  // 32-column slabs (one 128-byte line per warp row); a batch of few graphs gets narrower slabs so that about one wave of
+  // CTAs (8 per SM) is in flight
+  int sw = 32;
+  while (sw > 8 && (long long)n_graphs * div_up(D, sw) < kNumSMs * 8) sw >>= 1;
+  colnorm_graph_kernel<<<dim3(n_graphs, div_up(D, sw)), 256, 0, (cudaStream_t)stream>>>(x_dev, D, graph_nptr_dev, sw, out_dev);
   MPN_LAUNCH_OK();
   return MPN_OK;
 }

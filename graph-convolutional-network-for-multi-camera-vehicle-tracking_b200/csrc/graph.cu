@@ -1,4 +1,5 @@
-// K0: int32 CSR + task tables from the reference's edge_index (models/mpn.py:44 `row, col = edge_index`).
+// K0: int32 CSR + task tables from the reference's edge_index (models/mpn.py:44 `row, col = edge_index`), or built on the device
+// from the camera layout of one graph or of a batch (inference.py:407-414).
 #include <stdarg.h>
 #include <stdlib.h>
 
@@ -184,6 +185,19 @@ struct CamLayout {
   long long ebase[MPN_MAX_CAMERAS + 1];    // first edge of each camera's row block
 };
 
+// One warp writes the columns of global row r: [c0, c0 + deg + nk) without the row's own camera segment [lo, lo + nk), in
+// ascending order from local edge le0 on (coalesced, no per-edge division).  The reference's int64 pair goes to edge_index_out
+// ([2,E]) when that is not NULL.
+__device__ __forceinline__ void cross_camera_row_cols(int lane, long long r, int c0, int deg, int lo, int nk, long long le0,
+                                                      long long E, int* __restrict__ col32, long long* __restrict__ edge_index_out) {
+  for (int idx = lane; idx < deg; idx += 32) {
+    int c = c0 + idx;
+    if (c >= lo) c += nk;
+    col32[le0 + idx] = c;
+    if (edge_index_out) { edge_index_out[le0 + idx] = r; edge_index_out[E + le0 + idx] = c; }
+  }
+}
+
 // dense cross-camera graph straight from the camera layout: row r (camera k) lists every node outside [ptr[k], ptr[k+1]).
 // Works on a row block [row0, row0 + n_rows): local edge e corresponds to global edge e + gbase.
 __global__ void __launch_bounds__(256) cross_camera_kernel(const CamLayout L, int n_total, int row0, int n_rows, long long gbase,
@@ -200,8 +214,7 @@ __global__ void __launch_bounds__(256) cross_camera_kernel(const CamLayout L, in
     const long long deg = n_total - (L.ptr[k + 1] - L.ptr[k]);
     rowptr[lr] = (int)(L.ebase[k] + (r - L.ptr[k]) * deg - gbase);
   }
-  // one warp per local row: its columns are 0..n_total-1 without the row's own camera block, written in order (coalesced,
-  // no per-edge division)
+  // one warp per local row: its columns are 0..n_total-1 without the row's own camera block
   const int lane = threadIdx.x & 31;
   const long long warp0 = tid >> 5, nwarps = stride >> 5;
   for (long long lr = warp0; lr < n_rows; lr += nwarps) {
@@ -210,12 +223,47 @@ __global__ void __launch_bounds__(256) cross_camera_kernel(const CamLayout L, in
     while (k + 1 < L.n_cams && r >= L.ptr[k + 1]) ++k;
     const int lo = L.ptr[k], nk = L.ptr[k + 1] - lo;
     const int deg = n_total - nk;
-    const long long le0 = L.ebase[k] + (r - lo) * (long long)deg - gbase;
-    for (int idx = lane; idx < deg; idx += 32) {
-      const int c = idx < lo ? idx : idx + nk;
-      col32[le0 + idx] = c;
-      if (edge_index_out) { edge_index_out[le0 + idx] = r; edge_index_out[E + le0 + idx] = c; }
+    cross_camera_row_cols(lane, r, 0, deg, lo, nk, L.ebase[k] + (r - lo) * (long long)deg - gbase, E, col32, edge_index_out);
+  }
+}
+
+// last i in [0, n) with a[i] <= v (a ascending, a[0] <= v)
+__device__ __forceinline__ int last_le(const int* __restrict__ a, int n, long long v) {
+  int lo = 0, hi = n - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (a[mid] <= v) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// Block-diagonal cross-camera tables of a batch: row r of graph g = [gs, ge) in camera segment [ss, se) lists [gs, ss) and
+// [se, ge).  Segment s = (graph, camera) starts at node seg_ptr[s] and its row block at edge seg_ebase[s]; graph g owns
+// segments [graph_seg[g], graph_seg[g+1]).  One warp per row finds its segment and graph (binary searches that every lane makes
+// on the same words), writes rowptr / node_gid (and graph_nptr on a graph's first row), then the row's columns.
+__global__ void __launch_bounds__(256) cross_camera_batched_kernel(const int* __restrict__ seg_ptr, int n_segs,
+                                                                   const int* __restrict__ graph_seg, int n_graphs,
+                                                                   const long long* __restrict__ seg_ebase, int n, long long E,
+                                                                   int* __restrict__ rowptr, int* __restrict__ col32,
+                                                                   int* __restrict__ node_gid, int* __restrict__ graph_nptr,
+                                                                   long long* __restrict__ edge_index_out) {
+  pdl_wait();
+  const int lane = threadIdx.x & 31;
+  const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+  for (long long r = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n; r += nwarps) {
+    const int s = last_le(seg_ptr, n_segs, r);
+    const int g = last_le(graph_seg, n_graphs, s);
+    const int gs = seg_ptr[graph_seg[g]], ge = seg_ptr[graph_seg[g + 1]];
+    const int ss = seg_ptr[s], nk = seg_ptr[s + 1] - ss;
+    const int deg = ge - gs - nk;
+    const long long le0 = seg_ebase[s] + (r - ss) * (long long)deg;
+    if (lane == 0) {
+      rowptr[r] = (int)le0;
+      node_gid[r] = g;
+      if (r == gs) graph_nptr[g] = gs;
+      if (r == n - 1) { rowptr[n] = (int)E; graph_nptr[n_graphs] = n; }
     }
+    cross_camera_row_cols(lane, r, gs, deg, ss, nk, le0, E, col32, edge_index_out);
   }
 }
 
@@ -284,6 +332,51 @@ int mpn_graph_build_cross_camera(mpn_graph* g, const int32_t* cam_ptr, int32_t n
   mpn::launch(task_fill, min(kNumSMs * 8, div_up(g->n_nodes, 256)), 256, 0, st, g->taskptr, g->n_nodes, g->max_tasks, g->task_row);
   MPN_LAUNCH_OK();
   g->layout_hint = MPN_LAYOUT_ONE_GAP;         // every row: all nodes but its own camera's range
+  return MPN_OK;
+}
+
+int64_t mpn_cross_camera_batched_layout(const int32_t* seg_ptr, int32_t n_segs, const int32_t* graph_seg, int32_t n_graphs,
+                                        int64_t* seg_ebase) {
+  if (!seg_ptr || !graph_seg || n_segs < 1 || n_graphs < 1) return -1;
+  if (seg_ptr[0] != 0 || graph_seg[0] != 0 || graph_seg[n_graphs] != n_segs) return -1;
+  for (int s = 0; s < n_segs; ++s)
+    if (seg_ptr[s + 1] <= seg_ptr[s]) return -1;
+  long long e = 0;
+  for (int g = 0; g < n_graphs; ++g) {
+    const int s0 = graph_seg[g], s1 = graph_seg[g + 1];
+    if (s1 <= s0) return -1;
+    const long long ng = (long long)seg_ptr[s1] - seg_ptr[s0];
+    for (int s = s0; s < s1; ++s) {
+      const long long nk = (long long)seg_ptr[s + 1] - seg_ptr[s];
+      if (seg_ebase) seg_ebase[s] = e;
+      e += nk * (ng - nk);
+    }
+  }
+  if (seg_ebase) seg_ebase[n_segs] = e;
+  return e;
+}
+
+int mpn_graph_build_cross_camera_batched(mpn_graph* g, const int32_t* seg_ptr, int32_t n_segs, const int32_t* graph_seg,
+                                         const int64_t* seg_ebase, int64_t* edge_index_out, void* stream) {
+  using namespace mpn;
+  MPN_REQUIRE(g && seg_ptr && graph_seg && seg_ebase, "cross_camera_batched: NULL argument");
+  MPN_REQUIRE(n_segs >= 1 && g->n_graphs >= 1 && n_segs >= g->n_graphs, "cross_camera_batched: need n_segs >= n_graphs >= 1");
+  MPN_REQUIRE(g->n_nodes > 0 && g->n_cols == g->n_nodes && g->row_offset == 0, "cross_camera_batched: batched graphs cannot be row-sharded");
+  MPN_REQUIRE(g->n_edges >= 0 && g->n_edges < (1ll << 31), "n_edges must be < 2^31");
+  MPN_REQUIRE(g->chunk >= 32 && g->chunk <= 4096 && (g->chunk & (g->chunk - 1)) == 0, "chunk must be a power of two in [32,4096]");
+  MPN_REQUIRE(g->max_tasks >= g->n_edges / g->chunk + g->n_nodes, "max_tasks too small (need E/chunk + N)");
+  MPN_REQUIRE(g->rowptr && g->taskptr && g->task_row && g->n_tasks && (g->col || g->n_edges == 0) && g->node_gid && g->graph_nptr,
+              "graph table pointer is NULL");
+  cudaStream_t st = (cudaStream_t)stream;
+  mpn::launch(cross_camera_batched_kernel, min(kNumSMs * 16, div_up((long long)g->n_nodes * 32, 256)), 256, 0, st,
+              seg_ptr, n_segs, graph_seg, g->n_graphs, (const long long*)seg_ebase, g->n_nodes, (long long)g->n_edges, g->rowptr,
+              g->col, g->node_gid, g->graph_nptr, (long long*)edge_index_out);
+  MPN_LAUNCH_OK();
+  mpn::launch(task_scan, 1, 1024, 0, st, g->rowptr, g->n_nodes, g->chunk, g->taskptr, g->n_tasks);
+  MPN_LAUNCH_OK();
+  mpn::launch(task_fill, min(kNumSMs * 8, div_up(g->n_nodes, 256)), 256, 0, st, g->taskptr, g->n_nodes, g->max_tasks, g->task_row);
+  MPN_LAUNCH_OK();
+  g->layout_hint = MPN_LAYOUT_UNKNOWN;         // a row lists its own graph's columns only, not all columns but one gap
   return MPN_OK;
 }
 

@@ -98,6 +98,19 @@ def choose_chunk(n_edges: int) -> int:
     return chunk
 
 
+def host_node_ptr(ptr, n_nodes: int):
+    """The G+1 node offsets of a batch (PyG ``Batch.ptr``: host sequence, numpy array or tensor; a CUDA tensor is copied to the
+    host once) as an int64 numpy array, checked to run strictly increasing from 0 to ``n_nodes``."""
+    import numpy as np
+    p = np.asarray(ptr.detach().cpu() if isinstance(ptr, torch.Tensor) else ptr)
+    if p.ndim != 1 or p.size < 2 or not np.issubdtype(p.dtype, np.integer):
+        raise ValueError("ptr must be strictly increasing from 0 to num_nodes")
+    p = p.astype(np.int64)
+    if p[0] != 0 or p[-1] != n_nodes or np.any(p[1:] <= p[:-1]):
+        raise ValueError("ptr must be strictly increasing from 0 to num_nodes")
+    return p
+
+
 class TrackletGraph:
     """CSR + task tables on the device.  ``perm`` is None when the caller's edge order is already (row, col)-sorted,
     otherwise ``sorted_edge = original_edge[perm]``."""
@@ -222,15 +235,25 @@ class TrackletGraph:
         return self
 
     @classmethod
-    def from_cameras(cls, cam_ids, device, chunk: int = None, materialize_edge_index: bool = False, row_block=None):
+    def from_cameras(cls, cam_ids, device, chunk: int = None, materialize_edge_index: bool = False, row_block=None, ptr=None):
         """Dense cross-camera graph built on the device from the per-node camera ids (inference.py:407-414), without
         the int64 edge_index ever crossing PCIe or being read: 4 B/edge written instead of 16 B read + 4 B written.
         ``cam_ids``: host sequence / array / CPU tensor, nodes grouped by camera in ascending camera order
         (dataset.py:279-281).  ``materialize_edge_index`` also writes the reference's int64 [2,E] tensor (``.edge_index``).
         ``row_block=(n0, n1)`` builds only the rows of one shard (column ids stay global).
+        ``ptr``: G+1 node offsets of a batch of graphs (PyG ``Batch.ptr``); with G > 1 every graph gets its own dense
+        cross-camera rows (the per-graph edge_index offset by ptr[g], concatenated) and per-graph BatchNorm statistics, as
+        ``TrackletGraph(edge_index, N, ptr=ptr)``; cameras are grouped in ascending order within each graph.  Does not
+        synchronise (a CUDA ``ptr`` is read on the host once).
         """
         import numpy as np
         cam = np.asarray(cam_ids.cpu() if isinstance(cam_ids, torch.Tensor) else cam_ids).reshape(-1)
+        if ptr is not None:
+            nptr = host_node_ptr(ptr, cam.size)
+            if nptr.size > 2:
+                if row_block is not None:
+                    raise ValueError("batched graphs cannot be row-sharded")
+                return cls._from_cameras_batched(cam, nptr, device, chunk, materialize_edge_index)
         if cam.size < 2 or np.any(cam[1:] < cam[:-1]):
             raise ValueError("from_cameras needs nodes grouped by ascending camera id (as the reference dataset orders them)")
         starts = np.flatnonzero(np.r_[True, cam[1:] != cam[:-1]])
@@ -258,6 +281,66 @@ class TrackletGraph:
                                                       self.edge_index.data_ptr() if materialize_edge_index else None,
                                                       current_stream_ptr(dev)))
         self._keepalive = self.edge_index
+        return self
+
+    @classmethod
+    def _from_cameras_batched(cls, cam, nptr, device, chunk, materialize_edge_index):
+        import numpy as np
+        n, n_graphs = int(cam.size), int(nptr.size - 1)
+        first = np.zeros(n, dtype=bool)
+        first[nptr[:-1]] = True                                   # first node of every graph
+        if np.any((cam[1:] < cam[:-1]) & ~first[1:]):
+            raise ValueError("from_cameras needs nodes grouped by ascending camera id within every graph (as the reference "
+                             "dataset orders them)")
+        # one segment per (graph, camera); layout = [seg_ebase int64 [S+1] | seg_ptr [S+1] | graph_seg [G+1]] (int32 words)
+        starts = np.flatnonzero(first | np.r_[True, cam[1:] != cam[:-1]])
+        n_segs = int(starts.size)
+        n_ints = 2 * (n_segs + 1) + (n_segs + 1) + (n_graphs + 1)
+        host = np.empty(n_ints, dtype=np.int32)
+        seg_ebase = host[:2 * (n_segs + 1)].view(np.int64)
+        seg_ptr = host[2 * (n_segs + 1):3 * (n_segs + 1)]
+        graph_seg = host[3 * (n_segs + 1):]
+        seg_ptr[:-1], seg_ptr[-1] = starts, n
+        graph_seg[:] = np.searchsorted(starts, nptr)
+        L = _lib.lib()
+        E = int(L.mpn_cross_camera_batched_layout(seg_ptr.ctypes.data, n_segs, graph_seg.ctypes.data, n_graphs,
+                                                  seg_ebase.ctypes.data))
+        if E < 0:
+            raise ValueError("malformed camera layout")
+        e_per_graph = seg_ebase[graph_seg[1:]] - seg_ebase[graph_seg[:-1]]
+        n_per_graph = nptr[1:] - nptr[:-1]
+        if int(e_per_graph.min()) < 2 or int(n_per_graph.min()) < 2:
+            raise ValueError("every graph of a batch needs at least 2 nodes and 2 edges (BatchNorm over one value "
+                             "raises in the reference)")
+        if E >= (1 << 31):
+            raise ValueError("a batch of cross-camera graphs needs fewer than 2^31 edges (%d)" % E)
+        dev = torch.device(device)
+        _lib.require_device(dev.index if dev.index is not None else torch.cuda.current_device())
+        self = object.__new__(cls)
+        self.device, self.n_cols, self.n_nodes, self.row_offset, self.n_edges = dev, n, n, 0, E
+        self.chunk = int(chunk or choose_chunk(E))
+        self.max_tasks = E // self.chunk + n
+        ptrs = self._alloc_tables(dev)
+        self.perm = None
+        self.n_graphs, self.max_graph_nodes = n_graphs, int(n_per_graph.max())
+        # node_gid [N] | graph_nptr [G+1] | layout, in one allocation; the layout arrives in ONE copy from pinned memory
+        o_nptr = (n + 3) & ~3
+        o_lay = o_nptr + ((n_graphs + 1 + 3) & ~3)
+        aux = torch.empty(o_lay + n_ints, dtype=torch.int32, device=dev)
+        pinned = torch.empty(n_ints, dtype=torch.int32, pin_memory=True)
+        pinned.numpy()[:] = host
+        aux[o_lay:].copy_(pinned, non_blocking=True)
+        self.node_gid, self.graph_nptr = aux[:n], aux[o_nptr:o_nptr + n_graphs + 1]
+        base = aux.data_ptr() + 4 * o_lay
+        self.edge_index = torch.empty(2, E, dtype=torch.int64, device=dev) if materialize_edge_index else None
+        self.struct = _lib.MpnGraph(n, n, 0, self.chunk, E, self.max_tasks, 0, ptrs[0], ptrs[4], ptrs[1], ptrs[3], ptrs[2],
+                                    n_graphs, self.max_graph_nodes, self.node_gid.data_ptr(), self.graph_nptr.data_ptr())
+        with _on_device(dev):
+            _lib.check(L.mpn_graph_build_cross_camera_batched(C.byref(self.struct), base + 8 * (n_segs + 1), n_segs,
+                                                              base + 12 * (n_segs + 1), base,
+                                                              self.edge_index.data_ptr() if materialize_edge_index else None,
+                                                              current_stream_ptr(dev)))
+        self._keepalive = (self.edge_index, aux, pinned)         # pinned: the staging buffer outlives its copy
         return self
 
     @property

@@ -1,6 +1,6 @@
 """What inference.py:383-451 does per graph besides the edge list (SURVEY.md section 8f rows 1 and 4), on the device:
 
-  normalize_columns    F.normalize(node_embeds_g, p=2, dim=0)                        inference.py:403-404
+  normalize_columns    F.normalize(node_embeds_g, p=2, dim=0), one graph or every graph of a batch  inference.py:403-404
   edge_labels          the ground-truth edge labels (an O(E*N) Python comprehension)  inference.py:446-450
   pack_reid_features / load_packed_features
                        the reference keeps ONE pickle per tracklet (libs/reid_feature_extraction.py:176-184) and loads them one
@@ -16,22 +16,32 @@ import numpy as np
 import torch
 
 from . import _lib
-from .graph import TrackletGraph, current_stream_ptr, graph_for, workspace
+from .graph import TrackletGraph, current_stream_ptr, graph_for, host_node_ptr, workspace
 
 
-def normalize_columns(x: torch.Tensor, out: torch.Tensor = None) -> torch.Tensor:
-    """``F.normalize(x, p=2, dim=0)``: every feature column scaled to unit L2 norm over the nodes (eps 1e-12)."""
+def normalize_columns(x: torch.Tensor, out: torch.Tensor = None, ptr=None) -> torch.Tensor:
+    """``F.normalize(x, p=2, dim=0)``: every feature column scaled to unit L2 norm over the nodes (eps 1e-12).
+    ``ptr``: G+1 node offsets of a batch (PyG ``Batch.ptr``): every graph's rows ``x[ptr[g]:ptr[g+1]]`` are normalised on
+    their own, as inference.py:403-404 does inside the loop over graphs, in one kernel."""
     if not x.is_cuda:
         raise RuntimeError("normalize_columns needs a CUDA tensor: the B200 path has no CPU fallback")
     if x.dim() != 2:
         raise ValueError("x must be [N, D]")
+    nptr = host_node_ptr(ptr, x.shape[0]) if ptr is not None else None
     x = x.contiguous().float()
     out = torch.empty_like(x) if out is None else out
     L = _lib.lib()
-    ws = workspace("normalize_columns", x.device, L.mpn_normalize_columns_workspace_bytes(x.shape[1]))
+    stream = current_stream_ptr(x.device)
     with torch.cuda.device(x.device):
-        _lib.check(L.mpn_normalize_columns(x.data_ptr(), x.shape[0], x.shape[1], out.data_ptr(), ws.data_ptr(), ws.numel(),
-                                           current_stream_ptr(x.device)))
+        if nptr is not None and nptr.size > 2:
+            pinned = torch.from_numpy(nptr.astype(np.int32)).pin_memory()
+            gptr = pinned.to(x.device, non_blocking=True)
+            _lib.check(L.mpn_normalize_columns_batched(x.data_ptr(), x.shape[0], x.shape[1], gptr.data_ptr(), nptr.size - 1,
+                                                       out.data_ptr(), None, 0, stream))
+        else:
+            ws = workspace("normalize_columns", x.device, L.mpn_normalize_columns_workspace_bytes(x.shape[1]))
+            _lib.check(L.mpn_normalize_columns(x.data_ptr(), x.shape[0], x.shape[1], out.data_ptr(), ws.data_ptr(), ws.numel(),
+                                               stream))
     return out
 
 

@@ -112,6 +112,22 @@ int64_t mpn_cross_camera_edges(const int32_t* cam_ptr_host, int32_t n_cams);
 int64_t mpn_cross_camera_block_edges(const int32_t* cam_ptr_host, int32_t n_cams, int32_t row0, int32_t n_rows);
 int mpn_graph_build_cross_camera(mpn_graph* g, const int32_t* cam_ptr_host, int32_t n_cams, int64_t* edge_index_out_dev,
                                  void* stream);
+/* The same for a batch of graphs (inference.py:407-414 for every graph of the loop at inference.py:375): block-diagonal tables in
+ * which row r of graph g = [gs, ge), camera segment [ss, se), lists the columns [gs, ss) and [se, ge) in ascending order.  The
+ * layout is given by segments, one per (graph, camera): seg_ptr[s] = first node of segment s (seg_ptr[n_segs] = n_nodes), and
+ * graph_seg[g] = first segment of graph g (graph_seg[n_graphs] = n_segs).  Camera ids need not be contiguous or shared by the
+ * graphs; nodes are grouped by camera within each graph.
+ *   mpn_cross_camera_batched_layout   HOST: validates the layout (segments and graphs non-empty, offsets from 0) and fills
+ *                 seg_ebase_host[n_segs+1] (optional) with the first edge of each segment's row block; returns E, -1 if malformed.
+ *   mpn_graph_build_cross_camera_batched   fills rowptr / col / taskptr / task_row / n_tasks and node_gid / graph_nptr of `g`
+ *                 (g->n_graphs, g->max_graph_nodes and all table pointers set by the caller, g->n_edges = the layout's E, no row
+ *                 block) from the SAME arrays in device memory (seg_ebase_dev from the helper above); edge_index_out_dev: optional
+ *                 [2,E] int64, the per-graph reference edge_index offset by the graph's first node and concatenated.  Leaves
+ *                 layout_hint = MPN_LAYOUT_UNKNOWN (a row does not span all columns).  Does not synchronise. */
+int64_t mpn_cross_camera_batched_layout(const int32_t* seg_ptr_host, int32_t n_segs, const int32_t* graph_seg_host, int32_t n_graphs,
+                                        int64_t* seg_ebase_host);
+int mpn_graph_build_cross_camera_batched(mpn_graph* g, const int32_t* seg_ptr_dev, int32_t n_segs, const int32_t* graph_seg_dev,
+                                         const int64_t* seg_ebase_dev, int64_t* edge_index_out_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Edge features (K1).  Replaces inference.py:453-456:
@@ -479,11 +495,18 @@ int mpn_write_mtmc_txt_host(const char* path, const int64_t* table_host, int64_t
  *                           else 0.0f, in the graph's edge order; node_labels_dev int64 [n_cols].
  *   mpn_normalize_columns   F.normalize(node_embeds, p=2, dim=0) (inference.py:403-404): out[i,j] = x[i,j] / max(||x[:,j]||_2, 1e-12);
  *                           out may alias x.
+ *   mpn_normalize_columns_batched   the same for every graph of a batch alone (inference.py:403-404 inside the loop over graphs,
+ *                           inference.py:375): rows [graph_nptr[g], graph_nptr[g+1]) are scaled by their own column norms.  fp64 sums
+ *                           in a fixed order (deterministic), no workspace for n_graphs > 1; out may alias x.  n_graphs <= 1 is
+ *                           mpn_normalize_columns with the workspace given (graph_nptr_dev unused); for n_graphs > 1 the workspace
+ *                           arguments are unused and may be NULL / 0.
  * ---------------------------------------------------------------------------------------------- */
 int mpn_edge_labels(const mpn_graph* g, const int64_t* node_labels_dev, float* out_dev, void* stream);
 size_t mpn_normalize_columns_workspace_bytes(int32_t D);
 int mpn_normalize_columns(const float* x_dev, int32_t n, int32_t D, float* out_dev, void* workspace_dev, size_t workspace_bytes,
                           void* stream);
+int mpn_normalize_columns_batched(const float* x_dev, int32_t n, int32_t D, const int32_t* graph_nptr_dev, int32_t n_graphs,
+                                  float* out_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
