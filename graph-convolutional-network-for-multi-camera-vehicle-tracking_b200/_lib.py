@@ -15,6 +15,7 @@ MPN_SUMS_DOUBLES = 96
 ABI_VERSION = 6             # MPN_B200_ABI_VERSION of include/mpn_b200.h (bumped when a struct or a signature changes)
 STAGE_ENC0, STAGE_ENC1, STAGE_EDGE, STAGE_NODE, STAGE_APPLY = range(5)
 POST_CUT, POST_PRUNE, POST_SPLIT = 1, 2, 4
+MPN_X_F32, MPN_X_F16, MPN_X_BF16 = 0, 1, 2      # element kind of the node features x (the *_x entry points)
 
 # offsets inside mpn_weights.small (floats) — keep in sync with include/mpn_b200.h
 W_ENC1_W, W_ENC1_B, W_ENC1_G, W_ENC1_BETA = 0, 8, 12, 16
@@ -170,6 +171,26 @@ _PROTOS = {
                               C.c_void_p]),
     "mpn_gemm_nt": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int,
                               C.c_void_p, C.c_size_t, C.c_void_p]),
+    # the entry points that read x, with (x, x_kind) in place of an fp32 x
+    "mpn_edge_features_x": (C.c_int, [C.POINTER(MpnGraph), C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int, C.c_void_p,
+                                      C.c_size_t, C.c_void_p]),
+    "mpn_forward_x": (C.c_int, [C.POINTER(MpnGraph), C.POINTER(MpnWeights), C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32,
+                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpn_forward_with_edge_features_x": (C.c_int, [C.POINTER(MpnGraph), C.POINTER(MpnWeights), C.c_void_p, C.c_int32, C.c_void_p,
+                                                   C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                                   C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpn_forward_sharded_x": (C.c_int, [C.POINTER(MpnGraph), C.POINTER(MpnWeights), C.c_void_p, C.c_int32, C.c_void_p, C.c_int32,
+                                        C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
+                                        C.POINTER(MpnPeerCtx), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpn_forward_sharded_with_edge_features_x": (C.c_int, [C.POINTER(MpnGraph), C.POINTER(MpnWeights), C.c_void_p, C.c_int32,
+                                                           C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
+                                                           C.c_void_p, C.c_void_p, C.c_int, C.POINTER(MpnPeerCtx), C.c_void_p,
+                                                           C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpn_plan_node_encoder_x": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "mpn_normalize_columns_x": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t,
+                                          C.c_void_p]),
+    "mpn_normalize_columns_batched_x": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
+                                                  C.c_void_p, C.c_size_t, C.c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_PROTOS.keys())

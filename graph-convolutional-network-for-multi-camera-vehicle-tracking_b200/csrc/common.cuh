@@ -1,9 +1,13 @@
 // Shared helpers for the sm_100a kernels of the MPN path.
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
+
+#include <type_traits>
 
 #include "../../include/mpn_b200.h"
 
@@ -65,6 +69,25 @@ struct Arena {
 };
 
 static inline int div_up(long long a, long long b) { return (int)((a + b - 1) / b); }
+
+// node-feature element kinds (MPN_X_*): validity, element size, and the call of f with a typed null pointer of the element type
+static inline bool x_kind_ok(int kind) { return kind == MPN_X_F32 || kind == MPN_X_F16 || kind == MPN_X_BF16; }
+static inline size_t x_elem_bytes(int kind) { return kind == MPN_X_F32 ? sizeof(float) : 2; }
+// the vector loads of x (ld4 / cvt4) read four elements at once: 16 bytes for fp32, 8 for 16-bit types
+static inline bool x_vec4_aligned(const void* x, int kind) { return ((uintptr_t)x % (4 * x_elem_bytes(kind))) == 0; }
+template <typename P>
+using x_elem_t = std::remove_cv_t<std::remove_pointer_t<P>>;     // element type behind with_x_type's typed null pointer
+template <typename F>
+static inline int with_x_type(int kind, F&& f) {
+  switch (kind) {
+    case MPN_X_F32: return f((const float*)nullptr);
+    case MPN_X_F16: return f((const __half*)nullptr);
+    case MPN_X_BF16: return f((const __nv_bfloat16*)nullptr);
+  }
+  set_error("unknown node-feature element kind %d (MPN_X_F32, MPN_X_F16 or MPN_X_BF16)", kind);
+  return MPN_ERR_INVALID;
+}
+#define MPN_X_KIND_OK(kind) MPN_REQUIRE(mpn::x_kind_ok(kind), "unknown node-feature element kind %d (MPN_X_F32, MPN_X_F16 or MPN_X_BF16)", (int)(kind))
 
 // Programmatic dependent launch (on by default; mpn_set_pdl(0) switches it off for A/B measurements).  A kernel launched
 // through launch() carries the programmatic-stream-serialization attribute and may be scheduled while its predecessor in the
@@ -140,6 +163,30 @@ __device__ __forceinline__ void block_sum_lane_columns(double v, double* smem /*
     out[threadIdx.x] = s;
   }
   __syncthreads();
+}
+
+// Node features x of element type T (float, __half, __nv_bfloat16: MPN_X_F32 / F16 / BF16), converted to fp32 on load.  Both
+// 16-bit conversions are exact, so a kernel templated on T computes on the same fp32 values as on x.float().  ld4(p, i) reads
+// the i-th group of four consecutive elements from p, which an fp32 kernel reads as one float4 (16 bytes for fp32, 8 for 16-bit
+// types): every lane keeps its columns and every reduction its order and grouping, whatever the width of the element.
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <typename T>
+using vec4_t = std::conditional_t<sizeof(T) == 4, float4, uint2>;      // four elements of T as one load
+template <typename T>
+__device__ __forceinline__ float4 cvt4(const vec4_t<T>& v) {
+  if constexpr (sizeof(T) == 4) {
+    return v;
+  } else {
+    T e[4];
+    memcpy(e, &v, sizeof(v));
+    return make_float4(to_f32(e[0]), to_f32(e[1]), to_f32(e[2]), to_f32(e[3]));
+  }
+}
+template <typename T, typename I>
+__device__ __forceinline__ float4 ld4(const T* p, I i) {     // p: 16-byte aligned for fp32, 8-byte aligned for 16-bit types
+  return cvt4<T>(reinterpret_cast<const vec4_t<T>*>(p)[i]);
 }
 
 // streaming (read-once) loads: bypass L1 allocation

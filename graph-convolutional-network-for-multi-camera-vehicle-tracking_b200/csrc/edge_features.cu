@@ -16,7 +16,8 @@ namespace mpn {
 
 // column means of x [n, D] (fp64 accumulation): grid (32-column tiles, row splits) -> partials -> fixed-order finalize
 constexpr int CM_SPLITS = 32;
-__global__ void __launch_bounds__(256) col_mean_partial_kernel(const float* __restrict__ x, int n, int D, int rows_per_split,
+template <typename T>
+__global__ void __launch_bounds__(256) col_mean_partial_kernel(const T* __restrict__ x, int n, int D, int rows_per_split,
                                                                double* __restrict__ part /*[CM_SPLITS][D]*/) {
   pdl_wait();
   __shared__ double ssum[8][33];
@@ -25,7 +26,7 @@ __global__ void __launch_bounds__(256) col_mean_partial_kernel(const float* __re
   const int r0 = blockIdx.y * rows_per_split, r1 = min(r0 + rows_per_split, n);
   double s = 0.0;
   if (col < D)
-    for (int r = r0 + ry; r < r1; r += 8) s += x[(size_t)r * D + col];
+    for (int r = r0 + ry; r < r1; r += 8) s += to_f32(x[(size_t)r * D + col]);
   ssum[ry][cx] = s;
   __syncthreads();
   if (ry == 0 && col < D) {
@@ -44,7 +45,8 @@ __global__ void col_mean_finalize_kernel(const double* __restrict__ part, int n,
 
 // xc = x - mu; per-row statistics of the centred row (accumulated in fp64, stored as one float4 = one 16-byte gather
 // per edge; the Gram entry they are combined with is itself only fp32-accurate): st[r] = {|a'|^2, sum a', mu.a' + |mu|^2/2, |a|}
-__global__ void __launch_bounds__(256) center_rows_kernel(const float* __restrict__ x, const float* __restrict__ mu, int n, int D,
+template <typename T>
+__global__ void __launch_bounds__(256) center_rows_kernel(const T* __restrict__ x, const float* __restrict__ mu, int n, int D,
                                                           float* __restrict__ xc, float4* __restrict__ st,
                                                           unsigned int* __restrict__ amax_bits, const int* __restrict__ run_flag) {
   pdl_wait();
@@ -53,13 +55,13 @@ __global__ void __launch_bounds__(256) center_rows_kernel(const float* __restric
   const int gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int nwarps = (gridDim.x * blockDim.x) >> 5;
   for (int r = gwarp; r < n; r += nwarps) {
-    const float* p = x + (size_t)r * D;
+    const T* p = x + (size_t)r * D;
     float* q = xc + (size_t)r * D;
     double sq = 0.0, sx = 0.0, md = 0.0, mm = 0.0;
     float amax = 0.f;
     for (int k = lane; k < D; k += 32) {
       const float m = mu[k];
-      const float c = p[k] - m;
+      const float c = to_f32(p[k]) - m;
       q[k] = c;
       amax = fmaxf(amax, fabsf(c));
       sq += (double)c * c;
@@ -130,7 +132,8 @@ __global__ void __launch_bounds__(256) edge_feature_gather_kernel(const mpn_grap
 // direct recomputation for the flagged pairs (one warp per pair), fp32 elementwise like ATen
 // fixed_sums (optional, with the fused kernel only): the moment sums (a, b, aa, ab, bb) of the recomputed pairs are added as
 // 2^40 fixed point integers, so the total does not depend on the order in which the list was filled
-__global__ void __launch_bounds__(256) edge_feature_refine_kernel(const mpn_graph g, const float* __restrict__ x, int D,
+template <typename T>
+__global__ void __launch_bounds__(256) edge_feature_refine_kernel(const mpn_graph g, const T* __restrict__ x, int D,
                                                                   const int* __restrict__ refine_list,
                                                                   const int* __restrict__ refine_count,
                                                                   float2* __restrict__ edge_attr,
@@ -152,11 +155,11 @@ __global__ void __launch_bounds__(256) edge_feature_refine_kernel(const mpn_grap
       if (g.rowptr[mid] <= e) lo = mid; else hi = mid;
     }
     const int cnode = g.col[e];
-    const float* a = x + (size_t)(lo + g.row_offset) * D;
-    const float* b = x + (size_t)cnode * D;
+    const T* a = x + (size_t)(lo + g.row_offset) * D;
+    const T* b = x + (size_t)cnode * D;
     double d2 = 0.0, d2m = 0.0, ab = 0.0, aa = 0.0, bb = 0.0;
     for (int k = lane; k < D; k += 32) {
-      const float av = a[k], bv = b[k];
+      const float av = to_f32(a[k]), bv = to_f32(b[k]);
       const float df = av - bv + PAIRWISE_EPS;
       const float dfm = bv - av + PAIRWISE_EPS;
       d2 += (double)df * df;
@@ -255,14 +258,34 @@ static EfLayout ef_layout(const mpn_graph* g, int D, void* ws, size_t ws_bytes) 
   return L;
 }
 
+// the two launches of edge_features_impl that read x, instantiated for its element type
+static int center_rows(const void* x, int x_kind, const EfLayout& L, int n, int D, const int* run_flag, cudaStream_t st) {
+  return with_x_type(x_kind, [&](auto xt) {
+    mpn::launch(center_rows_kernel<x_elem_t<decltype(xt)>>, min(kNumSMs * 8, div_up((long long)n * 32, 256)), 256, 0,
+                st, (decltype(xt))x, L.mu, n, D, L.xc, L.st, L.amax_bits, run_flag);
+    MPN_LAUNCH_OK();
+    return MPN_OK;
+  });
+}
+static int refine_pairs(const mpn_graph& g, const void* x, int x_kind, int D, const EfLayout& L, float2* edge_attr,
+                        unsigned long long* fixed_sums, const int* not_one_gap, const GeShare& sh, cudaStream_t st) {
+  return with_x_type(x_kind, [&](auto xt) {
+    mpn::launch(edge_feature_refine_kernel<x_elem_t<decltype(xt)>>, kNumSMs * 4, 256, 0, st, g, (decltype(xt))x, D,
+                L.refine_list, L.refine_count, edge_attr, fixed_sums, not_one_gap, sh);
+    MPN_LAUNCH_OK();
+    return MPN_OK;
+  });
+}
+
 // moments (optional): the caller wants the first encoder BatchNorm's moment sums taken on the way (mpn_forward_with_edge_features).
 //   partials   [>= 148][MPN_SUMS_DOUBLES] zeroed by the caller; the fused kernel writes one row per CTA
 //   fixed_sums [5] zeroed by the caller; the refine pass adds the recomputed pairs' share as 2^40 fixed point
 //   handled    out: device flag, 0 = the fused kernel produced features AND moments, != 0 = the caller must sweep edge_attr itself;
 //              nullptr when that is already known on the host (known_fused tells which)
-int edge_features_impl(const mpn_graph* g, const float* x, int32_t D, float* edge_attr, int use_tc, void* ws, size_t ws_bytes,
-                       cudaStream_t st, EfMoments* moments, const GeShare* share) {
+int edge_features_impl(const mpn_graph* g, const void* x, int x_kind, int32_t D, float* edge_attr, int use_tc, void* ws,
+                       size_t ws_bytes, cudaStream_t st, EfMoments* moments, const GeShare* share) {
   MPN_REQUIRE(g && x && D > 0 && ws, "edge_features: NULL argument");
+  MPN_X_KIND_OK(x_kind);
   MPN_REQUIRE(edge_attr || g->n_edges == 0, "edge_features: NULL output");
   MPN_REQUIRE(((uintptr_t)ws & 255) == 0, "workspace must be 256-byte aligned");
   EfLayout L = ef_layout(g, D, ws, ws_bytes);
@@ -273,19 +296,21 @@ int edge_features_impl(const mpn_graph* g, const float* x, int32_t D, float* edg
   if (moments) { moments->handled_flag = nullptr; moments->known_fused = 0; }
   if (g->n_edges == 0) return MPN_OK;
   MPN_CUDA_OK(cudaMemsetAsync(L.refine_count, 0, 5 * 256, st));        // refine_count, amax_bits, mean ticket, not_one_gap, share mode (adjacent slices)
-  if ((D % 4) == 0 && D <= 8192 && (((uintptr_t)x) & 15) == 0) {          // (64 ticket slots: one per 128-column tile)
-    MPN_TRY(ge_col_mean(x, g->n_cols, D, L.mu_part, L.mu_ticket, L.mu, st));
+  if ((D % 4) == 0 && D <= 8192 && x_vec4_aligned(x, x_kind)) {          // (64 ticket slots: one per 128-column tile)
+    MPN_TRY(ge_col_mean(x, x_kind, g->n_cols, D, L.mu_part, L.mu_ticket, L.mu, st));
   } else {
-    mpn::launch(col_mean_partial_kernel, dim3(div_up(D, 32), CM_SPLITS), 256, 0, st, x, g->n_cols, D, div_up(g->n_cols, CM_SPLITS), L.mu_part);
-    MPN_LAUNCH_OK();
+    MPN_TRY(with_x_type(x_kind, [&](auto xt) {
+      mpn::launch(col_mean_partial_kernel<x_elem_t<decltype(xt)>>, dim3(div_up(D, 32), CM_SPLITS), 256, 0, st,
+                  (decltype(xt))x, g->n_cols, D, div_up(g->n_cols, CM_SPLITS), L.mu_part);
+      MPN_LAUNCH_OK();
+      return MPN_OK;
+    }));
     mpn::launch(col_mean_finalize_kernel, div_up(D, 128), 128, 0, st, L.mu_part, g->n_cols, D, L.mu);
     MPN_LAUNCH_OK();
   }
   if (g->n_graphs > 1 && g->node_gid && g->graph_nptr) {
     // batched small graphs: block-diagonal Gram (one ng x ng block per graph), gather epilogue
-    mpn::launch(center_rows_kernel, min(kNumSMs * 8, div_up((long long)g->n_cols * 32, 256)), 256, 0, st, x, L.mu, g->n_cols, D, L.xc, L.st, L.amax_bits,
-                (const int*)nullptr);
-    MPN_LAUNCH_OK();
+    MPN_TRY(center_rows(x, x_kind, L, g->n_cols, D, nullptr, st));
     MPN_REQUIRE(g->row_offset == 0 && g->n_cols == g->n_nodes && g->max_graph_nodes > 0, "batched edge features: bad graph");
     mpn::launch(gram_offsets_kernel, 1, 32, 0, st, g->graph_nptr, g->n_graphs, L.g_off);
     MPN_LAUNCH_OK();
@@ -299,16 +324,13 @@ int edge_features_impl(const mpn_graph* g, const float* x, int32_t D, float* edg
     mpn::launch(edge_feature_gather_kernel, kNumSMs * 8, 256, 0, st, *g, 0, g->n_nodes, L.G, L.g_off, L.st, D, (float2*)edge_attr, L.refine_list,
                                                            L.refine_count, (const int*)nullptr);
     MPN_LAUNCH_OK();
-    mpn::launch(edge_feature_refine_kernel, kNumSMs * 4, 256, 0, st, *g, x, D, L.refine_list, L.refine_count, (float2*)edge_attr,
-                (unsigned long long*)nullptr, (const int*)nullptr, GeShare{});
-    MPN_LAUNCH_OK();
-    return MPN_OK;
+    return refine_pairs(*g, x, x_kind, D, L, (float2*)edge_attr, nullptr, nullptr, GeShare{}, st);
   }
   // Dense cross-camera graphs (every row = all columns but one gap; verified on the device unless the builder of the graph
   // vouches for it through g->layout_hint): the features are formed in the epilogue of the Gram GEMM (gram_ef.cu).  Any other
   // graph: Gram block in HBM + gather.  With an unknown layout both sets of launches are enqueued, each kernel tests the
   // device flag first and one set returns at once.
-  const bool fused = use_tc && L.fused_possible;
+  const bool fused = use_tc && L.fused_possible && (((uintptr_t)x) & 15) == 0;     // (16-byte cp.async of the rows)
   const bool known_one_gap = fused && g->layout_hint == MPN_LAYOUT_ONE_GAP;
   GeShare sh;
   memset(&sh, 0, sizeof(sh));
@@ -320,15 +342,13 @@ int edge_features_impl(const mpn_graph* g, const float* x, int32_t D, float* edg
   const int* run_gather = nullptr;                   // old path: unconditional
   if (fused) {
     int n_rows = 0;
-    MPN_TRY(gram_ef_run(x, L.mu, g, D, L.gap, L.not_one_gap, (float2*)edge_attr, L.refine_list, L.refine_count,
+    MPN_TRY(gram_ef_run(x, x_kind, L.mu, g, D, L.gap, L.not_one_gap, (float2*)edge_attr, L.refine_list, L.refine_count,
                         moments ? moments->partials : nullptr, &n_rows, L.ge, st, share ? &sh : nullptr));
     if (moments) { moments->handled_flag = L.not_one_gap; moments->known_fused = known_one_gap ? 1 : 0; }
     run_gather = L.not_one_gap;
   }
   if (!known_one_gap) {
-    mpn::launch(center_rows_kernel, min(kNumSMs * 8, div_up((long long)g->n_cols * 32, 256)), 256, 0, st, x, L.mu, g->n_cols, D, L.xc, L.st, L.amax_bits,
-                run_gather);
-    MPN_LAUNCH_OK();
+    MPN_TRY(center_rows(x, x_kind, L, g->n_cols, D, run_gather, st));
     for (int r0 = 0; r0 < g->n_nodes; r0 += L.rows_per_block) {
       const int r1 = min(r0 + L.rows_per_block, g->n_nodes);
       const float* Ablk = L.xc + (size_t)(g->row_offset + r0) * D;
@@ -341,10 +361,8 @@ int edge_features_impl(const mpn_graph* g, const float* x, int32_t D, float* edg
       MPN_LAUNCH_OK();
     }
   }
-  mpn::launch(edge_feature_refine_kernel, kNumSMs * 4, 256, 0, st, *g, x, D, L.refine_list, L.refine_count, (float2*)edge_attr,
-              moments ? moments->fixed_sums : (unsigned long long*)nullptr, fused ? (const int*)L.not_one_gap : (const int*)nullptr, sh);
-  MPN_LAUNCH_OK();
-  return MPN_OK;
+  return refine_pairs(*g, x, x_kind, D, L, (float2*)edge_attr, moments ? moments->fixed_sums : nullptr,
+                      fused ? L.not_one_gap : nullptr, sh, st);
 }
 
 }  // namespace mpn
@@ -370,9 +388,14 @@ size_t mpn_edge_features_workspace_bytes(const mpn_graph* g, int32_t D) {
   return ef_layout(g, D, nullptr, 0).total + 256;
 }
 
+int mpn_edge_features_x(const mpn_graph* g, const void* x, int32_t x_kind, int32_t D, float* edge_attr, int use_tc, void* ws,
+                        size_t ws_bytes, void* stream) {
+  return mpn::edge_features_impl(g, x, x_kind, D, edge_attr, use_tc, ws, ws_bytes, (cudaStream_t)stream, nullptr);
+}
+
 int mpn_edge_features(const mpn_graph* g, const float* x, int32_t D, float* edge_attr, int use_tc, void* ws, size_t ws_bytes,
                       void* stream) {
-  return mpn::edge_features_impl(g, x, D, edge_attr, use_tc, ws, ws_bytes, (cudaStream_t)stream, nullptr);
+  return mpn_edge_features_x(g, x, MPN_X_F32, D, edge_attr, use_tc, ws, ws_bytes, stream);
 }
 
 }  // extern "C"

@@ -343,7 +343,8 @@ __global__ void __launch_bounds__(256) edge_labels_kernel(const mpn_graph g, con
 }
 
 constexpr int NC_SPLITS = 64;
-__global__ void __launch_bounds__(256) colsq_partial_kernel(const float* __restrict__ x, int n, int D, int rows_per_split,
+template <typename T>
+__global__ void __launch_bounds__(256) colsq_partial_kernel(const T* __restrict__ x, int n, int D, int rows_per_split,
                                                             double* __restrict__ part /*[NC_SPLITS][D]*/) {
   __shared__ double ssum[8][33];
   const int cx = threadIdx.x & 31, ry = threadIdx.x >> 5;
@@ -351,7 +352,7 @@ __global__ void __launch_bounds__(256) colsq_partial_kernel(const float* __restr
   const int r0 = blockIdx.y * rows_per_split, r1 = min(r0 + rows_per_split, n);
   double s = 0.0;
   if (col < D)
-    for (int r = r0 + ry; r < r1; r += 8) { const double v = x[(size_t)r * D + col]; s += v * v; }
+    for (int r = r0 + ry; r < r1; r += 8) { const double v = to_f32(x[(size_t)r * D + col]); s += v * v; }
   ssum[ry][cx] = s;
   __syncthreads();
   if (ry == 0 && col < D) {
@@ -367,10 +368,11 @@ __global__ void colnorm_finalize_kernel(const double* __restrict__ part, int D, 
   const float nrm = fmaxf((float)sqrt(s), 1e-12f);                 // F.normalize: v / max(||v||_2, eps)
   norm_out[col] = nrm;
 }
-__global__ void colnorm_apply_kernel(const float* __restrict__ x, long long total, int D, const float* __restrict__ norm,
+template <typename T>
+__global__ void colnorm_apply_kernel(const T* __restrict__ x, long long total, int D, const float* __restrict__ norm,
                                      float* __restrict__ out) {
   const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) out[i] = x[i] / norm[i % D];
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) out[i] = to_f32(x[i]) / norm[i % D];
 }
 
 
@@ -378,7 +380,8 @@ __global__ void colnorm_apply_kernel(const float* __restrict__ x, long long tota
 // thread (ry, cx) sums the squares of column cx over the graph's rows ry, ry + 256/sw, ... in fp64, then the 256/sw partials are
 // added in order (deterministic).  Pass 2 re-reads the slab, which is still in L2 (300 rows x 32 columns = 38 KB at S02 size), and
 // writes it scaled.  A CTA writes only the slab it has finished summing, so out may alias x (no __restrict__).
-__global__ void __launch_bounds__(256) colnorm_graph_kernel(const float* x, int D, const int* __restrict__ graph_nptr, int sw,
+template <typename T>
+__global__ void __launch_bounds__(256) colnorm_graph_kernel(const T* x, int D, const int* __restrict__ graph_nptr, int sw,
                                                             float* out) {
   __shared__ double part[256];
   __shared__ float nrm[32];
@@ -388,7 +391,7 @@ __global__ void __launch_bounds__(256) colnorm_graph_kernel(const float* x, int 
   double s = 0.0;
   if (col < D) {
 #pragma unroll 4
-    for (int r = r0 + ry; r < r1; r += nry) { const double v = x[(size_t)r * D + col]; s += v * v; }
+    for (int r = r0 + ry; r < r1; r += nry) { const double v = to_f32(x[(size_t)r * D + col]); s += v * v; }
   }
   part[threadIdx.x] = s;
   __syncthreads();
@@ -400,7 +403,7 @@ __global__ void __launch_bounds__(256) colnorm_graph_kernel(const float* x, int 
   if (col < D) {
     const float q = nrm[cx];
 #pragma unroll 4
-    for (int r = r0 + ry; r < r1; r += nry) out[(size_t)r * D + col] = x[(size_t)r * D + col] / q;
+    for (int r = r0 + ry; r < r1; r += nry) out[(size_t)r * D + col] = to_f32(x[(size_t)r * D + col]) / q;
   }
 }
 
@@ -418,7 +421,9 @@ int mpn_edge_labels(const mpn_graph* g, const int64_t* node_labels_dev, float* o
 
 size_t mpn_normalize_columns_workspace_bytes(int32_t D) { return (size_t)NC_SPLITS * D * sizeof(double) + (size_t)D * sizeof(float) + 512; }
 
-int mpn_normalize_columns(const float* x_dev, int32_t n, int32_t D, float* out_dev, void* ws, size_t ws_bytes, void* stream) {
+int mpn_normalize_columns_x(const void* x_dev, int32_t x_kind, int32_t n, int32_t D, float* out_dev, void* ws, size_t ws_bytes,
+                            void* stream) {
+  MPN_X_KIND_OK(x_kind);
   MPN_REQUIRE(n >= 0 && D > 0 && ws, "normalize_columns: bad argument");
   MPN_REQUIRE(ws_bytes >= mpn_normalize_columns_workspace_bytes(D), "normalize_columns workspace too small");
   MPN_REQUIRE(((uintptr_t)ws & 255) == 0, "workspace must be 256-byte aligned");
@@ -427,19 +432,26 @@ int mpn_normalize_columns(const float* x_dev, int32_t n, int32_t D, float* out_d
   cudaStream_t st = (cudaStream_t)stream;
   double* part = (double*)ws;
   float* norm = (float*)(part + (size_t)NC_SPLITS * D);
-  colsq_partial_kernel<<<dim3(div_up(D, 32), NC_SPLITS), 256, 0, st>>>(x_dev, n, D, div_up(n, NC_SPLITS), part);
-  MPN_LAUNCH_OK();
-  colnorm_finalize_kernel<<<div_up(D, 128), 128, 0, st>>>(part, D, norm);
-  MPN_LAUNCH_OK();
   const long long total = (long long)n * D;
-  colnorm_apply_kernel<<<grid_for(total), 256, 0, st>>>(x_dev, total, D, norm, out_dev);
-  MPN_LAUNCH_OK();
-  return MPN_OK;
+  return with_x_type(x_kind, [&](auto xt) {
+    colsq_partial_kernel<<<dim3(div_up(D, 32), NC_SPLITS), 256, 0, st>>>((decltype(xt))x_dev, n, D, div_up(n, NC_SPLITS), part);
+    MPN_LAUNCH_OK();
+    colnorm_finalize_kernel<<<div_up(D, 128), 128, 0, st>>>(part, D, norm);
+    MPN_LAUNCH_OK();
+    colnorm_apply_kernel<<<grid_for(total), 256, 0, st>>>((decltype(xt))x_dev, total, D, norm, out_dev);
+    MPN_LAUNCH_OK();
+    return MPN_OK;
+  });
 }
 
-int mpn_normalize_columns_batched(const float* x_dev, int32_t n, int32_t D, const int32_t* graph_nptr_dev, int32_t n_graphs,
-                                  float* out_dev, void* ws, size_t ws_bytes, void* stream) {
-  if (n_graphs <= 1) return mpn_normalize_columns(x_dev, n, D, out_dev, ws, ws_bytes, stream);
+int mpn_normalize_columns(const float* x_dev, int32_t n, int32_t D, float* out_dev, void* ws, size_t ws_bytes, void* stream) {
+  return mpn_normalize_columns_x(x_dev, MPN_X_F32, n, D, out_dev, ws, ws_bytes, stream);
+}
+
+int mpn_normalize_columns_batched_x(const void* x_dev, int32_t x_kind, int32_t n, int32_t D, const int32_t* graph_nptr_dev,
+                                    int32_t n_graphs, float* out_dev, void* ws, size_t ws_bytes, void* stream) {
+  if (n_graphs <= 1) return mpn_normalize_columns_x(x_dev, x_kind, n, D, out_dev, ws, ws_bytes, stream);
+  MPN_X_KIND_OK(x_kind);
   MPN_REQUIRE(n > 0 && D > 0, "normalize_columns_batched: bad argument");
   MPN_REQUIRE(x_dev && out_dev && graph_nptr_dev, "normalize_columns_batched: NULL argument");
   MPN_REQUIRE(div_up(D, 8) <= 65535, "normalize_columns_batched: D must be <= 524280");
@@ -447,9 +459,16 @@ int mpn_normalize_columns_batched(const float* x_dev, int32_t n, int32_t D, cons
   // CTAs (8 per SM) is in flight
   int sw = 32;
   while (sw > 8 && (long long)n_graphs * div_up(D, sw) < kNumSMs * 8) sw >>= 1;
-  colnorm_graph_kernel<<<dim3(n_graphs, div_up(D, sw)), 256, 0, (cudaStream_t)stream>>>(x_dev, D, graph_nptr_dev, sw, out_dev);
-  MPN_LAUNCH_OK();
-  return MPN_OK;
+  return with_x_type(x_kind, [&](auto xt) {
+    colnorm_graph_kernel<<<dim3(n_graphs, div_up(D, sw)), 256, 0, (cudaStream_t)stream>>>((decltype(xt))x_dev, D, graph_nptr_dev, sw, out_dev);
+    MPN_LAUNCH_OK();
+    return MPN_OK;
+  });
+}
+
+int mpn_normalize_columns_batched(const float* x_dev, int32_t n, int32_t D, const int32_t* graph_nptr_dev, int32_t n_graphs,
+                                  float* out_dev, void* ws, size_t ws_bytes, void* stream) {
+  return mpn_normalize_columns_batched_x(x_dev, MPN_X_F32, n, D, graph_nptr_dev, n_graphs, out_dev, ws, ws_bytes, stream);
 }
 
 }  // extern "C"

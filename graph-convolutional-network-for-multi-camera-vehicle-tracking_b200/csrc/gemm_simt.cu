@@ -9,25 +9,25 @@ namespace mpn {
 
 constexpr int BM = 64, BN = 64, BK = 16, GT = 256;
 
-template <bool ALIGNED>
-__device__ __forceinline__ float4 load4(const float* __restrict__ base, int r, int rows, int k, int K, long long ld) {
+template <bool ALIGNED, typename T>
+__device__ __forceinline__ float4 load4(const T* __restrict__ base, int r, int rows, int k, int K, long long ld) {
   float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
   if (r < rows) {
-    const float* p = base + (long long)r * ld + k;
+    const T* p = base + (long long)r * ld + k;
     if (ALIGNED && k + 3 < K) {
-      v = *reinterpret_cast<const float4*>(p);
+      v = ld4(p, 0);
     } else {
-      if (k + 0 < K) v.x = p[0];
-      if (k + 1 < K) v.y = p[1];
-      if (k + 2 < K) v.z = p[2];
-      if (k + 3 < K) v.w = p[3];
+      if (k + 0 < K) v.x = to_f32(p[0]);
+      if (k + 1 < K) v.y = to_f32(p[1]);
+      if (k + 2 < K) v.z = to_f32(p[2]);
+      if (k + 3 < K) v.w = to_f32(p[3]);
     }
   }
   return v;
 }
 
-template <bool ALIGNED>
-__global__ void __launch_bounds__(GT) gemm_nt_simt_kernel(const float* __restrict__ A, const float* __restrict__ B,
+template <bool ALIGNED, typename TA>
+__global__ void __launch_bounds__(GT) gemm_nt_simt_kernel(const TA* __restrict__ A, const float* __restrict__ B,
                                                           const float* __restrict__ bias, const float* __restrict__ a_scale,
                                                           const float* __restrict__ a_shift, const int* __restrict__ row_gid,
                                                           float* __restrict__ C, int M, int N, int K) {
@@ -93,17 +93,20 @@ __global__ void __launch_bounds__(GT) gemm_nt_simt_kernel(const float* __restric
   }
 }
 
-int gemm_nt_simt(const float* A, const float* B, const float* bias, const float* a_scale, const float* a_shift, float* C,
-                 int M, int N, int K, cudaStream_t st, const int* row_gid) {
+int gemm_nt_simt(const void* A, const float* B, const float* bias, const float* a_scale, const float* a_shift, float* C,
+                 int M, int N, int K, cudaStream_t st, const int* row_gid, int a_kind) {
   MPN_REQUIRE(M > 0 && N > 0 && K > 0, "gemm: bad shape %d x %d x %d", M, N, K);
   dim3 grid(div_up(N, BN), div_up(M, BM));
   const bool aligned = (K % 4 == 0) && (((uintptr_t)A | (uintptr_t)B) % 16 == 0);
-  if (aligned)
-    mpn::launch(gemm_nt_simt_kernel<true>, grid, GT, 0, st, A, B, bias, a_scale, a_shift, row_gid, C, M, N, K);
-  else
-    mpn::launch(gemm_nt_simt_kernel<false>, grid, GT, 0, st, A, B, bias, a_scale, a_shift, row_gid, C, M, N, K);
-  MPN_LAUNCH_OK();
-  return MPN_OK;
+  return with_x_type(a_kind, [&](auto at) {
+    using TA = x_elem_t<decltype(at)>;
+    if (aligned)
+      mpn::launch(gemm_nt_simt_kernel<true, TA>, grid, GT, 0, st, (const TA*)A, B, bias, a_scale, a_shift, row_gid, C, M, N, K);
+    else
+      mpn::launch(gemm_nt_simt_kernel<false, TA>, grid, GT, 0, st, (const TA*)A, B, bias, a_scale, a_shift, row_gid, C, M, N, K);
+    MPN_LAUNCH_OK();
+    return MPN_OK;
+  });
 }
 
 }  // namespace mpn

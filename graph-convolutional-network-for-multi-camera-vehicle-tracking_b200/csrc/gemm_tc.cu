@@ -223,13 +223,14 @@ gemm_nt_3xtf32_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid
 
 // x -> (hi, lo) TF32 planes.  Optional fused input transform f(x)[m,k] = relu(x*scale[k] + shift[k]): the BatchNorm+ReLU of
 // the previous encoder layer (models/mlp.py:14-19), so the activation is never re-written in fp32.
-__global__ void __launch_bounds__(256) split_tf32_kernel(const float4* __restrict__ x, long long n4, int K, const float* __restrict__ scale,
+template <typename T>
+__global__ void __launch_bounds__(256) split_tf32_kernel(const T* __restrict__ x, long long n4, int K, const float* __restrict__ scale,
                                                          const float* __restrict__ shift, const int* __restrict__ row_gid,
                                                          float4* __restrict__ hi, float4* __restrict__ lo) {
   pdl_wait();
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
-    const float4 v = x[i];
+    const float4 v = ld4(x, i);
     float in[4] = {v.x, v.y, v.z, v.w};
     if (scale != nullptr) {
       const int k = (int)((i * 4) % K);                 // K % 4 == 0: the four lanes stay inside one row
@@ -322,7 +323,7 @@ int make_tma_map_2d(CUtensorMap* map, const void* base, int rows, int K, int box
 int split_tf32(const float* x, long long n, float* hi, float* lo, cudaStream_t st) {
   MPN_REQUIRE(x && hi && lo && n > 0 && (n % 4) == 0, "split_tf32: bad arguments (n must be a positive multiple of 4)");
   MPN_REQUIRE((((uintptr_t)x | (uintptr_t)hi | (uintptr_t)lo) & 15) == 0, "split_tf32: pointers must be 16-byte aligned");
-  mpn::launch(split_tf32_kernel, (int)min((long long)kNumSMs * 8, (n / 4 + 255) / 256), 256, 0, st, (const float4*)x, n / 4, 4, nullptr, nullptr, nullptr, (float4*)hi, (float4*)lo);
+  mpn::launch(split_tf32_kernel<float>, (int)min((long long)kNumSMs * 8, (n / 4 + 255) / 256), 256, 0, st, x, n / 4, 4, nullptr, nullptr, nullptr, (float4*)hi, (float4*)lo);
   MPN_LAUNCH_OK();
   return MPN_OK;
 }
@@ -352,12 +353,12 @@ static int launch_tc(const CUtensorMap& ah, const CUtensorMap& al, const CUtenso
   return MPN_OK;
 }
 
-int gemm_nt_tc(const float* A, const float* B, const float* bias, float* C, int M, int N, int K, void* ws, size_t ws_bytes,
+int gemm_nt_tc(const void* A, const float* B, const float* bias, float* C, int M, int N, int K, void* ws, size_t ws_bytes,
                cudaStream_t st, const float* a_scale, const float* a_shift, const float* b_hi_cached, const float* b_lo_cached,
-               const int* row_gid) {
+               const int* row_gid, int a_kind) {
   MPN_REQUIRE(gemm_tc_supported(M, N, K), "tcgen05 GEMM: unsupported shape %d x %d x %d", M, N, K);
   MPN_REQUIRE(ws && ws_bytes >= gemm_tc_workspace_bytes(M, N, K), "tcgen05 GEMM: workspace too small");
-  MPN_REQUIRE((((uintptr_t)A | (uintptr_t)B) & 15) == 0, "tcgen05 GEMM: operands must be 16-byte aligned");
+  MPN_REQUIRE((((uintptr_t)B) & 15) == 0 && x_vec4_aligned(A, a_kind), "tcgen05 GEMM: operands must be aligned to four elements");
   char* w = (char*)(((uintptr_t)ws + 255) & ~(uintptr_t)255);
   const size_t plane_b = (((size_t)N * K * sizeof(float)) + 255) & ~(size_t)255;
   const size_t plane_a = (((size_t)M * K * sizeof(float)) + 255) & ~(size_t)255;
@@ -369,17 +370,22 @@ int gemm_nt_tc(const float* A, const float* B, const float* bias, float* C, int 
     b_hi = (float*)b_hi_cached;
     b_lo = (float*)b_lo_cached;
   } else {
-    mpn::launch(split_tf32_kernel, split_grid, 256, 0, st, (const float4*)B, (long long)N * K / 4, K, nullptr, nullptr, nullptr, (float4*)b_hi, (float4*)b_lo);
+    mpn::launch(split_tf32_kernel<float>, split_grid, 256, 0, st, B, (long long)N * K / 4, K, nullptr, nullptr, nullptr, (float4*)b_hi, (float4*)b_lo);
     MPN_LAUNCH_OK();
   }
-  if (a_scale == nullptr && A >= B && A + (size_t)M * K <= B + (size_t)N * K) {      // A is a row block of B (Gram matrix): share the planes
-    a_hi = b_hi + (A - B);
-    a_lo = b_lo + (A - B);
+  const float* Af = (const float*)A;
+  if (a_kind == MPN_X_F32 && a_scale == nullptr && Af >= B && Af + (size_t)M * K <= B + (size_t)N * K) {   // A is a row block of B (Gram matrix): share the planes
+    a_hi = b_hi + (Af - B);
+    a_lo = b_lo + (Af - B);
   } else {
     a_hi = (float*)(w + 2 * plane_b);
     a_lo = (float*)(w + 2 * plane_b + plane_a);
-    mpn::launch(split_tf32_kernel, split_grid, 256, 0, st, (const float4*)A, (long long)M * K / 4, K, a_scale, a_shift, row_gid, (float4*)a_hi, (float4*)a_lo);
-    MPN_LAUNCH_OK();
+    MPN_TRY(with_x_type(a_kind, [&](auto at) {
+      mpn::launch(split_tf32_kernel<x_elem_t<decltype(at)>>, split_grid, 256, 0, st, (decltype(at))A, (long long)M * K / 4, K, a_scale, a_shift, row_gid,
+                  (float4*)a_hi, (float4*)a_lo);
+      MPN_LAUNCH_OK();
+      return MPN_OK;
+    }));
   }
   CUtensorMap ah, al, bh, bl;
   static int forced_bn = -1;                         // diagnostics: MPN_TC_BN=128|256 overrides the tile width
@@ -393,7 +399,7 @@ int gemm_nt_tc(const float* A, const float* B, const float* bias, float* C, int 
   MPN_TRY(make_tma_map_2d(&al, a_lo, M, K, TC_BM, false));
   MPN_TRY(make_tma_map_2d(&bh, b_hi, N, K, BN, false));
   MPN_TRY(make_tma_map_2d(&bl, b_lo, N, K, BN, false));
-  const bool sym = (A == B) && (M == N) && bias == nullptr;     // Gram matrix: half the tiles
+  const bool sym = (Af == B) && (M == N) && bias == nullptr;    // Gram matrix: half the tiles
   if (BN == 256) return launch_tc<256, false>(ah, al, bh, bl, bias, C, M, N, K, st);
   if (sym) return launch_tc<128, true>(ah, al, bh, bl, bias, C, M, N, K, st);
   return launch_tc<128, false>(ah, al, bh, bl, bias, C, M, N, K, st);
@@ -401,7 +407,8 @@ int gemm_nt_tc(const float* A, const float* B, const float* bias, float* C, int 
 
 // fp16 operand planes with the fused input transform f(x)[m,k] = relu(x*scale[k] + shift[k]) of the previous encoder layer.
 // The plane scale comes from *amax_dev (float bits, device) when given, else from amax_host; out_scale = 1 / (s_a * b_scale).
-__global__ void __launch_bounds__(256) split_f16_bn_kernel(const float4* __restrict__ x, long long n4, int K, const float* __restrict__ scale,
+template <typename T>
+__global__ void __launch_bounds__(256) split_f16_bn_kernel(const T* __restrict__ x, long long n4, int K, const float* __restrict__ scale,
                                                            const float* __restrict__ shift, const int* __restrict__ row_gid,
                                                            const float* __restrict__ amax_dev, float amax_host, float b_scale,
                                                            uint2* __restrict__ hi, uint2* __restrict__ lo, float* __restrict__ out_scale) {
@@ -410,7 +417,7 @@ __global__ void __launch_bounds__(256) split_f16_bn_kernel(const float4* __restr
   if (out_scale && blockIdx.x == 0 && threadIdx.x == 0) *out_scale = (1.f / s) * (1.f / b_scale);
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
-    const float4 v = x[i];
+    const float4 v = ld4(x, i);
     float in[4] = {v.x, v.y, v.z, v.w};
     if (scale != nullptr) {
       const int k = (int)((i * 4) % K);
@@ -437,12 +444,13 @@ __global__ void __launch_bounds__(256) split_f16_bn_kernel(const float4* __restr
     lo[i] = pl;
   }
 }
-__global__ void __launch_bounds__(256) absmax_kernel(const float4* __restrict__ x, long long n4, unsigned int* __restrict__ amax_bits) {
+template <typename T>
+__global__ void __launch_bounds__(256) absmax_kernel(const T* __restrict__ x, long long n4, unsigned int* __restrict__ amax_bits) {
   pdl_wait();
   float m = 0.f;
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
-    const float4 v = x[i];
+    const float4 v = ld4(x, i);
     m = fmaxf(m, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
   }
 #pragma unroll
@@ -461,7 +469,7 @@ float f16_plane_scale_host(float amax) {
 int split_f16_host_scale(const float* x, long long n, float amax, void* hi, void* lo, float* scale_out, cudaStream_t st) {
   MPN_REQUIRE(x && hi && lo && n > 0 && (n % 4) == 0, "split_f16: bad arguments (n must be a positive multiple of 4)");
   MPN_REQUIRE((((uintptr_t)x | (uintptr_t)hi | (uintptr_t)lo) & 15) == 0, "split_f16: pointers must be 16-byte aligned");
-  mpn::launch(split_f16_bn_kernel, (int)min((long long)kNumSMs * 8, (n / 4 + 255) / 256), 256, 0, st, (const float4*)x, n / 4, 4, nullptr, nullptr, nullptr,
+  mpn::launch(split_f16_bn_kernel<float>, (int)min((long long)kNumSMs * 8, (n / 4 + 255) / 256), 256, 0, st, x, n / 4, 4, nullptr, nullptr, nullptr,
                                                                                            nullptr, amax, 1.f, (uint2*)hi, (uint2*)lo, nullptr);
   MPN_LAUNCH_OK();
   if (scale_out) *scale_out = f16_plane_scale_host(amax);
@@ -470,12 +478,13 @@ int split_f16_host_scale(const float* x, long long n, float amax, void* hi, void
 
 // C = f(A) B^T + bias on 3xFP16 planes: A split here (fused BatchNorm+ReLU of the previous layer), B planes cached.
 // a_amax_dev == nullptr && a_amax_host <= 0: max |A| is measured first (one pass over A; layer 0).
-int gemm_nt_tc_f16(const float* A, const float* bias, float* C, int M, int N, int K, void* ws, size_t ws_bytes, cudaStream_t st,
+int gemm_nt_tc_f16(const void* A, const float* bias, float* C, int M, int N, int K, void* ws, size_t ws_bytes, cudaStream_t st,
                    const float* a_scale, const float* a_shift, const int* row_gid, float a_amax_host, const void* b_hi16,
-                   const void* b_lo16, float b_scale) {
+                   const void* b_lo16, float b_scale, int a_kind) {
   MPN_REQUIRE(gemm_tc_supported(M, N, K) && (K % 8) == 0, "tcgen05 fp16-plane GEMM: unsupported shape %d x %d x %d", M, N, K);
   MPN_REQUIRE(ws && ws_bytes >= gemm_tc_workspace_bytes(M, N, K), "tcgen05 GEMM: workspace too small");
   MPN_REQUIRE(b_hi16 && b_lo16 && b_scale > 0.f, "tcgen05 fp16-plane GEMM: missing weight planes");
+  MPN_REQUIRE(x_vec4_aligned(A, a_kind), "tcgen05 fp16-plane GEMM: A must be aligned to four elements");
   char* w = (char*)(((uintptr_t)ws + 255) & ~(uintptr_t)255);
   const size_t plane = (((size_t)M * K * sizeof(__half)) + 255) & ~(size_t)255;
   __half* a_hi = (__half*)w;
@@ -483,15 +492,19 @@ int gemm_nt_tc_f16(const float* A, const float* bias, float* C, int M, int N, in
   float* out_scale = (float*)(w + 2 * plane);
   unsigned int* amax_bits = (unsigned int*)(w + 2 * plane + 256);
   const float* amax_dev = nullptr;
-  if (!(a_amax_host > 0.f)) {
-    MPN_CUDA_OK(cudaMemsetAsync(amax_bits, 0, sizeof(unsigned int), st));
-    mpn::launch(absmax_kernel, kNumSMs * 8, 256, 0, st, (const float4*)A, (long long)M * K / 4, amax_bits);
+  if (!(a_amax_host > 0.f)) MPN_CUDA_OK(cudaMemsetAsync(amax_bits, 0, sizeof(unsigned int), st));
+  MPN_TRY(with_x_type(a_kind, [&](auto at) {
+    using T = x_elem_t<decltype(at)>;
+    if (!(a_amax_host > 0.f)) {
+      mpn::launch(absmax_kernel<T>, kNumSMs * 8, 256, 0, st, (const T*)A, (long long)M * K / 4, amax_bits);
+      MPN_LAUNCH_OK();
+      amax_dev = (const float*)amax_bits;
+    }
+    mpn::launch(split_f16_bn_kernel<T>, kNumSMs * 8, 256, 0, st, (const T*)A, (long long)M * K / 4, K, a_scale, a_shift, row_gid, amax_dev,
+                a_amax_host, b_scale, (uint2*)a_hi, (uint2*)a_lo, out_scale);
     MPN_LAUNCH_OK();
-    amax_dev = (const float*)amax_bits;
-  }
-  mpn::launch(split_f16_bn_kernel, kNumSMs * 8, 256, 0, st, (const float4*)A, (long long)M * K / 4, K, a_scale, a_shift, row_gid, amax_dev, a_amax_host,
-                                                   b_scale, (uint2*)a_hi, (uint2*)a_lo, out_scale);
-  MPN_LAUNCH_OK();
+    return MPN_OK;
+  }));
   CUtensorMap ah, al, bh, bl;
   MPN_TRY(make_tma_map_2d(&ah, a_hi, M, K, TC_BM, true));
   MPN_TRY(make_tma_map_2d(&al, a_lo, M, K, TC_BM, true));
@@ -554,7 +567,7 @@ int gram_blockdiag_tc(const float* X, int N, int K, const int* graph_nptr, const
     return launch_tc<128, true, true>(mh16, ml16, mh16, ml16, nullptr, Gbuf, N, N, K, st, graph_nptr, g_off, n_graphs, max_ng, out_scale);
   }
   float *hi = (float*)w, *lo = (float*)(w + plane);
-  mpn::launch(split_tf32_kernel, kNumSMs * 8, 256, 0, st, (const float4*)X, (long long)N * K / 4, K, nullptr, nullptr, nullptr, (float4*)hi, (float4*)lo);
+  mpn::launch(split_tf32_kernel<float>, kNumSMs * 8, 256, 0, st, X, (long long)N * K / 4, K, nullptr, nullptr, nullptr, (float4*)hi, (float4*)lo);
   MPN_LAUNCH_OK();
   CUtensorMap mh, ml;
   MPN_TRY(make_tma_map_2d(&mh, hi, N, K, TC_BM, false));

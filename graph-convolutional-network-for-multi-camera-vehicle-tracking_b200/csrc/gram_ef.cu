@@ -81,7 +81,8 @@ __device__ __forceinline__ float rsqrt_approx(float x) {
 // row per step; block partials go to part[split][col]; the last row split of a column tile to finish adds that tile's partials in
 // a fixed order (one ticket counter per column tile).
 constexpr int GE_CM_SPLITS = 37;                             // 16 column tiles x 37 row splits = 592 blocks at D = 2048
-__global__ void __launch_bounds__(256) ge_col_mean_kernel(const float* __restrict__ x, int n, int D, int rows_per_split,
+template <typename T>
+__global__ void __launch_bounds__(256) ge_col_mean_kernel(const T* __restrict__ x, int n, int D, int rows_per_split,
                                                           double* __restrict__ part, unsigned int* __restrict__ ticket,
                                                           float* __restrict__ mu) {
   pdl_wait();
@@ -93,17 +94,18 @@ __global__ void __launch_bounds__(256) ge_col_mean_kernel(const float* __restric
   const int r0 = blockIdx.y * rows_per_split, r1 = min(r0 + rows_per_split, n);
   double s[4] = {0.0, 0.0, 0.0, 0.0};
   if (c4 < D4) {
-    const float4* p = reinterpret_cast<const float4*>(x) + c4;
+    const vec4_t<T>* p = reinterpret_cast<const vec4_t<T>*>(x) + c4;
     int r = r0 + warp;
-    for (; r + 24 < r1; r += 32) {                           // four independent 16-byte loads in flight per lane
-      const float4 v0 = p[(size_t)r * D4], v1 = p[(size_t)(r + 8) * D4], v2 = p[(size_t)(r + 16) * D4], v3 = p[(size_t)(r + 24) * D4];
+    for (; r + 24 < r1; r += 32) {                           // four independent vector loads in flight per lane
+      const float4 v0 = cvt4<T>(p[(size_t)r * D4]), v1 = cvt4<T>(p[(size_t)(r + 8) * D4]), v2 = cvt4<T>(p[(size_t)(r + 16) * D4]),
+                   v3 = cvt4<T>(p[(size_t)(r + 24) * D4]);
       s[0] += ((double)v0.x + (double)v1.x) + ((double)v2.x + (double)v3.x);
       s[1] += ((double)v0.y + (double)v1.y) + ((double)v2.y + (double)v3.y);
       s[2] += ((double)v0.z + (double)v1.z) + ((double)v2.z + (double)v3.z);
       s[3] += ((double)v0.w + (double)v1.w) + ((double)v2.w + (double)v3.w);
     }
     for (; r < r1; r += 8) {
-      const float4 v = p[(size_t)r * D4];
+      const float4 v = cvt4<T>(p[(size_t)r * D4]);
       s[0] += v.x; s[1] += v.y; s[2] += v.z; s[3] += v.w;
     }
   }
@@ -152,25 +154,28 @@ __global__ void __launch_bounds__(256) ge_col_mean_kernel(const float* __restric
 // before the gap, the gap length after it -> 32-ary search for the first k with col[beg+k] != k.  The row is "all columns but
 // [k, k+gl)" iff the entry after the gap is k+gl and the last entry is n_cols-1; any other row raises *not_one_gap.
 constexpr int GE_CS_WARPS = 4;
-template <bool STAGE>
-__global__ void __launch_bounds__(32 * GE_CS_WARPS) ge_center_split_kernel(const float* __restrict__ x, const float* __restrict__ mu, int n, int D,
+template <bool STAGE, typename T>
+__global__ void __launch_bounds__(32 * GE_CS_WARPS) ge_center_split_kernel(const T* __restrict__ x, const float* __restrict__ mu, int n, int D,
                                                               uint2* __restrict__ hi, uint2* __restrict__ lo, float4* __restrict__ rec,
                                                               float* __restrict__ scale_inv, const mpn_graph g, int2* __restrict__ gap,
                                                               int* __restrict__ not_one_gap) {
   pdl_wait();
-  extern __shared__ float4 cs_rows[];                        // STAGE: [GE_CS_WARPS][D / 4]
+  extern __shared__ float4 cs_rows[];                        // STAGE: [GE_CS_WARPS][D * sizeof(T) / 16]
+  constexpr bool KEEP_CENTRED = sizeof(T) == sizeof(float);  // fp32: the centred row replaces the staged one; 16-bit: re-centred
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int nwarps = (gridDim.x * blockDim.x) >> 5;
   const int D4 = D >> 2;
   const float4* mu4 = reinterpret_cast<const float4*>(mu);
-  float4* mine = cs_rows + (size_t)warp * D4;
+  const int D16 = D4 * (int)sizeof(T) / 4;                   // 16-byte chunks of a row
+  float4* mine = cs_rows + (size_t)warp * D16;
+  const T* srow = reinterpret_cast<const T*>(mine);
   for (int r = gwarp; r < n; r += nwarps) {
-    const float4* p = reinterpret_cast<const float4*>(x + (size_t)r * D);
+    const T* p = x + (size_t)r * D;
     if (STAGE) {                                             // the row's bytes are in flight while the gap search runs
       __syncwarp();
-      for (int k = lane; k < D4; k += 32)
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(mine + k)), "l"(p + k) : "memory");
+      for (int k = lane; k < D16; k += 32)
+        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(mine + k)), "l"(reinterpret_cast<const float4*>(p) + k) : "memory");
       asm volatile("cp.async.commit_group;" ::: "memory");
     }
     const int lr = r - g.row_offset;
@@ -203,11 +208,11 @@ __global__ void __launch_bounds__(32 * GE_CS_WARPS) ge_center_split_kernel(const
     double sq = 0.0, sx = 0.0, md = 0.0, mm = 0.0;
     float amax = 0.f;
     for (int k = lane; k < D4; k += 32) {
-      const float4 v = STAGE ? mine[k] : p[k];
+      const float4 v = ld4(STAGE ? srow : p, k);
       const float4 m = __ldg(mu4 + k);
       const float c[4] = {v.x - m.x, v.y - m.y, v.z - m.z, v.w - m.w};
       const float mv[4] = {m.x, m.y, m.z, m.w};
-      if (STAGE) mine[k] = make_float4(c[0], c[1], c[2], c[3]);
+      if (STAGE && KEEP_CENTRED) mine[k] = make_float4(c[0], c[1], c[2], c[3]);
       float q = 0.f, s1 = 0.f, d1 = 0.f, m2 = 0.f;           // four terms in fp32, then one conversion each
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
@@ -236,11 +241,11 @@ __global__ void __launch_bounds__(32 * GE_CS_WARPS) ge_center_split_kernel(const
     uint2* ol = lo + (size_t)r * D4;
     for (int k = lane; k < D4; k += 32) {
       float c[4];
-      if (STAGE) {
+      if (STAGE && KEEP_CENTRED) {
         const float4 cv = mine[k];
         c[0] = cv.x * s; c[1] = cv.y * s; c[2] = cv.z * s; c[3] = cv.w * s;
-      } else {
-        const float4 v = p[k], m = __ldg(mu4 + k);
+      } else {                                               // the same fp32 difference as the staged one, scaled
+        const float4 v = ld4(STAGE ? srow : p, k), m = __ldg(mu4 + k);
         c[0] = (v.x - m.x) * s; c[1] = (v.y - m.y) * s; c[2] = (v.z - m.z) * s; c[3] = (v.w - m.w) * s;
       }
       __half h[4], l[4];
@@ -691,29 +696,36 @@ bool gram_ef_shape_ok(int M, int N, int D) { return M >= 1 && N >= 2 && D >= GE_
 static int g_profile_gram = 0;
 static cudaEvent_t g_prof_ev[2] = {nullptr, nullptr};
 
-int ge_col_mean(const float* x, int n, int D, double* part, unsigned int* ticket, float* mu, cudaStream_t st) {
-  MPN_REQUIRE((D % 4) == 0 && (((uintptr_t)x) & 15) == 0, "column means: D must be a multiple of 4 and x 16-byte aligned");
+int ge_col_mean(const void* x, int x_kind, int n, int D, double* part, unsigned int* ticket, float* mu, cudaStream_t st) {
+  MPN_REQUIRE((D % 4) == 0 && x_vec4_aligned(x, x_kind), "column means: D must be a multiple of 4 and x aligned to four elements");
   const int splits = min(GE_CM_SPLITS, max(1, n / 8));
-  mpn::launch(ge_col_mean_kernel, dim3(div_up(D, 128), splits), 256, 0, st, x, n, D, div_up(n, splits), part, ticket, mu);
-  MPN_LAUNCH_OK();
-  return MPN_OK;
+  return with_x_type(x_kind, [&](auto xt) {
+    mpn::launch(ge_col_mean_kernel<x_elem_t<decltype(xt)>>, dim3(div_up(D, 128), splits), 256, 0, st, (decltype(xt))x, n, D, div_up(n, splits),
+                part, ticket, mu);
+    MPN_LAUNCH_OK();
+    return MPN_OK;
+  });
 }
 
-int gram_ef_run(const float* x, const float* mu, const mpn_graph* g, int D, int2* gap, int* not_one_gap, float2* edge_attr,
+int gram_ef_run(const void* x, int x_kind, const float* mu, const mpn_graph* g, int D, int2* gap, int* not_one_gap, float2* edge_attr,
                 int* refine_list, int* refine_count, double* partials, int* n_partial_rows, const GeWorkspace& L, cudaStream_t st,
                 const GeShare* share) {
   const int N = g->n_cols, M = g->n_nodes;
   MPN_REQUIRE(gram_ef_shape_ok(M, N, D), "fused edge features: unsupported shape M=%d N=%d D=%d", M, N, D);
   const int cs_grid = min(kNumSMs * 16, div_up((long long)N, GE_CS_WARPS));
-  const size_t cs_smem = (size_t)GE_CS_WARPS * D * sizeof(float);
-  if (cs_smem <= 48 * 1024) {                              // rows of up to 3072 floats are staged in shared memory
-    mpn::launch(ge_center_split_kernel<true>, cs_grid, 32 * GE_CS_WARPS, cs_smem, st, x, mu, N, D, (uint2*)L.hi, (uint2*)L.lo, L.rec, L.scale_inv, *g,
-                gap, not_one_gap);
-  } else {
-    mpn::launch(ge_center_split_kernel<false>, cs_grid, 32 * GE_CS_WARPS, 0, st, x, mu, N, D, (uint2*)L.hi, (uint2*)L.lo, L.rec, L.scale_inv, *g,
-                gap, not_one_gap);
-  }
-  MPN_LAUNCH_OK();
+  MPN_TRY(with_x_type(x_kind, [&](auto xt) {
+    using T = x_elem_t<decltype(xt)>;
+    const size_t cs_smem = (size_t)GE_CS_WARPS * D * sizeof(T);
+    if (cs_smem <= 48 * 1024) {                            // rows of up to 48 KB / GE_CS_WARPS are staged in shared memory
+      mpn::launch(ge_center_split_kernel<true, T>, cs_grid, 32 * GE_CS_WARPS, cs_smem, st, (const T*)x, mu, N, D, (uint2*)L.hi, (uint2*)L.lo, L.rec,
+                  L.scale_inv, *g, gap, not_one_gap);
+    } else {
+      mpn::launch(ge_center_split_kernel<false, T>, cs_grid, 32 * GE_CS_WARPS, 0, st, (const T*)x, mu, N, D, (uint2*)L.hi, (uint2*)L.lo, L.rec,
+                  L.scale_inv, *g, gap, not_one_gap);
+    }
+    MPN_LAUNCH_OK();
+    return MPN_OK;
+  }));
   GeShare sh;
   memset(&sh, 0, sizeof(sh));
   if (share != nullptr) {

@@ -45,9 +45,10 @@ int ge_workspace_layout(int n_cols, int M, int D, GeWorkspace* L, void* ws, size
 bool gram_ef_shape_ok(int M, int N, int D);
 // column means of x [n, D] (fp64 partial sums, fixed order): part [ge_col_mean_splits()][D] doubles, *ticket zeroed once
 int ge_col_mean_splits();
-int ge_col_mean(const float* x, int n, int D, double* part, unsigned int* ticket, float* mu, cudaStream_t st);
+// x: node features of element kind x_kind (MPN_X_*), read in place here and in gram_ef_run / edge_features_impl
+int ge_col_mean(const void* x, int x_kind, int n, int D, double* part, unsigned int* ticket, float* mu, cudaStream_t st);
 // fills gap / *not_one_gap (zeroed by the caller) for the rows of g, then runs the fused kernels
-int gram_ef_run(const float* x, const float* mu, const mpn_graph* g, int D, int2* gap, int* not_one_gap, float2* edge_attr,
+int gram_ef_run(const void* x, int x_kind, const float* mu, const mpn_graph* g, int D, int2* gap, int* not_one_gap, float2* edge_attr,
                 int* refine_list, int* refine_count, double* partials, int* n_partial_rows, const GeWorkspace& L, cudaStream_t st,
                 const GeShare* share = nullptr);
 
@@ -58,20 +59,22 @@ struct EfMoments {                 // in: partials [>= kNumSMs][MPN_SUMS_DOUBLES
   const int* handled_flag;         // out: device flag, 0 = features AND moments came from the fused kernel (nullptr: gather path)
   int known_fused;                 // out: 1 = the host already knows the fused kernel ran (the graph's layout hint)
 };
-int edge_features_impl(const mpn_graph* g, const float* x, int32_t D, float* edge_attr, int use_tc, void* ws, size_t ws_bytes,
+int edge_features_impl(const mpn_graph* g, const void* x, int x_kind, int32_t D, float* edge_attr, int use_tc, void* ws, size_t ws_bytes,
                        cudaStream_t st, EfMoments* moments, const GeShare* share = nullptr);   // share->mode is set here
 
 // gemm_simt.cu
-int gemm_nt_simt(const float* A, const float* B, const float* bias, const float* a_scale, const float* a_shift,
-                 float* C, int M, int N, int K, cudaStream_t st, const int* row_gid = nullptr);
+// a_kind: element kind of A (MPN_X_*; layer 0 of the node encoder reads x in place)
+int gemm_nt_simt(const void* A, const float* B, const float* bias, const float* a_scale, const float* a_shift,
+                 float* C, int M, int N, int K, cudaStream_t st, const int* row_gid = nullptr, int a_kind = MPN_X_F32);
 
 // gemm_tc.cu  (tcgen05 3xTF32; operands are pre-split hi/lo planes)
 size_t gemm_tc_workspace_bytes(int M, int N, int K);
 // a_scale/a_shift (optional, [K]): A is read as relu(A*scale + shift) while it is split (fused BatchNorm+ReLU)
-int gemm_nt_tc(const float* A, const float* B, const float* bias, float* C, int M, int N, int K,
+int gemm_nt_tc(const void* A, const float* B, const float* bias, float* C, int M, int N, int K,
                void* workspace, size_t workspace_bytes, cudaStream_t st, const float* a_scale = nullptr,
                const float* a_shift = nullptr, const float* b_hi_cached = nullptr, const float* b_lo_cached = nullptr,
-               const int* row_gid = nullptr);   // row_gid: a_scale/a_shift are [n_graphs][K] tables indexed by the row's graph
+               const int* row_gid = nullptr,    // row_gid: a_scale/a_shift are [n_graphs][K] tables indexed by the row's graph
+               int a_kind = MPN_X_F32);         // element kind of A (MPN_X_*)
 int split_tf32(const float* x, long long n, float* hi, float* lo, cudaStream_t st);
 // Gram block of the row block [a_row0, a_row0+M) of X [N,K] against all of X: 3xFP16 planes scaled by max|X| (amax_dev: float
 // bits on the device) when K % 8 == 0, else / when amax_dev is NULL the TF32 path of gemm_nt_tc
@@ -81,9 +84,9 @@ int gram_nt_tc(const float* X, int a_row0, float* C, int M, int N, int K, const 
 bool gemm_tc_supported(int M, int N, int K);
 // 3xFP16 variant for the node encoder: A is split here into fp16 planes (fused BatchNorm+ReLU; plane scale from a_amax_host, or
 // measured on the device when a_amax_host <= 0), B planes (b_hi16/b_lo16, scaled by b_scale) are cached by the caller
-int gemm_nt_tc_f16(const float* A, const float* bias, float* C, int M, int N, int K, void* workspace, size_t workspace_bytes,
+int gemm_nt_tc_f16(const void* A, const float* bias, float* C, int M, int N, int K, void* workspace, size_t workspace_bytes,
                    cudaStream_t st, const float* a_scale, const float* a_shift, const int* row_gid, float a_amax_host,
-                   const void* b_hi16, const void* b_lo16, float b_scale);
+                   const void* b_hi16, const void* b_lo16, float b_scale, int a_kind = MPN_X_F32);
 int split_f16_host_scale(const float* x, long long n, float amax, void* hi, void* lo, float* scale_out, cudaStream_t st);
 int gram_blockdiag_tc(const float* X, int N, int K, const int* graph_nptr, const long long* g_off, int n_graphs, int max_ng,
                       float* Gbuf, void* ws, size_t ws_bytes, cudaStream_t st, const float* amax_dev = nullptr);

@@ -1872,30 +1872,34 @@ static float encoder_input_bound(const mpn_fwd_plan* p, int l, int M_total) {
 
 // layers [l_begin, l_end) of the node encoder; l_end == n_node_layers also writes h.  The pieces of one forward are enqueued in
 // order on one stream (layer l reads the activations, column scale and shift that layer l-1 left in the plan's buffers).
-static int node_encoder_layers(mpn_fwd_plan* p, const float* x, int l_begin, int l_end, cudaStream_t st) {
+// x: node features of element kind x_kind (MPN_X_*), read in place by layer 0's operand split
+static int node_encoder_layers(mpn_fwd_plan* p, const void* x, int x_kind, int l_begin, int l_end, cudaStream_t st) {
   MPN_REQUIRE(p && x, "node_encoder: NULL argument");
+  MPN_X_KIND_OK(x_kind);
   const int M = p->g.n_cols;
   const bool batched = p->n_graphs > 1;
   if (l_begin == 0) MPN_CUDA_OK(cudaMemsetAsync(p->col_counter, 0, sizeof(unsigned int) * ((size_t)p->max_dim / 32 + 1), st));
   float* bufs[2] = {p->act0, p->act1};
-  const float* in = l_begin == 0 ? x : bufs[(l_begin - 1) & 1];
+  const void* in = l_begin == 0 ? x : bufs[(l_begin - 1) & 1];
+  int in_kind = l_begin == 0 ? x_kind : MPN_X_F32;
   const float *sc = l_begin == 0 ? nullptr : p->colscale, *sh = l_begin == 0 ? nullptr : p->colshift;
   for (int l = l_begin; l < l_end; ++l) {
     const int K = p->w.node_dims[l], Nc = p->w.node_dims[l + 1];
     float* out = bufs[l & 1];
     bool done = false;
     const int* gid = batched ? p->g.node_gid : nullptr;        // per-graph BatchNorm tables [G][K] when batched
-    if (p->use_tc && gemm_tc_supported(M, Nc, K)) {
+    // the operand splits read four elements at once; a layer-0 input that is not aligned to that takes the SIMT loader
+    if (p->use_tc && gemm_tc_supported(M, Nc, K) && x_vec4_aligned(in, in_kind)) {
       // tensor-core path: BatchNorm+ReLU of the previous layer is applied while the operand is split into its two planes
       if (encoder_f16(p, l, K))
         MPN_TRY(gemm_nt_tc_f16(in, p->w.node_b[l], out, M, Nc, K, p->gemm_ws, p->gemm_ws_bytes, st, sc, sh, gid,
-                               encoder_input_bound(p, l, M), p->w.node_w_hi16[l], p->w.node_w_lo16[l], p->w.node_w_scale16[l]));
+                               encoder_input_bound(p, l, M), p->w.node_w_hi16[l], p->w.node_w_lo16[l], p->w.node_w_scale16[l], in_kind));
       else
         MPN_TRY(gemm_nt_tc(in, p->w.node_w[l], p->w.node_b[l], out, M, Nc, K, p->gemm_ws, p->gemm_ws_bytes, st, sc, sh,
-                           p->w.node_w_hi[l], p->w.node_w_lo[l], gid));
+                           p->w.node_w_hi[l], p->w.node_w_lo[l], gid, in_kind));
       done = true;
     }
-    if (!done) MPN_TRY(gemm_nt_simt(in, p->w.node_w[l], p->w.node_b[l], sc, sh, out, M, Nc, K, st, gid));
+    if (!done) MPN_TRY(gemm_nt_simt(in, p->w.node_w[l], p->w.node_b[l], sc, sh, out, M, Nc, K, st, gid, in_kind));
     if (batched) {
       mpn::launch(colstats_graph_kernel, dim3(div_up(Nc, 32), p->n_graphs), 256, 0, st, out, Nc, p->g.graph_nptr, p->w.node_gamma[l],
                                                                               p->w.node_beta[l], p->colscale, p->colshift);
@@ -1908,40 +1912,49 @@ static int node_encoder_layers(mpn_fwd_plan* p, const float* x, int l_begin, int
     }
     MPN_LAUNCH_OK();
     in = out;
+    in_kind = MPN_X_F32;
     sc = p->colscale;
     sh = p->colshift;
   }
   if (l_end < p->w.n_node_layers) return MPN_OK;
-  mpn::launch(bn_relu_apply_kernel, min(kNumSMs * 4, div_up((long long)M * MPN_DH, 256)), 256, 0, st, in, (long long)M * MPN_DH, MPN_DH, sc, sh, batched ? p->g.node_gid : nullptr, p->h_full);
+  MPN_REQUIRE(in_kind == MPN_X_F32, "node_encoder: no encoder layer between x and h");
+  mpn::launch(bn_relu_apply_kernel, min(kNumSMs * 4, div_up((long long)M * MPN_DH, 256)), 256, 0, st, (const float*)in, (long long)M * MPN_DH, MPN_DH, sc, sh, batched ? p->g.node_gid : nullptr, p->h_full);
   MPN_LAUNCH_OK();
   return MPN_OK;
 }
 
-int mpn_plan_node_encoder(mpn_fwd_plan* p, const float* x, void* stream) {
+int mpn_plan_node_encoder_x(mpn_fwd_plan* p, const void* x, int32_t x_kind, void* stream) {
   MPN_REQUIRE(p && x, "node_encoder: NULL argument");
-  return node_encoder_layers(p, x, 0, p->w.n_node_layers, (cudaStream_t)stream);
+  return node_encoder_layers(p, x, x_kind, 0, p->w.n_node_layers, (cudaStream_t)stream);
 }
+
+int mpn_plan_node_encoder(mpn_fwd_plan* p, const float* x, void* stream) { return mpn_plan_node_encoder_x(p, x, MPN_X_F32, stream); }
 
 // node encoder over this rank's row block only; BatchNorm column sums all-reduced through peer memory per layer;
 // the encoded rows land in every rank's h buffer (publish of the h flag is left to the caller)
-static int node_encoder_sharded(mpn_fwd_plan* p, const float* x, const PeerArgs& P, unsigned long long& seq_c, cudaStream_t st,
+static int node_encoder_sharded(mpn_fwd_plan* p, const void* x, int x_kind, const PeerArgs& P, unsigned long long& seq_c, cudaStream_t st,
                                 int l_begin, int l_end) {                 // layers [l_begin, l_end), as node_encoder_layers
   const int M = p->g.n_nodes, off = p->g.row_offset;
   float* bufs[2] = {p->act0, p->act1};
-  const float* in = l_begin == 0 ? x + (size_t)off * p->w.node_dims[0] : bufs[(l_begin - 1) & 1];
+  const void* in = l_begin == 0 ? (const void*)((const char*)x + (size_t)off * p->w.node_dims[0] * x_elem_bytes(x_kind))
+                                 : (const void*)bufs[(l_begin - 1) & 1];
+  int in_kind = l_begin == 0 ? x_kind : MPN_X_F32;
   const float *sc = l_begin == 0 ? nullptr : p->colscale, *sh = l_begin == 0 ? nullptr : p->colshift;
   for (int l = l_begin; l < l_end; ++l) {
     const int K = p->w.node_dims[l], Nc = p->w.node_dims[l + 1];
     MPN_REQUIRE(Nc <= MPN_PEER_CSTAT_COLS, "sharded node encoder: layer width %d > %d", Nc, MPN_PEER_CSTAT_COLS);
     float* out = bufs[l & 1];
-    if (p->use_tc && gemm_tc_supported(M, Nc, K) && encoder_f16(p, l, K))
+    // a 16-bit row block at offset off*K is aligned to four elements only when off*K % 4 == 0: else the SIMT loader
+    const bool tc = p->use_tc && gemm_tc_supported(M, Nc, K) && x_vec4_aligned(in, in_kind);
+    if (tc && encoder_f16(p, l, K))
       MPN_TRY(gemm_nt_tc_f16(in, p->w.node_b[l], out, M, Nc, K, p->gemm_ws, p->gemm_ws_bytes, st, sc, sh, nullptr,
-                             encoder_input_bound(p, l, p->g.n_cols), p->w.node_w_hi16[l], p->w.node_w_lo16[l], p->w.node_w_scale16[l]));
-    else if (p->use_tc && gemm_tc_supported(M, Nc, K))
+                             encoder_input_bound(p, l, p->g.n_cols), p->w.node_w_hi16[l], p->w.node_w_lo16[l], p->w.node_w_scale16[l],
+                             in_kind));
+    else if (tc)
       MPN_TRY(gemm_nt_tc(in, p->w.node_w[l], p->w.node_b[l], out, M, Nc, K, p->gemm_ws, p->gemm_ws_bytes, st, sc, sh,
-                         p->w.node_w_hi[l], p->w.node_w_lo[l], nullptr));
+                         p->w.node_w_hi[l], p->w.node_w_lo[l], nullptr, in_kind));
     else
-      MPN_TRY(gemm_nt_simt(in, p->w.node_w[l], p->w.node_b[l], sc, sh, out, M, Nc, K, st, nullptr));
+      MPN_TRY(gemm_nt_simt(in, p->w.node_w[l], p->w.node_b[l], sc, sh, out, M, Nc, K, st, nullptr, in_kind));
     int splits = div_up(M, 256);
     splits = splits > CS_ROWSPLIT_MAX ? CS_ROWSPLIT_MAX : splits;
     const int rps = div_up(M, splits);
@@ -1952,11 +1965,13 @@ static int node_encoder_sharded(mpn_fwd_plan* p, const float* x, const PeerArgs&
                                             p->colshift, P, ++seq_c);
     MPN_LAUNCH_OK();
     in = out;
+    in_kind = MPN_X_F32;
     sc = p->colscale;
     sh = p->colshift;
   }
   if (l_end < p->w.n_node_layers) return MPN_OK;
-  mpn::launch(bn_relu_apply_peer_kernel, min(kNumSMs * 4, div_up((long long)M * MPN_DH, 256)), 256, 0, st, in, M, off, sc, sh, P);
+  MPN_REQUIRE(in_kind == MPN_X_F32, "node_encoder: no encoder layer between x and h");
+  mpn::launch(bn_relu_apply_peer_kernel, min(kNumSMs * 4, div_up((long long)M * MPN_DH, 256)), 256, 0, st, (const float*)in, M, off, sc, sh, P);
   MPN_LAUNCH_OK();
   return MPN_OK;
 }
@@ -2174,11 +2189,12 @@ static void tl_mark(const char* name, cudaStream_t st, bool first = false) {
 
 // ef_ws != NULL: edge_attr is an OUTPUT, produced here by mpn_edge_features on the main stream while the node encoder runs on
 // the side stream (both only read x)
-static int forward_impl(const mpn_graph* g, const mpn_weights* w, const float* x, float* edge_attr_rw, int32_t L, int32_t n_cls,
-                        float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out, int use_tc, void* ws, size_t ws_bytes,
-                        void* ef_ws, size_t ef_ws_bytes, void* stream) {
+static int forward_impl(const mpn_graph* g, const mpn_weights* w, const void* x, int x_kind, float* edge_attr_rw, int32_t L,
+                        int32_t n_cls, float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out, int use_tc, void* ws,
+                        size_t ws_bytes, void* ef_ws, size_t ef_ws_bytes, void* stream) {
   const float* edge_attr = edge_attr_rw;
   MPN_REQUIRE(g && x && edge_attr && logits_out, "forward: NULL argument");
+  MPN_X_KIND_OK(x_kind);
   MPN_REQUIRE(g->row_offset == 0 && g->n_cols == g->n_nodes, "mpn_forward runs an unsharded graph; use the plan API for row blocks");
   cudaStream_t st = (cudaStream_t)stream;
   mpn_fwd_plan* p = nullptr;
@@ -2200,13 +2216,13 @@ static int forward_impl(const mpn_graph* g, const mpn_weights* w, const float* x
     bool encoder_enqueued = false;
     int enc_done_layers = 0;
 #define ENQUEUE_ENCODER() do { if (!encoder_enqueued) { encoder_enqueued = true; \
-      STEP_TRY(node_encoder_layers(p, x, enc_done_layers, p->w.n_node_layers, fork ? ss->stream : st)); \
+      STEP_TRY(node_encoder_layers(p, x, x_kind, enc_done_layers, p->w.n_node_layers, fork ? ss->stream : st)); \
       tl_mark("node_encoder_end(side stream)", fork ? ss->stream : st); \
       if (fork && cudaEventRecord(ss->join, ss->stream) != cudaSuccess) { set_error("event record failed"); rc = MPN_ERR_CUDA; goto done; } } } while (0)
     if (!fork || ef_ws == nullptr) ENQUEUE_ENCODER();
     else if (p->w.n_node_layers > 1) {
       // the first (largest) encoder layer starts on the idle device; the later, small ones fit beside the Gram kernel
-      STEP_TRY(node_encoder_layers(p, x, 0, 1, ss->stream));
+      STEP_TRY(node_encoder_layers(p, x, x_kind, 0, 1, ss->stream));
       enc_done_layers = 1;
     }
     bool enc0_done = false;
@@ -2217,7 +2233,7 @@ static int forward_impl(const mpn_graph* g, const mpn_weights* w, const float* x
       if (clear_moment_state(p, st) != cudaSuccess) { set_error("memset failed"); rc = MPN_ERR_CUDA; goto done; }
       EfMoments mom;
       mom.partials = p->partials; mom.fixed_sums = p->fix_sums; mom.handled_flag = nullptr; mom.known_fused = 0;
-      STEP_TRY(edge_features_impl(g, x, w->node_dims[0], edge_attr_rw, use_tc, ef_ws, ef_ws_bytes, st, &mom));
+      STEP_TRY(edge_features_impl(g, x, x_kind, w->node_dims[0], edge_attr_rw, use_tc, ef_ws, ef_ws_bytes, st, &mom));
       ENQUEUE_ENCODER();
       if (mom.handled_flag != nullptr) {
         if (!mom.known_fused) {
@@ -2238,7 +2254,7 @@ static int forward_impl(const mpn_graph* g, const mpn_weights* w, const float* x
         enc0_done = true;
       }
     } else if (ef_ws != nullptr) {
-      STEP_TRY(mpn_edge_features(g, x, w->node_dims[0], edge_attr_rw, use_tc, ef_ws, ef_ws_bytes, st));
+      STEP_TRY(edge_features_impl(g, x, x_kind, w->node_dims[0], edge_attr_rw, use_tc, ef_ws, ef_ws_bytes, st, nullptr));
     }
     ENQUEUE_ENCODER();
 #undef ENQUEUE_ENCODER
@@ -2282,28 +2298,43 @@ done:
   return rc;
 }
 
+int mpn_forward_x(const mpn_graph* g, const mpn_weights* w, const void* x, int32_t x_kind, const float* edge_attr, int32_t L,
+                  int32_t n_cls, float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out, int use_tc, void* ws,
+                  size_t ws_bytes, void* stream) {
+  return forward_impl(g, w, x, x_kind, const_cast<float*>(edge_attr), L, n_cls, logits_out, h_out, pred_out, prob1_out, use_tc, ws,
+                      ws_bytes, nullptr, 0, stream);
+}
+
 int mpn_forward(const mpn_graph* g, const mpn_weights* w, const float* x, const float* edge_attr, int32_t L, int32_t n_cls,
                 float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out, int use_tc, void* ws, size_t ws_bytes,
                 void* stream) {
-  return forward_impl(g, w, x, const_cast<float*>(edge_attr), L, n_cls, logits_out, h_out, pred_out, prob1_out, use_tc, ws, ws_bytes,
-                      nullptr, 0, stream);
+  return mpn_forward_x(g, w, x, MPN_X_F32, edge_attr, L, n_cls, logits_out, h_out, pred_out, prob1_out, use_tc, ws, ws_bytes, stream);
+}
+
+int mpn_forward_with_edge_features_x(const mpn_graph* g, const mpn_weights* w, const void* x, int32_t x_kind, float* edge_attr_out,
+                                     int32_t L, int32_t n_cls, float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out,
+                                     int use_tc, void* ws, size_t ws_bytes, void* ef_ws, size_t ef_ws_bytes, void* stream) {
+  MPN_REQUIRE(ef_ws != nullptr && edge_attr_out != nullptr, "forward_with_edge_features: NULL edge-feature buffer / workspace");
+  return forward_impl(g, w, x, x_kind, edge_attr_out, L, n_cls, logits_out, h_out, pred_out, prob1_out, use_tc, ws, ws_bytes, ef_ws,
+                      ef_ws_bytes, stream);
 }
 
 int mpn_forward_with_edge_features(const mpn_graph* g, const mpn_weights* w, const float* x, float* edge_attr_out, int32_t L,
                                    int32_t n_cls, float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out, int use_tc,
                                    void* ws, size_t ws_bytes, void* ef_ws, size_t ef_ws_bytes, void* stream) {
-  MPN_REQUIRE(ef_ws != nullptr && edge_attr_out != nullptr, "forward_with_edge_features: NULL edge-feature buffer / workspace");
-  return forward_impl(g, w, x, edge_attr_out, L, n_cls, logits_out, h_out, pred_out, prob1_out, use_tc, ws, ws_bytes, ef_ws,
-                      ef_ws_bytes, stream);
+  return mpn_forward_with_edge_features_x(g, w, x, MPN_X_F32, edge_attr_out, L, n_cls, logits_out, h_out, pred_out, prob1_out, use_tc,
+                                          ws, ws_bytes, ef_ws, ef_ws_bytes, stream);
 }
 
 // ef_ws != NULL: edge_attr is an OUTPUT, produced here by the fused edge-feature kernel on the caller's stream (it overlaps the
 // node encoder on the side stream and hands over the first encoder BatchNorm's moment sums: no ENC0 sweep)
-static int forward_sharded_impl(const mpn_graph* g, const mpn_weights* w, const float* x, float* edge_attr_rw, int32_t L, int32_t n_cls,
-                                int64_t total_edges, float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out, int use_tc,
-                                const mpn_peer_ctx* peers, void* ws, size_t ws_bytes, void* ef_ws, size_t ef_ws_bytes, void* stream) {
+static int forward_sharded_impl(const mpn_graph* g, const mpn_weights* w, const void* x, int x_kind, float* edge_attr_rw, int32_t L,
+                                int32_t n_cls, int64_t total_edges, float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out,
+                                int use_tc, const mpn_peer_ctx* peers, void* ws, size_t ws_bytes, void* ef_ws, size_t ef_ws_bytes,
+                                void* stream) {
   const float* edge_attr = edge_attr_rw;
   MPN_REQUIRE(g && x && edge_attr && logits_out && peers, "forward_sharded: NULL argument");
+  MPN_X_KIND_OK(x_kind);
   MPN_REQUIRE(peers->world >= 1 && peers->world <= MPN_MAX_PEERS && peers->rank >= 0 && peers->rank < peers->world, "forward_sharded: bad rank/world");
   MPN_REQUIRE(g->n_graphs <= 1, "forward_sharded: batched graphs cannot be row-sharded");
   MPN_REQUIRE(L >= 1, "forward_sharded needs num_enc_steps >= 1");
@@ -2366,7 +2397,7 @@ static int forward_sharded_impl(const mpn_graph* g, const mpn_weights* w, const 
       if (clear_moment_state(p, st) != cudaSuccess) { set_error("memset failed"); rc = MPN_ERR_CUDA; goto done; } \
       EfMoments mom_; \
       mom_.partials = p->partials; mom_.fixed_sums = p->fix_sums; mom_.handled_flag = nullptr; mom_.known_fused = 0; \
-      STEP_TRY(edge_features_impl(g, x, w->node_dims[0], edge_attr_rw, use_tc, ef_ws, ef_ws_bytes, st, &mom_, share_ptr)); \
+      STEP_TRY(edge_features_impl(g, x, x_kind, w->node_dims[0], edge_attr_rw, use_tc, ef_ws, ef_ws_bytes, st, &mom_, share_ptr)); \
       if (mom_.handled_flag != nullptr) { \
         if (!mom_.known_fused) {   /* layout decided on the device: the sweep runs only if the fused kernel did not */ \
           const int fg_ = (int)min((long long)SWEEP_GRID, (long long)div_up(g->n_edges > 0 ? g->n_edges : 1, SWEEP_THREADS)); \
@@ -2395,11 +2426,11 @@ static int forward_sharded_impl(const mpn_graph* g, const mpn_weights* w, const 
     cudaStream_t es = fork ? ss->stream : st;
     // enqueue order as in forward_impl: first encoder layer, edge features (they head the critical path), later layers
     const int n_first = (fork && ef_ws != nullptr && p->w.n_node_layers > 1) ? 1 : p->w.n_node_layers;
-    STEP_TRY(node_encoder_sharded(p, x, P, seq_c, es, 0, n_first));
+    STEP_TRY(node_encoder_sharded(p, x, x_kind, P, seq_c, es, 0, n_first));
     if (n_first < p->w.n_node_layers) {
       ENC0_STAGE();
       tl_mark("edge_features+enc0_end", st);
-      STEP_TRY(node_encoder_sharded(p, x, P, seq_c, es, n_first, p->w.n_node_layers));
+      STEP_TRY(node_encoder_sharded(p, x, x_kind, P, seq_c, es, n_first, p->w.n_node_layers));
     }
     mpn::launch(peer_publish_h_kernel, 1, 32, 0, es, P, ++seq_h);
     ++mpn::g_kernel_launches;
@@ -2417,7 +2448,7 @@ static int forward_sharded_impl(const mpn_graph* g, const mpn_weights* w, const 
   } else {
     SideStream* ss = side_stream();
     const bool fork = ss != nullptr && cudaEventRecord(ss->fork, st) == cudaSuccess && cudaStreamWaitEvent(ss->stream, ss->fork, 0) == cudaSuccess;
-    STEP_TRY(mpn_plan_node_encoder(p, x, fork ? ss->stream : st));
+    STEP_TRY(mpn_plan_node_encoder_x(p, x, x_kind, fork ? ss->stream : st));
     if (fork && cudaEventRecord(ss->join, ss->stream) != cudaSuccess) { set_error("event record failed"); rc = MPN_ERR_CUDA; goto done; }
     ENC0_STAGE();
     STEP_TRY(mpn_plan_sweep(p, 0, MPN_STAGE_ENC1, edge_attr, nullptr, nullptr, nullptr, st));
@@ -2472,20 +2503,35 @@ done:
   return rc;
 }
 
+int mpn_forward_sharded_x(const mpn_graph* g, const mpn_weights* w, const void* x, int32_t x_kind, const float* edge_attr, int32_t L,
+                          int32_t n_cls, int64_t total_edges, float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out,
+                          int use_tc, const mpn_peer_ctx* peers, void* ws, size_t ws_bytes, void* stream) {
+  return forward_sharded_impl(g, w, x, x_kind, const_cast<float*>(edge_attr), L, n_cls, total_edges, logits_out, h_out, pred_out,
+                              prob1_out, use_tc, peers, ws, ws_bytes, nullptr, 0, stream);
+}
+
 int mpn_forward_sharded(const mpn_graph* g, const mpn_weights* w, const float* x, const float* edge_attr, int32_t L, int32_t n_cls,
                         int64_t total_edges, float* logits_out, float* h_out, uint8_t* pred_out, float* prob1_out, int use_tc,
                         const mpn_peer_ctx* peers, void* ws, size_t ws_bytes, void* stream) {
-  return forward_sharded_impl(g, w, x, const_cast<float*>(edge_attr), L, n_cls, total_edges, logits_out, h_out, pred_out, prob1_out, use_tc,
-                              peers, ws, ws_bytes, nullptr, 0, stream);
+  return mpn_forward_sharded_x(g, w, x, MPN_X_F32, edge_attr, L, n_cls, total_edges, logits_out, h_out, pred_out, prob1_out, use_tc,
+                               peers, ws, ws_bytes, stream);
+}
+
+int mpn_forward_sharded_with_edge_features_x(const mpn_graph* g, const mpn_weights* w, const void* x, int32_t x_kind,
+                                             float* edge_attr_out, int32_t L, int32_t n_cls, int64_t total_edges, float* logits_out,
+                                             float* h_out, uint8_t* pred_out, float* prob1_out, int use_tc, const mpn_peer_ctx* peers,
+                                             void* ws, size_t ws_bytes, void* ef_ws, size_t ef_ws_bytes, void* stream) {
+  MPN_REQUIRE(ef_ws != nullptr && edge_attr_out != nullptr, "forward_sharded_with_edge_features: NULL edge-feature buffer / workspace");
+  return forward_sharded_impl(g, w, x, x_kind, edge_attr_out, L, n_cls, total_edges, logits_out, h_out, pred_out, prob1_out, use_tc,
+                              peers, ws, ws_bytes, ef_ws, ef_ws_bytes, stream);
 }
 
 int mpn_forward_sharded_with_edge_features(const mpn_graph* g, const mpn_weights* w, const float* x, float* edge_attr_out, int32_t L,
                                            int32_t n_cls, int64_t total_edges, float* logits_out, float* h_out, uint8_t* pred_out,
                                            float* prob1_out, int use_tc, const mpn_peer_ctx* peers, void* ws, size_t ws_bytes,
                                            void* ef_ws, size_t ef_ws_bytes, void* stream) {
-  MPN_REQUIRE(ef_ws != nullptr && edge_attr_out != nullptr, "forward_sharded_with_edge_features: NULL edge-feature buffer / workspace");
-  return forward_sharded_impl(g, w, x, edge_attr_out, L, n_cls, total_edges, logits_out, h_out, pred_out, prob1_out, use_tc, peers, ws,
-                              ws_bytes, ef_ws, ef_ws_bytes, stream);
+  return mpn_forward_sharded_with_edge_features_x(g, w, x, MPN_X_F32, edge_attr_out, L, n_cls, total_edges, logits_out, h_out, pred_out,
+                                                  prob1_out, use_tc, peers, ws, ws_bytes, ef_ws, ef_ws_bytes, stream);
 }
 
 int mpn_pack_decisions(const uint8_t* pred, int64_t E, uint32_t* words_out, void* stream) {

@@ -58,6 +58,23 @@ def current_stream_ptr(device: torch.device) -> int:
     return torch.cuda.current_stream(device).cuda_stream
 
 
+_X_KINDS = {torch.float32: _lib.MPN_X_F32, torch.float16: _lib.MPN_X_F16, torch.bfloat16: _lib.MPN_X_BF16}
+
+
+def node_features(x: torch.Tensor):
+    """(contiguous x, its MPN_X_* element kind) for the kernels that read node features.  fp32, fp16 and bf16 are read in
+    place, converted to fp32 element by element on load (exact: every output equals the one on ``x.float()``); any other
+    dtype is converted to fp32 first."""
+    if x.dtype not in _X_KINDS:
+        x = x.float()
+    x = x.contiguous()
+    if x.element_size() == 2 and x.data_ptr() % 16:
+        # a view at an odd offset: the kernels take the same paths as on x.float() (16-byte row copies, four-element vector
+        # loads) only from an aligned base, so the 16-bit rows are copied once to a fresh allocation
+        x = x.clone()
+    return x, _X_KINDS[x.dtype]
+
+
 class _NoContext:
     def __enter__(self):
         return self

@@ -16,32 +16,38 @@ import numpy as np
 import torch
 
 from . import _lib
-from .graph import TrackletGraph, current_stream_ptr, graph_for, host_node_ptr, workspace
+from .graph import TrackletGraph, current_stream_ptr, graph_for, host_node_ptr, node_features, workspace
 
 
 def normalize_columns(x: torch.Tensor, out: torch.Tensor = None, ptr=None) -> torch.Tensor:
     """``F.normalize(x, p=2, dim=0)``: every feature column scaled to unit L2 norm over the nodes (eps 1e-12).
     ``ptr``: G+1 node offsets of a batch (PyG ``Batch.ptr``): every graph's rows ``x[ptr[g]:ptr[g+1]]`` are normalised on
-    their own, as inference.py:403-404 does inside the loop over graphs, in one kernel."""
+    their own, as inference.py:403-404 does inside the loop over graphs, in one kernel.
+    ``x`` may be fp32, fp16 or bf16 (16-bit features are read in place); the result is always fp32, equal to the one on
+    ``x.float()``.  ``out``: a contiguous fp32 tensor of x's shape on x's device (``out=x`` normalises an fp32 x in place)."""
     if not x.is_cuda:
         raise RuntimeError("normalize_columns needs a CUDA tensor: the B200 path has no CPU fallback")
     if x.dim() != 2:
         raise ValueError("x must be [N, D]")
+    if out is not None and (out.dtype != torch.float32 or out.shape != x.shape or out.device != x.device
+                            or not out.is_contiguous()):
+        raise ValueError("out must be a contiguous float32 tensor of x's shape %s on %s (got %s %s on %s)"
+                         % (tuple(x.shape), x.device, out.dtype, tuple(out.shape), out.device))
     nptr = host_node_ptr(ptr, x.shape[0]) if ptr is not None else None
-    x = x.contiguous().float()
-    out = torch.empty_like(x) if out is None else out
+    x, x_kind = node_features(x)
+    out = torch.empty(x.shape, dtype=torch.float32, device=x.device) if out is None else out
     L = _lib.lib()
     stream = current_stream_ptr(x.device)
     with torch.cuda.device(x.device):
         if nptr is not None and nptr.size > 2:
             pinned = torch.from_numpy(nptr.astype(np.int32)).pin_memory()
             gptr = pinned.to(x.device, non_blocking=True)
-            _lib.check(L.mpn_normalize_columns_batched(x.data_ptr(), x.shape[0], x.shape[1], gptr.data_ptr(), nptr.size - 1,
-                                                       out.data_ptr(), None, 0, stream))
+            _lib.check(L.mpn_normalize_columns_batched_x(x.data_ptr(), x_kind, x.shape[0], x.shape[1], gptr.data_ptr(),
+                                                         nptr.size - 1, out.data_ptr(), None, 0, stream))
         else:
             ws = workspace("normalize_columns", x.device, L.mpn_normalize_columns_workspace_bytes(x.shape[1]))
-            _lib.check(L.mpn_normalize_columns(x.data_ptr(), x.shape[0], x.shape[1], out.data_ptr(), ws.data_ptr(), ws.numel(),
-                                               stream))
+            _lib.check(L.mpn_normalize_columns_x(x.data_ptr(), x_kind, x.shape[0], x.shape[1], out.data_ptr(), ws.data_ptr(),
+                                                 ws.numel(), stream))
     return out
 
 
@@ -68,6 +74,8 @@ def edge_labels(node_labels, edge_index: torch.Tensor = None, graph: TrackletGra
 
 # ------------------------------------------------------------------------------------------------ packed ReID features
 MAGIC = b"MPNFEAT1"
+# header dtype -> element type of the feature matrix (bfloat16 is stored as its raw 16-bit words)
+_PACKED_DTYPES = {"float32": torch.float32, "float16": torch.float16, "bfloat16": torch.bfloat16}
 
 
 def reid_feature_path(root, scenario, id_cam, track_id, file, cnn_model_name):
@@ -76,17 +84,25 @@ def reid_feature_path(root, scenario, id_cam, track_id, file, cnn_model_name):
                         file + '_' + cnn_model_name + '.pkl')
 
 
-def pack_reid_features(path, features, cam_ids, track_ids):
-    """Write one packed file: header (JSON) + id_cam int64[N] + id int64[N] + features float32[N,D] (row-major, 4096-byte
-    aligned so the matrix can be mapped).  ``features``: [N,D] array / tensor, or a list of per-tracklet vectors."""
-    if isinstance(features, (list, tuple)):
-        features = np.stack([np.asarray(f.cpu() if torch.is_tensor(f) else f, dtype=np.float32).reshape(-1) for f in features])
-    x = np.ascontiguousarray(features.cpu().numpy() if torch.is_tensor(features) else features, dtype=np.float32)
+def pack_reid_features(path, features, cam_ids, track_ids, dtype="float32"):
+    """Write one packed file: header (JSON) + id_cam int64[N] + id int64[N] + features [N,D] (row-major, 4096-byte aligned so
+    the matrix can be mapped).  ``features``: [N,D] array / tensor, or a list of per-tracklet vectors.  ``dtype``: element type
+    stored, ``"float32"``, ``"float16"`` or ``"bfloat16"`` (or the torch dtype); fp32 values are rounded to nearest even.
+    Half-width files halve the bytes read and copied to the device; the features are then exact 16-bit values."""
+    name = str(dtype).replace("torch.", "")
+    if name not in _PACKED_DTYPES:
+        raise ValueError("dtype must be float32, float16 or bfloat16 (got %r)" % (dtype,))
+    if isinstance(features, (list, tuple)):                       # (.float(): numpy has no bfloat16; the widening is exact)
+        features = np.stack([np.asarray(f.detach().cpu().float() if torch.is_tensor(f) else f, dtype=np.float32).reshape(-1)
+                             for f in features])
+    x = np.ascontiguousarray(features.detach().cpu().float().numpy() if torch.is_tensor(features) else features, dtype=np.float32)
+    if name != "float32":                                        # 16-bit: raw words of the rounded values
+        x = torch.from_numpy(x).to(_PACKED_DTYPES[name]).view(torch.int16).numpy()
     cam = np.ascontiguousarray(np.asarray(cam_ids), dtype=np.int64).reshape(-1)
     tid = np.ascontiguousarray(np.asarray(track_ids), dtype=np.int64).reshape(-1)
     if x.ndim != 2 or not (x.shape[0] == cam.size == tid.size):
         raise ValueError("features must be [N,D] with one camera id and one track id per row")
-    header = json.dumps({"n": int(x.shape[0]), "d": int(x.shape[1]), "dtype": "float32"}).encode()
+    header = json.dumps({"n": int(x.shape[0]), "d": int(x.shape[1]), "dtype": name}).encode()
     pre = len(MAGIC) + 8 + len(header) + cam.nbytes + tid.nbytes
     pad = (-pre) % 4096
     with open(path, "wb") as f:
@@ -110,34 +126,47 @@ def pack_reid_features_from_pickles(path, root, scenario, file, cnn_model_name, 
 
 
 def read_packed_features(path):
-    """Host view of a packed file: (features float32 [N,D] memory-mapped, id_cam int64 [N], id int64 [N])."""
+    """Host view of a packed file: (features [N,D] memory-mapped, id_cam int64 [N], id int64 [N]).  The features keep the
+    file's element type: a numpy float32 / float16 array, or for bfloat16 (which numpy lacks) a torch.bfloat16 tensor over a
+    copy-on-write mapping of the file."""
     with open(path, "rb") as f:
         if f.read(len(MAGIC)) != MAGIC:
             raise ValueError("%s is not a packed ReID feature file" % path)
         hlen = int(np.frombuffer(f.read(8), dtype=np.int64)[0])
         h = json.loads(f.read(hlen).decode())
         n, d = int(h["n"]), int(h["d"])
+        name = h.get("dtype", "float32")
+        if name not in _PACKED_DTYPES:
+            raise ValueError("%s: unknown feature dtype %r in the header" % (path, name))
         cam = np.frombuffer(f.read(8 * n), dtype=np.int64).copy()
         tid = np.frombuffer(f.read(8 * n), dtype=np.int64).copy()
         pre = len(MAGIC) + 8 + hlen + 16 * n
         off = pre + ((-pre) % 4096)
-    x = np.memmap(path, dtype=np.float32, mode="r", offset=off, shape=(n, d)) if n else np.zeros((0, d), dtype=np.float32)
+    if name == "bfloat16":
+        words = np.memmap(path, dtype=np.int16, mode="c", offset=off, shape=(n, d)) if n else np.zeros((0, d), dtype=np.int16)
+        return torch.from_numpy(words).view(torch.bfloat16), cam, tid
+    npt = np.float32 if name == "float32" else np.float16
+    x = np.memmap(path, dtype=npt, mode="r", offset=off, shape=(n, d)) if n else np.zeros((0, d), dtype=npt)
     return x, cam, tid
 
 
 def load_packed_features(path, device, l2norm: bool = False):
     """One pinned staging buffer, one H->D copy (the reference does N pickle loads + N ``.cuda()`` calls, inference.py:383-401).
-    Returns (x [N,D] on the device, id_cam int64 [N] host array, id int64 [N] host array); ``l2norm`` applies
-    inference.py:403-404 on the device."""
+    Returns (x [N,D] on the device in the file's dtype, id_cam int64 [N] host array, id int64 [N] host array); ``l2norm``
+    applies inference.py:403-404 on the device (in place for an fp32 file; a 16-bit file gives a new fp32 tensor)."""
     dev = torch.device(device)
     if dev.type != "cuda":
         raise RuntimeError("load_packed_features copies to a CUDA device: the B200 path has no CPU fallback")
     x, cam, tid = read_packed_features(path)
-    pinned = torch.empty(x.shape, dtype=torch.float32).pin_memory()
-    np.copyto(pinned.numpy(), x)
-    xd = torch.empty(x.shape, dtype=torch.float32, device=dev)
+    dt = x.dtype if torch.is_tensor(x) else torch.from_numpy(np.empty(0, dtype=x.dtype)).dtype
+    pinned = torch.empty(x.shape, dtype=dt).pin_memory()
+    if torch.is_tensor(x):
+        pinned.copy_(x)
+    else:
+        np.copyto(pinned.numpy(), x)
+    xd = torch.empty(x.shape, dtype=dt, device=dev)
     xd.copy_(pinned, non_blocking=True)
     torch.cuda.current_stream(dev).synchronize()                    # the staging buffer is released on return
     if l2norm and xd.shape[0]:
-        xd = normalize_columns(xd, out=xd)
+        xd = normalize_columns(xd, out=xd if dt == torch.float32 else None)
     return xd, cam, tid

@@ -13,7 +13,7 @@ import torch
 from torch import nn
 
 from . import _lib
-from .graph import _on_device, current_stream_ptr, graph_for, workspace
+from .graph import _on_device, current_stream_ptr, graph_for, node_features, workspace
 
 USE_TENSOR_CORES = True
 
@@ -25,11 +25,11 @@ class _GraphedForward:
     replayed with a single launch, outputs are cloned so the caller still receives fresh tensors like the reference.
     """
 
-    def __init__(self, W, g, x, ea, L, n_cls, n_out, fused):
+    def __init__(self, W, g, x, x_kind, ea, L, n_cls, n_out, fused):
         from .graph import TrackletGraph
         dev = x.device
         self.W, self.L, self.n_cls = W, L, n_cls
-        self.x, self.ea = torch.empty_like(x), torch.empty_like(ea)
+        self.x, self.ea = torch.empty_like(x), torch.empty_like(ea)      # x staged in its own dtype
         # static graph tables with the same sizes as the caller's
         self.g = object.__new__(TrackletGraph)
         for name in ("device", "n_cols", "n_nodes", "row_offset", "n_edges", "chunk", "max_tasks"):
@@ -58,11 +58,11 @@ class _GraphedForward:
         self._stage(g, x, ea)
 
         def launch():
-            _lib.check(lib.mpn_forward(self.g.ref, C.byref(W), self.x.data_ptr(), self.ea.data_ptr(), L, n_cls,
-                                       self.logits.data_ptr(), self.h.data_ptr(),
-                                       self.pred.data_ptr() if fused else None, self.prob1.data_ptr() if fused else None,
-                                       int(bool(USE_TENSOR_CORES)), self.ws.data_ptr(), self.ws.numel(),
-                                       current_stream_ptr(dev)))
+            _lib.check(lib.mpn_forward_x(self.g.ref, C.byref(W), self.x.data_ptr(), x_kind, self.ea.data_ptr(), L, n_cls,
+                                         self.logits.data_ptr(), self.h.data_ptr(),
+                                         self.pred.data_ptr() if fused else None, self.prob1.data_ptr() if fused else None,
+                                         int(bool(USE_TENSOR_CORES)), self.ws.data_ptr(), self.ws.numel(),
+                                         current_stream_ptr(dev)))
         with torch.cuda.device(dev):
             side = torch.cuda.Stream(device=dev)
             side.wait_stream(torch.cuda.current_stream(dev))
@@ -206,7 +206,7 @@ class MOTMPNet(nn.Module):
         # small graphs are launch-bound (~30 dependent kernels): replay the forward as one CUDA graph
         self.use_cuda_graph = True
         self.cuda_graph_max_edges = 1 << 21
-        self._graphs = {}            # (device, N, E, D, L, n_cls, fused, weights key) -> _GraphedForward
+        self._graphs = {}            # (device, N, E, D, x dtype, L, n_cls, fused, weights key) -> _GraphedForward
         self.fuse_decisions = False  # when True forward also stores self.last_pred (uint8) / self.last_prob1 (fp32)
         self.last_pred = self.last_prob1 = None
 
@@ -310,7 +310,8 @@ class MOTMPNet(nn.Module):
     # ------------------------------------------------------------------------------------------
     @torch.no_grad()
     def forward(self, data):
-        """data.x [N,D] fp32, data.edge_index [2,E] int64, data.edge_attr [E,2] fp32, all on one CUDA device.
+        """data.x [N,D] fp32 (or fp16 / bf16: read in place, every output equals the one on ``data.x.float()``),
+        data.edge_index [2,E] int64, data.edge_attr [E,2] fp32, all on one CUDA device.
         Returns ({'classified_edges': [logits [E,2], ...]}, latent_node_feats [N,32]) as models/mpn.py:299.
 
         Extension: when ``data.edge_attr`` is None (or absent) the initial edge features of inference.py:453-456 are computed
@@ -325,7 +326,7 @@ class MOTMPNet(nn.Module):
         if self.training:
             raise _unsupported("training mode (dropout active / autograd); call .eval() as main.py:98 does")
         dev = x.device
-        x = x.contiguous().float()
+        x, x_kind = node_features(x)
         g = pre if pre is not None else graph_for(data, edge_index, x.shape[0])
         W = self._weights(dev)
         make_features = edge_attr is None
@@ -353,13 +354,13 @@ class MOTMPNet(nn.Module):
         n_out = 1 if L == 0 else n_cls
         fused = bool(self.fuse_decisions) and n_out > 0
         if self.use_cuda_graph and g.n_edges <= self.cuda_graph_max_edges and g.n_edges > 1:
-            key = (dev.index, g.n_nodes, g.n_edges, g.n_graphs, g.chunk, g.max_tasks, g.max_graph_nodes, x.shape[1], L, n_cls,
-                   bool(self.fuse_decisions), self._packed[0])
+            key = (dev.index, g.n_nodes, g.n_edges, g.n_graphs, g.chunk, g.max_tasks, g.max_graph_nodes, x.shape[1], x.dtype, L,
+                   n_cls, bool(self.fuse_decisions), self._packed[0])
             ent = self._graphs.get(key)
             if ent is None:
                 if len(self._graphs) >= 8:
                     self._graphs.pop(next(iter(self._graphs)))
-                ent = self._graphs[key] = _GraphedForward(W, g, x, ea, L, n_cls, max(n_out, 1), fused)
+                ent = self._graphs[key] = _GraphedForward(W, g, x, x_kind, ea, L, n_cls, max(n_out, 1), fused)
             logits, h, pred, prob1 = ent.run(g, x, ea)
         else:
             logits = torch.empty(max(n_out, 1), g.n_edges, 2, dtype=torch.float32, device=dev)
@@ -372,16 +373,16 @@ class MOTMPNet(nn.Module):
             with _on_device(dev):
                 if fused_features:
                     ef_ws = workspace("edge_features", dev, lib.mpn_edge_features_workspace_bytes(g.ref, x.shape[1]))
-                    _lib.check(lib.mpn_forward_with_edge_features(
-                        g.ref, C.byref(W), x.data_ptr(), ea.data_ptr(), L, n_cls, logits.data_ptr(), h.data_ptr(),
+                    _lib.check(lib.mpn_forward_with_edge_features_x(
+                        g.ref, C.byref(W), x.data_ptr(), x_kind, ea.data_ptr(), L, n_cls, logits.data_ptr(), h.data_ptr(),
                         pred.data_ptr() if pred is not None else None, prob1.data_ptr() if prob1 is not None else None,
                         int(bool(USE_TENSOR_CORES)), ws.data_ptr(), ws.numel(), ef_ws.data_ptr(), ef_ws.numel(),
                         current_stream_ptr(dev)))
                 else:
-                    _lib.check(lib.mpn_forward(g.ref, C.byref(W), x.data_ptr(), ea.data_ptr(), L, n_cls, logits.data_ptr(),
-                                               h.data_ptr(), pred.data_ptr() if pred is not None else None,
-                                               prob1.data_ptr() if prob1 is not None else None, int(bool(USE_TENSOR_CORES)),
-                                               ws.data_ptr(), ws.numel(), current_stream_ptr(dev)))
+                    _lib.check(lib.mpn_forward_x(g.ref, C.byref(W), x.data_ptr(), x_kind, ea.data_ptr(), L, n_cls,
+                                                 logits.data_ptr(), h.data_ptr(), pred.data_ptr() if pred is not None else None,
+                                                 prob1.data_ptr() if prob1 is not None else None, int(bool(USE_TENSOR_CORES)),
+                                                 ws.data_ptr(), ws.numel(), current_stream_ptr(dev)))
         if g.perm is not None:                       # back to the caller's edge order
             inv = torch.empty_like(logits)
             inv[:, g.perm] = logits

@@ -60,24 +60,25 @@ class GraphStream:
         self._id = GraphStream._instances
 
     def submit(self, x_host, cam_ids, pred_host, prob_host=None):
-        """``x_host``: pinned fp32 [N, D] (column-normalised ReID features, inference.py:403-404); ``cam_ids``: host sequence of
+        """``x_host``: pinned fp32, fp16 or bf16 [N, D] (column-normalised ReID features, inference.py:403-404; 16-bit features
+        cross PCIe in half the bytes and give the decisions of their fp32 widening); ``cam_ids``: host sequence of
         per-node camera ids, nodes grouped by ascending camera (dataset.py:279-281); ``pred_host``: pinned uint8 [E] that
         receives argmax(logits) (inference.py:479) in the graph's edge order; ``prob_host``: optional pinned fp32 [E] for
         softmax(logits)[:, 1] (inference.py:475-477).  Returns the ticket to pass to ``wait``."""
         if x_host.is_cuda or pred_host.is_cuda or not (x_host.is_pinned() and pred_host.is_pinned()):
             raise ValueError("GraphStream.submit takes pinned HOST tensors (x_host, pred_host)")
-        if x_host.dtype != torch.float32 or x_host.dim() != 2 or not x_host.is_contiguous():
-            raise ValueError("x_host must be a contiguous float32 [N, D] tensor")
+        if x_host.dtype not in (torch.float32, torch.float16, torch.bfloat16) or x_host.dim() != 2 or not x_host.is_contiguous():
+            raise ValueError("x_host must be a contiguous float32, float16 or bfloat16 [N, D] tensor")
         dev = self.device
         compute = torch.cuda.current_stream(dev)
         slot = self.slots[self.n_submitted % self.depth]
         ticket = self.n_submitted
         with torch.cuda.device(dev):
             full_shape = self._device_feature_shape(x_host, cam_ids)
-            if slot.x_dev is None or tuple(slot.x_dev.shape) != tuple(full_shape):
+            if slot.x_dev is None or tuple(slot.x_dev.shape) != tuple(full_shape) or slot.x_dev.dtype != x_host.dtype:
                 if slot.busy:
                     slot.compute_done.synchronize()
-                slot.x_dev = torch.empty(full_shape, dtype=torch.float32, device=dev)
+                slot.x_dev = torch.empty(full_shape, dtype=x_host.dtype, device=dev)
                 self.copy_in.wait_stream(compute)          # the allocator may hand out memory this stream still uses
             if slot.busy:
                 compute.wait_event(slot.out_done)            # the previous occupant's outputs have left the device: free them
@@ -159,7 +160,7 @@ class GraphStream:
         import numpy as np
         cam = np.ascontiguousarray(np.asarray(cam_ids.cpu() if isinstance(cam_ids, torch.Tensor) else cam_ids).reshape(-1))
         self.model._weights(self.device)                   # refreshes the packed-weights key if a parameter changed
-        return (slot.x_dev.data_ptr(), tuple(slot.x_dev.shape), str(cam.dtype), cam.tobytes(), self.model._packed[0])
+        return (slot.x_dev.data_ptr(), tuple(slot.x_dev.shape), slot.x_dev.dtype, str(cam.dtype), cam.tobytes(), self.model._packed[0])
 
     def _capture(self, slot, cam_ids, index):
         """One CUDA graph of K0 + K1 + forward + decisions for this slot.  Tensors allocated while capturing (graph tables,
@@ -236,7 +237,8 @@ class _Batch:
 class ShardedGraphStream(GraphStream):
     """The same pipeline for a row-block sharded graph (one process per GPU, ``ShardedMPN``): every rank copies only ITS rows of
     the features from its pinned host buffer, the ranks all-gather them over NVLink on the copy-in stream (NCCL), each rank runs
-    its shard (tables of its row block, edge features of its rows, sharded forward) and copies its shard's decisions back.  One
+    its shard (tables of its row block, edge features of its rows, sharded forward) and copies its shard's decisions back (fp16 /
+    bf16 rows are gathered in half and read in place, as in ``GraphStream``).  One
     graph computes at a time (the peer-memory exchange buffers of ``ShardedMPN`` are single-buffered); the copies and the
     all-gather of graph i+1 overlap the kernels of graph i.  ``submit(x_rows_host, cam_ids, pred_host)``: ``x_rows_host`` =
     rows ``blocks[rank]`` of the feature matrix."""

@@ -13,7 +13,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from .graph import TrackletGraph, _on_device, current_stream_ptr, workspace
+from .graph import TrackletGraph, _on_device, current_stream_ptr, node_features, workspace
 
 
 def partition_rows(rowptr: torch.Tensor, world: int):
@@ -187,7 +187,8 @@ class CudaPhases:
         return current_stream_ptr(self.dev)
 
     def node_encoder(self):
-        _lib.check(self.lib.mpn_plan_node_encoder(self.plan, self.x.data_ptr(), self.stream))
+        x, x_kind = node_features(self.x)
+        _lib.check(self.lib.mpn_plan_node_encoder_x(self.plan, x.data_ptr(), x_kind, self.stream))
 
     def node_tables(self, step):
         _lib.check(self.lib.mpn_plan_node_tables(self.plan, step, self.stream))
@@ -406,7 +407,7 @@ class ShardedMPN:
         if L > 0:
             n_cls = min(n_cls, L)         # as MOTMPNet.forward (models/mpn.py:281,290)
         n_out = 1 if L == 0 else n_cls
-        x = x.contiguous().float()
+        x, x_kind = node_features(x)
         make_features = local_edge_attr is None          # edge features of this rank's rows computed inside the call
         logits = torch.empty(max(n_out, 1), g.n_edges, 2, dtype=torch.float32, device=dev)
         pred = torch.empty(g.n_edges, dtype=torch.uint8, device=dev) if fuse_decisions else None
@@ -442,18 +443,18 @@ class ShardedMPN:
             with _on_device(dev):
                 if make_features:
                     ef_ws = workspace("edge_features", dev, lib.mpn_edge_features_workspace_bytes(g.ref, x.shape[1]))
-                    _lib.check(lib.mpn_forward_sharded_with_edge_features(
-                        g.ref, C.byref(W), x.data_ptr(), ea.data_ptr(), L, n_cls, total, logits.data_ptr(), h_local.data_ptr(),
+                    _lib.check(lib.mpn_forward_sharded_with_edge_features_x(
+                        g.ref, C.byref(W), x.data_ptr(), x_kind, ea.data_ptr(), L, n_cls, total, logits.data_ptr(), h_local.data_ptr(),
                         pred.data_ptr() if pred is not None else None, prob1.data_ptr() if prob1 is not None else None,
                         int(bool(USE_TENSOR_CORES)), C.byref(ctx), ws.data_ptr(), ws.numel(), ef_ws.data_ptr(), ef_ws.numel(),
                         current_stream_ptr(dev)))
                 else:
-                    _lib.check(lib.mpn_forward_sharded(g.ref, C.byref(W), x.data_ptr(), ea.data_ptr(), L, n_cls, total,
-                                                       logits.data_ptr(), h_local.data_ptr(),
-                                                       pred.data_ptr() if pred is not None else None,
-                                                       prob1.data_ptr() if prob1 is not None else None,
-                                                       int(bool(USE_TENSOR_CORES)), C.byref(ctx), ws.data_ptr(), ws.numel(),
-                                                       current_stream_ptr(dev)))
+                    _lib.check(lib.mpn_forward_sharded_x(g.ref, C.byref(W), x.data_ptr(), x_kind, ea.data_ptr(), L, n_cls, total,
+                                                         logits.data_ptr(), h_local.data_ptr(),
+                                                         pred.data_ptr() if pred is not None else None,
+                                                         prob1.data_ptr() if prob1 is not None else None,
+                                                         int(bool(USE_TENSOR_CORES)), C.byref(ctx), ws.data_ptr(), ws.numel(),
+                                                         current_stream_ptr(dev)))
             peers.advance(L, shard_enc, n_layers, shared_gram=shared)
             self._last_ef = (g, int(x.shape[1]), ef_ws) if make_features else None
             return {'classified_edges': [logits[i] for i in range(n_out)]}, h_local, pred, prob1

@@ -508,6 +508,45 @@ int mpn_normalize_columns(const float* x_dev, int32_t n, int32_t D, float* out_d
 int mpn_normalize_columns_batched(const float* x_dev, int32_t n, int32_t D, const int32_t* graph_nptr_dev, int32_t n_graphs,
                                   float* out_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Half-width node features.  Every entry point that reads the node features x has an `_x` twin that takes
+ * `const void* x_dev, int32_t x_kind` in place of `const float* x_dev` and is otherwise identical (the fp32 entry points are
+ * these twins called with MPN_X_F32).  The kernels that read x convert each element to fp32 on load (exact for fp16 and bf16)
+ * and keep every reduction's order, so each output is bit-identical to the same call on the fp32 copy of x; no such copy is
+ * made.  The outputs stay fp32 (mpn_normalize_columns_x writes fp32 out_dev, which then cannot alias a 16-bit x).  An unknown
+ * x_kind returns MPN_ERR_INVALID.  Half-precision features are the caller's choice: they are exact inputs, but not the
+ * fp32 embeddings they were rounded from.
+ * ---------------------------------------------------------------------------------------------- */
+#define MPN_X_F32 0
+#define MPN_X_F16 1
+#define MPN_X_BF16 2
+int mpn_edge_features_x(const mpn_graph* g, const void* x_dev, int32_t x_kind, int32_t D, float* edge_attr_dev,
+                        int use_tensor_cores, void* workspace_dev, size_t workspace_bytes, void* stream);
+int mpn_forward_x(const mpn_graph* g, const mpn_weights* w, const void* x_dev, int32_t x_kind, const float* edge_attr_dev,
+                  int32_t num_enc_steps, int32_t num_class_steps, float* logits_out_dev, float* h_out_dev,
+                  uint8_t* pred_out_dev, float* prob1_out_dev, int use_tensor_cores,
+                  void* workspace_dev, size_t workspace_bytes, void* stream);
+int mpn_forward_with_edge_features_x(const mpn_graph* g, const mpn_weights* w, const void* x_dev, int32_t x_kind,
+                                     float* edge_attr_out_dev, int32_t num_enc_steps, int32_t num_class_steps, float* logits_out_dev,
+                                     float* h_out_dev, uint8_t* pred_out_dev, float* prob1_out_dev, int use_tensor_cores,
+                                     void* workspace_dev, size_t workspace_bytes, void* ef_workspace_dev, size_t ef_workspace_bytes,
+                                     void* stream);
+int mpn_forward_sharded_x(const mpn_graph* g, const mpn_weights* w, const void* x_dev, int32_t x_kind, const float* edge_attr_dev,
+                          int32_t num_enc_steps, int32_t num_class_steps, int64_t total_edges, float* logits_out_dev,
+                          float* h_out_dev, uint8_t* pred_out_dev, float* prob1_out_dev, int use_tensor_cores,
+                          const mpn_peer_ctx* peers, void* workspace_dev, size_t workspace_bytes, void* stream);
+int mpn_forward_sharded_with_edge_features_x(const mpn_graph* g, const mpn_weights* w, const void* x_dev, int32_t x_kind,
+                                             float* edge_attr_out_dev, int32_t num_enc_steps, int32_t num_class_steps,
+                                             int64_t total_edges, float* logits_out_dev, float* h_out_dev, uint8_t* pred_out_dev,
+                                             float* prob1_out_dev, int use_tensor_cores, const mpn_peer_ctx* peers,
+                                             void* workspace_dev, size_t workspace_bytes, void* ef_workspace_dev,
+                                             size_t ef_workspace_bytes, void* stream);
+int mpn_plan_node_encoder_x(mpn_fwd_plan* plan, const void* x_dev, int32_t x_kind, void* stream);
+int mpn_normalize_columns_x(const void* x_dev, int32_t x_kind, int32_t n, int32_t D, float* out_dev, void* workspace_dev,
+                            size_t workspace_bytes, void* stream);
+int mpn_normalize_columns_batched_x(const void* x_dev, int32_t x_kind, int32_t n, int32_t D, const int32_t* graph_nptr_dev,
+                                    int32_t n_graphs, float* out_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
