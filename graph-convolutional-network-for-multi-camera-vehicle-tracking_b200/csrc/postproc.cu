@@ -8,7 +8,6 @@
 // candidates, utils.py:288-289), components use min-id union-find.
 #include <algorithm>
 #include <atomic>
-#include <chrono>
 #include <cstdlib>
 #include <string>
 #include <thread>
@@ -22,6 +21,18 @@ namespace mpn {
 constexpr int EPB = 4096;            // edges per compaction block (256 threads x 16 flags)
 constexpr unsigned int HASH_EMPTY = 0xFFFFFFFFu;
 
+// Which graph a node belongs to and that graph's camera count (PRUNE bounds degrees by it minus one, SPLIT cluster sizes by it).
+// A batch reads node_gid and the per-graph counts on the device; gid == nullptr is one graph, graph 0 with ncam1 cameras, with no
+// load.  The single-graph entry points pass that view for any table, so a batch given to them is one disjoint-union graph.
+struct Graphs {
+  const int* gid;
+  const int* ncam;
+  int ncam1;
+  __device__ __forceinline__ int graph_of(int n) const { return gid ? gid[n] : 0; }
+  __device__ __forceinline__ int limit_of(int n) const { return gid ? ncam[gid[n]] : ncam1; }
+};
+static Graphs one_graph(int num_cameras) { return Graphs{nullptr, nullptr, num_cameras}; }
+
 struct PostCtx {
   mpn_graph g;
   cudaStream_t st;
@@ -31,17 +42,17 @@ struct PostCtx {
   int *fo, *fi, *label, *size, *od_src, *od_dst, *counters;      // counters[8]
   int *dirty_nodes, *dirty_edges;                                // SPLIT: nodes of oversized clusters, active-list entries touching them
   unsigned long long *mo, *mi;
-  unsigned int *mbits, *hash;
+  unsigned int* mbits;
+  unsigned long long* hash;                                      // SPLIT: the dropped minima, keyed by (graph id, probability bits)
   int hash_cap;
   int *wcc, *wccflag;                                            // SPLIT: weakly connected components and the flagged ones
-  unsigned int* tie_keys;                                        // SPLIT: probability values of the dirty edges ...
-  int* tie_counts;                                               // ... and how many active edges carry each
+  unsigned long long* tie_keys;                                  // SPLIT: (graph id, probability) of the dirty edges ...
+  int* tie_counts;                                               // ... and how many active edges of that graph carry each
   int tie_cap;
   float* a_prob;                                                 // SPLIT: probabilities in active-list order
   uint8_t *sel, *tiedb;                                          // SPLIT: entry selected for the host; value carried by >= 2 active edges
-  // batched graphs only (n_graphs > 1)
-  int *a_gptr, *gflag, *groots;                                  // first active-list entry per graph [G+1]; per-graph flag, root count [G]
-  unsigned long long *hash64, *tie_keys64;                       // SPLIT sets keyed by (graph id, probability bits)
+  int *a_gptr, *gflag, *groots;      // first active-list entry per graph [G+1]; SPLIT host-order flag per graph [G] + tied-edge count
+                                     // (one copy to the host); SCC count per graph [G]
   size_t total;
   // host
   int n_active;
@@ -70,28 +81,24 @@ static void post_layout(PostCtx& c, void* ws, size_t ws_bytes) {
   int cap = 1024;
   while ((size_t)cap < N) cap <<= 1;
   c.hash_cap = cap;
-  c.hash = a.take<unsigned int>(cap);
+  // the SPLIT sets key (graph id, probability bits) for one graph too: 8 B a slot where a value-only set would take 4, which at
+  // configs[3] (1 M nodes, ~92 M edges) is ~138 MB more, and one set of kernels serves one graph and a batch
+  c.hash = a.take<unsigned long long>(cap);
   c.wcc = a.take<int>(N);
   c.wccflag = a.take<int>(N);
   int tcap = 1024;
   while ((size_t)tcap < E / 4) tcap <<= 1;
   c.tie_cap = tcap;
-  c.tie_keys = a.take<unsigned int>(tcap);
+  c.tie_keys = a.take<unsigned long long>(tcap);
   c.tie_counts = a.take<int>(tcap);
   c.a_prob = a.take<float>(E);
   c.sel = a.take<uint8_t>(E);
   c.tiedb = a.take<uint8_t>(E);
   c.counters = a.take<int>(16);
-  c.a_gptr = c.gflag = c.groots = nullptr;
-  c.hash64 = c.tie_keys64 = nullptr;
-  if (c.g.n_graphs > 1) {                                        // appended: the single-graph layout is unchanged
-    const size_t G = (size_t)c.g.n_graphs;
-    c.a_gptr = a.take<int>(G + 1);
-    c.gflag = a.take<int>(G);
-    c.groots = a.take<int>(G);
-    c.hash64 = a.take<unsigned long long>(c.hash_cap);
-    c.tie_keys64 = a.take<unsigned long long>(c.tie_cap);
-  }
+  const size_t G = (size_t)std::max(1, c.g.n_graphs);
+  c.a_gptr = a.take<int>(G + 1);
+  c.gflag = a.take<int>(G + 1);
+  c.groots = a.take<int>(G);
   c.total = a.off;
 }
 
@@ -246,8 +253,9 @@ __global__ void flow_count_kernel(int A, const int* __restrict__ a_eid, const in
     atomicAdd(&fi[a_dst[i]], 1);
   }
 }
+// the bound of a node is the camera count of its graph minus one (an edge's endpoints lie in one graph)
 __global__ void prune_pick_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ a_dst,
-                                  const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride, int limit,
+                                  const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride, const Graphs graphs,
                                   const int* __restrict__ fo, const int* __restrict__ fi, unsigned long long* __restrict__ mo,
                                   unsigned long long* __restrict__ mi, int* __restrict__ any_violation) {
   bool viol = false;
@@ -255,27 +263,7 @@ __global__ void prune_pick_kernel(int A, const int* __restrict__ a_eid, const in
     const int e = a_eid[i];
     if (!act[e]) continue;
     const int u = a_src[i], v = a_dst[i];
-    const bool bo = fo[u] > limit, bi = fi[v] > limit;
-    if (!(bo || bi)) continue;
-    viol = true;
-    const unsigned long long key = ((unsigned long long)__float_as_uint(prob[(size_t)e * pstride]) << 32) | (unsigned int)e;
-    if (bo) atomicMin(&mo[u], key);
-    if (bi) atomicMin(&mi[v], key);
-  }
-  if (viol) *any_violation = 1;
-}
-// batched graphs: the bound of a node is num_cameras[its graph] - 1 (an edge's endpoints lie in one graph)
-__global__ void prune_pick_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src,
-                                          const int* __restrict__ a_dst, const uint8_t* __restrict__ act, const float* __restrict__ prob,
-                                          int pstride, const int* __restrict__ gid, const int* __restrict__ ncam,
-                                          const int* __restrict__ fo, const int* __restrict__ fi, unsigned long long* __restrict__ mo,
-                                          unsigned long long* __restrict__ mi, int* __restrict__ any_violation) {
-  bool viol = false;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
-    const int e = a_eid[i];
-    if (!act[e]) continue;
-    const int u = a_src[i], v = a_dst[i];
-    const int limit = ncam[gid[u]] - 1;
+    const int limit = graphs.limit_of(u) - 1;
     const bool bo = fo[u] > limit, bi = fi[v] > limit;
     if (!(bo || bi)) continue;
     viol = true;
@@ -304,11 +292,9 @@ __global__ void prune_reset_kernel(int N, int* __restrict__ fo, int* __restrict_
 // Rounds are enqueued PRUNE_BATCH at a time with one flag word each and the host reads the flags once per batch: a round without
 // a violating node removes nothing, so the rounds enqueued past the fixed point are no-ops (the violation flags of a batch are a
 // prefix of ones).  One host round trip per 8 rounds instead of one per round (the smoke graph needs 87 rounds).
-// BATCH: per-graph bounds num_cameras_dev[node_gid[n]]; a graph that has converged sees no-op rounds while the others go on.
+// In a batch a graph that has converged sees no-op rounds while the others go on.
 constexpr int PRUNE_BATCH = 8;
-template <bool BATCH = false>
-static int prune_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride, int num_cameras, int* changed, int* rounds,
-                       const int* num_cameras_dev = nullptr) {
+static int prune_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride, const Graphs& graphs, int* changed, int* rounds) {
   const int A = c.n_active, N = c.g.n_nodes;
   *changed = 0;
   *rounds = 0;
@@ -321,12 +307,8 @@ static int prune_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride,
       MPN_LAUNCH_OK();
       flow_count_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.fo, c.fi);
       MPN_LAUNCH_OK();
-      if constexpr (BATCH)
-        prune_pick_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, prob, pstride, c.g.node_gid,
-                                                                  num_cameras_dev, c.fo, c.fi, c.mo, c.mi, flags + r);
-      else
-        prune_pick_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, prob, pstride, num_cameras - 1, c.fo,
-                                                          c.fi, c.mo, c.mi, flags + r);
+      prune_pick_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, prob, pstride, graphs, c.fo, c.fi, c.mo,
+                                                        c.mi, flags + r);
       MPN_LAUNCH_OK();
       prune_remove_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.mo, c.mi, act);
       MPN_LAUNCH_OK();
@@ -521,74 +503,60 @@ static int scc_stage(PostCtx& c, const uint8_t* act, int* n_components) {
 
 // ------------------------------------------------------------------------------------------------
 // SPLIT (utils.py:54-123) as parallel rounds: every oversized SCC contributes the minimum probability among the
-// active edges touching it (either endpoint, utils.py:71); every edge whose probability equals one of those
-// values is deactivated (global float equality, utils.py:96-98); repeat until no SCC has more than C nodes.
+// active edges touching it (either endpoint, utils.py:71); every edge of its graph whose probability equals one of those
+// values is deactivated (float equality, utils.py:96-98); repeat until no SCC has more than C nodes.
+// The reference removes the edges of ITS graph only, so in a batch a value shared by two different graphs must neither couple
+// them nor count as a tie: the sets below are keyed by (graph id, probability bits).
 // ------------------------------------------------------------------------------------------------
 __global__ void comp_size_kernel(int N, const int* __restrict__ label, int* __restrict__ size) {
   for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) atomicAdd(&size[label[n]], 1);
-}
-__global__ void split_min_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ a_dst,
-                                 const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
-                                 const int* __restrict__ label, const int* __restrict__ size, int limit,
-                                 unsigned int* __restrict__ mbits) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
-    const int e = a_eid[i];
-    if (!act[e]) continue;
-    const int lu = label[a_src[i]], lv = label[a_dst[i]];
-    const unsigned int pb = __float_as_uint(prob[(size_t)e * pstride]);
-    if (size[lu] > limit) atomicMin(&mbits[lu], pb);
-    if (lv != lu && size[lv] > limit) atomicMin(&mbits[lv], pb);
-  }
 }
 __device__ __forceinline__ unsigned int hash_u32(unsigned int x) {
   x ^= x >> 16; x *= 0x7feb352dU; x ^= x >> 15; x *= 0x846ca68bU; x ^= x >> 16;
   return x;
 }
-__global__ void split_collect_kernel(int N, const int* __restrict__ label, const int* __restrict__ size, int limit,
-                                     const unsigned int* __restrict__ mbits, unsigned int* __restrict__ hash, int cap,
-                                     int* __restrict__ n_big) {
-  for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) {
-    if (label[n] != n || size[n] <= limit) continue;
-    atomicAdd(n_big, 1);
-    const unsigned int key = mbits[n];
-    if (key == HASH_EMPTY) continue;
-    unsigned int slot = hash_u32(key) & (cap - 1);
-    for (;;) {
-      const unsigned int old = atomicCAS(&hash[slot], HASH_EMPTY, key);
-      if (old == HASH_EMPTY || old == key) break;
-      slot = (slot + 1) & (cap - 1);
-    }
+constexpr unsigned long long HASH64_EMPTY = ~0ull;         // never a key: graph ids are < 2^31
+__device__ __forceinline__ unsigned long long graph_value_key(int g, unsigned int bits) {
+  return ((unsigned long long)(unsigned int)g << 32) | bits;
+}
+__device__ __forceinline__ unsigned int hash_u64(unsigned long long k) {
+  return hash_u32((unsigned int)k ^ hash_u32((unsigned int)(k >> 32) + 0x9e3779b9u));
+}
+__device__ __forceinline__ void set64_insert(unsigned long long* __restrict__ t, int cap, unsigned long long key) {
+  unsigned int slot = hash_u64(key) & (cap - 1);
+  for (;;) {
+    const unsigned long long old = atomicCAS(&t[slot], HASH64_EMPTY, key);
+    if (old == HASH64_EMPTY || old == key) return;
+    slot = (slot + 1) & (cap - 1);
   }
 }
-__global__ void split_remove_kernel(int A, const int* __restrict__ a_eid, uint8_t* __restrict__ act, const float* __restrict__ prob,
-                                    int pstride, const unsigned int* __restrict__ hash, int cap) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
-    const int e = a_eid[i];
-    if (!act[e]) continue;
-    const unsigned int key = __float_as_uint(prob[(size_t)e * pstride]);
-    unsigned int slot = hash_u32(key) & (cap - 1);
-    for (;;) {
-      const unsigned int v = hash[slot];
-      if (v == key) { act[e] = 0; break; }
-      if (v == HASH_EMPTY) break;
-      slot = (slot + 1) & (cap - 1);
-    }
+__device__ __forceinline__ int set64_find(const unsigned long long* __restrict__ t, int cap, unsigned long long key) {
+  unsigned int slot = hash_u64(key) & (cap - 1);
+  for (;;) {
+    const unsigned long long v = t[slot];
+    if (v == key) return (int)slot;
+    if (v == HASH64_EMPTY) return -1;
+    slot = (slot + 1) & (cap - 1);
   }
 }
 
-// ---- list-restricted variants: after the first round only the nodes of oversized clusters ("dirty") and the active
+// ---- list-restricted rounds: after the first round only the nodes of oversized clusters ("dirty") and the active
 // edges touching them can change the outcome, so every later round works on those two lists only.
-__global__ void mark_dirty_nodes_kernel(int N, const int* __restrict__ label, const int* __restrict__ size, int limit,
-                                        int* __restrict__ list, int* __restrict__ count) {
+// skip (optional): graphs whose clusters are left out (they went through the reference order on the host)
+__global__ void mark_dirty_nodes_kernel(int N, const int* __restrict__ label, const int* __restrict__ size, const Graphs graphs,
+                                        const int* __restrict__ skip, int* __restrict__ list, int* __restrict__ count) {
   for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x)
-    if (size[label[n]] > limit) list[atomicAdd(count, 1)] = n;
+    if ((skip == nullptr || !skip[graphs.graph_of(n)]) && size[label[n]] > graphs.limit_of(n)) list[atomicAdd(count, 1)] = n;
 }
 __global__ void mark_dirty_edges_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ a_dst,
                                         const uint8_t* __restrict__ act, const int* __restrict__ label, const int* __restrict__ size,
-                                        int limit, int* __restrict__ list, int* __restrict__ count) {
+                                        const Graphs graphs, const int* __restrict__ skip, int* __restrict__ list, int* __restrict__ count) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
     if (!act[a_eid[i]]) continue;
-    if (size[label[a_src[i]]] > limit || size[label[a_dst[i]]] > limit) list[atomicAdd(count, 1)] = i;
+    const int u = a_src[i];
+    if (skip != nullptr && skip[graphs.graph_of(u)]) continue;
+    const int limit = graphs.limit_of(u);
+    if (size[label[u]] > limit || size[label[a_dst[i]]] > limit) list[atomicAdd(count, 1)] = i;
   }
 }
 __global__ void reset_nodes_kernel(int n_list, const int* __restrict__ list, int* __restrict__ label, int* __restrict__ size,
@@ -622,8 +590,8 @@ __global__ void flatten_list_kernel(int n_list, const int* __restrict__ list, in
 }
 __global__ void one_dir_edges_list_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ a_eid,
                                           const int* __restrict__ a_src, const int* __restrict__ a_dst, const int* __restrict__ a_rev,
-                                          const uint8_t* __restrict__ act, const int* __restrict__ label, const int* __restrict__ is_dirty_size,
-                                          int limit_unused, int* __restrict__ od_src, int* __restrict__ od_dst, int* __restrict__ od_count) {
+                                          const uint8_t* __restrict__ act, const int* __restrict__ label, int* __restrict__ od_src,
+                                          int* __restrict__ od_dst, int* __restrict__ od_count) {
   for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
     const int i = list[k];
     if (!act[a_eid[i]]) continue;
@@ -641,33 +609,40 @@ __global__ void comp_size_list_kernel(int n_list, const int* __restrict__ list, 
 }
 __global__ void split_min_list_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ a_eid, const int* __restrict__ a_src,
                                       const int* __restrict__ a_dst, const uint8_t* __restrict__ act, const float* __restrict__ prob,
-                                      int pstride, const int* __restrict__ label, const int* __restrict__ size, int limit,
+                                      int pstride, const int* __restrict__ label, const int* __restrict__ size, const Graphs graphs,
                                       unsigned int* __restrict__ mbits) {
   for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
     const int i = list[k];
     const int e = a_eid[i];
     if (!act[e]) continue;
-    const int lu = label[a_src[i]], lv = label[a_dst[i]];
+    const int u = a_src[i];
+    const int lu = label[u], lv = label[a_dst[i]];
+    const int limit = graphs.limit_of(u);
     const unsigned int pb = __float_as_uint(prob[(size_t)e * pstride]);
     if (size[lu] > limit) atomicMin(&mbits[lu], pb);
     if (lv != lu && size[lv] > limit) atomicMin(&mbits[lv], pb);
   }
 }
 __global__ void split_collect_list_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ label,
-                                          const int* __restrict__ size, int limit, const unsigned int* __restrict__ mbits,
-                                          unsigned int* __restrict__ hash, int cap, int* __restrict__ n_big) {
+                                          const int* __restrict__ size, const Graphs graphs, const unsigned int* __restrict__ mbits,
+                                          unsigned long long* __restrict__ hash, int cap, int* __restrict__ n_big) {
   for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
     const int n = list[k];
-    if (label[n] != n || size[n] <= limit) continue;
+    if (label[n] != n || size[n] <= graphs.limit_of(n)) continue;
     atomicAdd(n_big, 1);
-    const unsigned int key = mbits[n];
-    if (key == HASH_EMPTY) continue;
-    unsigned int slot = hash_u32(key) & (cap - 1);
-    for (;;) {
-      const unsigned int old = atomicCAS(&hash[slot], HASH_EMPTY, key);
-      if (old == HASH_EMPTY || old == key) break;
-      slot = (slot + 1) & (cap - 1);
-    }
+    const unsigned int bits = mbits[n];
+    if (bits == HASH_EMPTY) continue;
+    set64_insert(hash, cap, graph_value_key(graphs.graph_of(n), bits));
+  }
+}
+// every active edge of a graph whose probability equals one of that graph's dropped minima (utils.py:96-98)
+__global__ void split_remove_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const Graphs graphs,
+                                    uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
+                                    const unsigned long long* __restrict__ hash, int cap) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
+    const int e = a_eid[i];
+    if (!act[e]) continue;
+    if (set64_find(hash, cap, graph_value_key(graphs.graph_of(a_src[i]), __float_as_uint(prob[(size_t)e * pstride]))) >= 0) act[e] = 0;
   }
 }
 
@@ -683,8 +658,8 @@ static int scc_dirty(PostCtx& c, const uint8_t* act, int Dn, int De) {
   flatten_list_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label);
   MPN_LAUNCH_OK();
   if (De > 0) {
-    one_dir_edges_list_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, c.a_dst, c.a_rev, act, c.label, c.size,
-                                                             0, c.od_src, c.od_dst, c.counters + 3);
+    one_dir_edges_list_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, c.a_dst, c.a_rev, act, c.label,
+                                                             c.od_src, c.od_dst, c.counters + 3);
     MPN_LAUNCH_OK();
   }
   int n_od = 0;
@@ -714,41 +689,29 @@ static int scc_dirty(PostCtx& c, const uint8_t* act, int Dn, int De) {
 
 // ---- probability ties -------------------------------------------------------------------------------------------------
 // The rounds above equal the reference's one-cluster-at-a-time loop exactly when no probability value that an oversized
-// cluster can drop is carried by a second active edge: the reference removes EVERY edge with that value (utils.py:96-98), so
-// a shared value couples two clusters and the order in which the reference visits them (utils.py:60-64,112) decides the
-// outcome.  Ties are detected on the device; a graph that has one goes through the exact order on the host
+// cluster can drop is carried by a second active edge of its graph: the reference removes EVERY edge with that value
+// (utils.py:96-98), so a shared value couples two clusters and the order in which the reference visits them (utils.py:60-64,112)
+// decides the outcome.  Ties are detected on the device; a graph that has one goes through the exact order on the host
 // (split_exact.cu), restricted to the weakly connected components that SPLITTING can touch.
-//   table: open addressing over the probability bits of the active edges touching oversized clusters ("dirty" edges);
-//   count: how many active edges of the whole graph carry each of those values.
-__global__ void tie_insert_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ a_eid, const uint8_t* __restrict__ act,
-                                  const float* __restrict__ prob, int pstride, unsigned int* __restrict__ keys, int cap) {
+//   table: open addressing over (graph, probability bits) of the active edges touching oversized clusters ("dirty" edges);
+//   count: how many active edges of the same graph carry each of those values.
+__global__ void tie_insert_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ a_eid, const int* __restrict__ a_src,
+                                  const Graphs graphs, const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
+                                  unsigned long long* __restrict__ keys, int cap) {
   for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
-    const int e = a_eid[list[k]];
+    const int i = list[k];
+    const int e = a_eid[i];
     if (!act[e]) continue;
-    const unsigned int key = __float_as_uint(prob[(size_t)e * pstride]);
-    unsigned int slot = hash_u32(key) & (cap - 1);
-    for (;;) {
-      const unsigned int old = atomicCAS(&keys[slot], HASH_EMPTY, key);
-      if (old == HASH_EMPTY || old == key) break;
-      slot = (slot + 1) & (cap - 1);
-    }
+    set64_insert(keys, cap, graph_value_key(graphs.graph_of(a_src[i]), __float_as_uint(prob[(size_t)e * pstride])));
   }
 }
-__device__ __forceinline__ int tie_find(const unsigned int* __restrict__ keys, int cap, unsigned int key) {
-  unsigned int slot = hash_u32(key) & (cap - 1);
-  for (;;) {
-    const unsigned int v = keys[slot];
-    if (v == key) return (int)slot;
-    if (v == HASH_EMPTY) return -1;
-    slot = (slot + 1) & (cap - 1);
-  }
-}
-__global__ void tie_count_kernel(int A, const int* __restrict__ a_eid, const uint8_t* __restrict__ act, const float* __restrict__ prob,
-                                 int pstride, const unsigned int* __restrict__ keys, int* __restrict__ counts, int cap) {
+__global__ void tie_count_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const Graphs graphs,
+                                 const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
+                                 const unsigned long long* __restrict__ keys, int* __restrict__ counts, int cap) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
     const int e = a_eid[i];
     if (!act[e]) continue;
-    const int slot = tie_find(keys, cap, __float_as_uint(prob[(size_t)e * pstride]));
+    const int slot = set64_find(keys, cap, graph_value_key(graphs.graph_of(a_src[i]), __float_as_uint(prob[(size_t)e * pstride])));
     if (slot >= 0) atomicAdd(&counts[slot], 1);
   }
 }
@@ -758,26 +721,32 @@ __global__ void union_all_kernel(int A, const int* __restrict__ a_eid, const int
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x)
     if (act[a_eid[i]]) uf_union(parent, a_src[i], a_dst[i]);
 }
-// flag the components SPLITTING can touch: those holding an oversized cluster, those holding an edge with a tied value
+// flag the components SPLITTING can touch: those holding an oversized cluster, those holding an edge with a tied value; and the
+// graphs that have a tie (gtied)
 __global__ void flag_wcc_nodes_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ wcc, int* __restrict__ flag) {
   for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) flag[wcc[list[k]]] = 1;
 }
-__global__ void flag_wcc_ties_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const uint8_t* __restrict__ act,
-                                     const float* __restrict__ prob, int pstride, const unsigned int* __restrict__ keys,
-                                     const int* __restrict__ counts, int cap, const int* __restrict__ wcc, int* __restrict__ flag,
-                                     uint8_t* __restrict__ tiedb, int* __restrict__ n_tied_edges) {
+__global__ void flag_wcc_ties_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const Graphs graphs,
+                                     const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
+                                     const unsigned long long* __restrict__ keys, const int* __restrict__ counts, int cap,
+                                     const int* __restrict__ wcc, int* __restrict__ flag, uint8_t* __restrict__ tiedb,
+                                     int* __restrict__ gtied, int* __restrict__ n_tied_edges) {
   int tied = 0;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
     const int e = a_eid[i];
     uint8_t t = 0;
     if (act[e]) {
-      const int slot = tie_find(keys, cap, __float_as_uint(prob[(size_t)e * pstride]));
-      if (slot >= 0 && counts[slot] >= 2) { flag[wcc[a_src[i]]] = 1; ++tied; t = 1; }
+      const int g = graphs.graph_of(a_src[i]);
+      const int slot = set64_find(keys, cap, graph_value_key(g, __float_as_uint(prob[(size_t)e * pstride])));
+      if (slot >= 0 && counts[slot] >= 2) { flag[wcc[a_src[i]]] = 1; gtied[g] = 1; ++tied; t = 1; }
     }
     tiedb[i] = t;
   }
   tied = __reduce_add_sync(0xffffffffu, tied);
   if ((threadIdx.x & 31) == 0 && tied) atomicAdd(n_tied_edges, tied);
+}
+__global__ void flag_graphs_of_nodes_kernel(int n_list, const int* __restrict__ list, const Graphs graphs, int* __restrict__ gflag) {
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) gflag[graphs.graph_of(list[k])] = 1;
 }
 // per active-list entry: probability (compacted) and whether its component is flagged (activity included)
 __global__ void gather_select_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const uint8_t* __restrict__ act,
@@ -787,6 +756,19 @@ __global__ void gather_select_kernel(int A, const int* __restrict__ a_eid, const
     const int e = a_eid[i];
     a_prob[i] = prob[(size_t)e * pstride];
     sel[i] = (act[e] && flag[wcc[a_src[i]]]) ? 1 : 0;
+  }
+}
+// a_gptr[g] = first active-list entry at or after the first edge of graph g (a_eid ascends); a_gptr[G] = A
+__global__ void active_graph_ptr_kernel(int G, const int* __restrict__ rowptr, const int* __restrict__ nptr, const int* __restrict__ a_eid,
+                                        int A, int* __restrict__ a_gptr) {
+  for (int g = blockIdx.x * blockDim.x + threadIdx.x; g <= G; g += gridDim.x * blockDim.x) {
+    const int e0 = rowptr[nptr[g]];
+    int lo = 0, hi = A;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (a_eid[mid] < e0) lo = mid + 1; else hi = mid;
+    }
+    a_gptr[g] = lo;
   }
 }
 
@@ -817,333 +799,28 @@ __global__ void apply_keep_kernel(int A, const int* __restrict__ a_eid, const ui
 int split_exact_host_impl(const int* src, const int* dst, const float* prob, long long m, int n_nodes, int C, uint8_t* keep,
                           int64_t* stats_out, const uint8_t* tied, const int* seeds, long long n_seeds, const uint8_t* sel);      // split_exact.cu
 
-// the reference's order on the host for the flagged components (every oversized cluster lives in one of them)
-static int split_in_reference_order(PostCtx& c, uint8_t* act, const float* prob, int pstride, int num_cameras, int Dn, bool have_ties,
-                                    int* rounds) {
-  const int A = c.n_active, N = c.g.n_nodes;
-  static const bool dbg = getenv("MPN_POST_DEBUG") != nullptr;
-  auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-  const double t0 = now();
-  gather_select_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, act, prob, pstride, c.wcc, c.wccflag, c.a_prob, c.sel);
-  MPN_LAUNCH_OK();
-  // pinned staging (grow-only, per host thread): pageable destinations would be staged by the driver at a few GB/s
-  const size_t Au = (size_t)A, A16 = (Au + 15) & ~(size_t)15;
-  char* pin = (char*)g_split_pin.get(12 * A16 + 3 * A16 + 64);
-  MPN_REQUIRE(pin != nullptr, "split: out of pinned host memory (%zu bytes)", 15 * A16 + 64);
-  int* hs = (int*)pin;
-  int* hd = (int*)(pin + 4 * A16);
-  float* hp = (float*)(pin + 8 * A16);
-  uint8_t* hsel = (uint8_t*)(pin + 12 * A16);
-  uint8_t* htied = hsel + A16;
-  uint8_t* keep_all = htied + A16;
-  std::vector<int> seeds(Dn);
-  MPN_CUDA_OK(cudaMemcpyAsync(seeds.data(), c.dirty_nodes, sizeof(int) * Dn, cudaMemcpyDeviceToHost, c.st));
-  if (have_ties) MPN_CUDA_OK(cudaMemcpyAsync(htied, c.tiedb, Au, cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaMemcpyAsync(hsel, c.sel, Au, cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaMemcpyAsync(hs, c.a_src, sizeof(int) * Au, cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaMemcpyAsync(hd, c.a_dst, sizeof(int) * Au, cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaMemcpyAsync(hp, c.a_prob, sizeof(float) * Au, cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  long long m = 0;                                  // the sub-problem: selected entries (they keep their position as edge id)
-  for (int i = 0; i < A; ++i) m += hsel[i];
-  const double t1 = now();
-  int64_t st[4] = {0, 0, 0, 0};
-  const double t2 = now();
-  if (m > 0) MPN_TRY(split_exact_host_impl(hs, hd, hp, A, N, num_cameras, keep_all, st, have_ties ? htied : nullptr, seeds.data(),
-                                           (long long)seeds.size(), hsel));
-  else memset(keep_all, 1, Au);
-  const double t3 = now();
-  MPN_CUDA_OK(cudaMemcpyAsync(c.sel, keep_all, Au, cudaMemcpyHostToDevice, c.st));
-  apply_keep_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.sel, act);
-  MPN_LAUNCH_OK();
-  MPN_CUDA_OK(cudaStreamSynchronize(c.st));        // the staging buffer is reused by the next call
-  if (dbg) fprintf(stderr, "[split host] A=%d m=%lld seeds=%d: D2H+select %.2f ms, gather %.2f ms, engine %.2f ms, write-back %.2f ms\n", A, m, Dn,
-                   t1 - t0, t2 - t1, t3 - t2, now() - t3);
-  *rounds = (int)st[0];
-  g_split_stats[1] = st[0];
-  g_split_stats[2] = st[1];
-  g_split_stats[3] = 1;
-  return MPN_OK;
-}
-
-static int split_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride, int num_cameras, int* rounds) {
-  const int A = c.n_active, N = c.g.n_nodes;
-  *rounds = 0;
-  g_split_stats[0] = g_split_stats[1] = g_split_stats[2] = g_split_stats[3] = 0;
-  if (A == 0) return MPN_OK;
-  // round 0 on the whole graph: components, sizes, dirty lists
-  MPN_TRY(scc_stage(c, act, nullptr));
-  MPN_CUDA_OK(cudaMemsetAsync(c.size, 0, sizeof(int) * N, c.st));
-  MPN_CUDA_OK(cudaMemsetAsync(c.counters + 5, 0, 4 * sizeof(int), c.st));
-  comp_size_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size);
-  MPN_LAUNCH_OK();
-  mark_dirty_nodes_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size, num_cameras, c.dirty_nodes, c.counters + 5);
-  MPN_LAUNCH_OK();
-  mark_dirty_edges_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.label, c.size, num_cameras, c.dirty_edges,
-                                                         c.counters + 6);
-  MPN_LAUNCH_OK();
-  int h[2] = {0, 0};
-  MPN_CUDA_OK(cudaMemcpyAsync(h, c.counters + 5, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  const int Dn = h[0], De = h[1];
-  static const bool dbg = getenv("MPN_POST_DEBUG") != nullptr;
-  if (dbg) fprintf(stderr, "[split] A=%d N=%d dirty nodes=%d dirty edges=%d\n", A, N, Dn, De);
-  if (Dn == 0) return MPN_OK;
-  // ---- probability ties among the values an oversized cluster can drop?
-  iota_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.wcc);
-  MPN_LAUNCH_OK();
-  union_all_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.wcc);
-  MPN_LAUNCH_OK();
-  flatten_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.wcc, nullptr);
-  MPN_LAUNCH_OK();
-  MPN_CUDA_OK(cudaMemsetAsync(c.wccflag, 0, sizeof(int) * N, c.st));
-  const bool table_fits = (long long)De * 5 <= (long long)c.tie_cap * 3;       // load factor <= 0.6
-  int n_tied = 0;
-  if (table_fits) {
-    MPN_CUDA_OK(cudaMemsetAsync(c.tie_keys, 0xFF, sizeof(unsigned int) * c.tie_cap, c.st));
-    MPN_CUDA_OK(cudaMemsetAsync(c.tie_counts, 0, sizeof(int) * c.tie_cap, c.st));
-    if (De > 0) {
-      tie_insert_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, act, prob, pstride, c.tie_keys, c.tie_cap);
-      MPN_LAUNCH_OK();
-    }
-    tie_count_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, act, prob, pstride, c.tie_keys, c.tie_counts, c.tie_cap);
-    MPN_LAUNCH_OK();
-    flag_wcc_ties_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, act, prob, pstride, c.tie_keys, c.tie_counts, c.tie_cap,
-                                                         c.wcc, c.wccflag, c.tiedb, c.counters + 7);
-    MPN_LAUNCH_OK();
-    MPN_CUDA_OK(cudaMemcpyAsync(&n_tied, c.counters + 7, sizeof(int), cudaMemcpyDeviceToHost, c.st));
-    MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  }
-  g_split_stats[0] = table_fits ? n_tied : -1;
-  if (dbg) fprintf(stderr, "[split] active edges carrying a tied value: %d%s\n", n_tied, table_fits ? "" : " (table too small: all active edges go to the host)");
-  if (!table_fits || n_tied > 0) {
-    if (!table_fits) {
-      MPN_CUDA_OK(cudaMemsetAsync(c.wccflag, 0x01, sizeof(int) * N, c.st));   // every component (any non-zero flag)
-    } else {
-      flag_wcc_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.wcc, c.wccflag);
-      MPN_LAUNCH_OK();
-    }
-    return split_in_reference_order(c, act, prob, pstride, num_cameras, Dn, table_fits, rounds);
-  }
-  // ---- no ties: the clusters are independent, every oversized cluster drops its minimum in the same round
-  for (;;) {
-    // per-cluster minimum probability over the active edges touching each oversized cluster
-    reset_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, c.mbits, 4);
-    MPN_LAUNCH_OK();
-    MPN_CUDA_OK(cudaMemsetAsync(c.hash, 0xFF, sizeof(unsigned int) * c.hash_cap, c.st));
-    MPN_CUDA_OK(cudaMemsetAsync(c.counters + 4, 0, sizeof(int), c.st));
-    if (De > 0) {
-      split_min_list_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, c.a_dst, act, prob, pstride, c.label,
-                                                           c.size, num_cameras, c.mbits);
-      MPN_LAUNCH_OK();
-    }
-    split_collect_list_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, num_cameras, c.mbits, c.hash,
-                                                              c.hash_cap, c.counters + 4);
-    MPN_LAUNCH_OK();
-    int n_big = 0;
-    MPN_CUDA_OK(cudaMemcpyAsync(&n_big, c.counters + 4, sizeof(int), cudaMemcpyDeviceToHost, c.st));
-    MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-    if (n_big == 0) break;
-    ++*rounds;
-    if (*rounds > A + 1) { set_error("split did not converge"); return MPN_ERR_INVALID; }
-    // every edge anywhere whose probability equals one of the minima (utils.py:96-98)
-    split_remove_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, act, prob, pstride, c.hash, c.hash_cap);
-    MPN_LAUNCH_OK();
-    // recompute components and sizes of the dirty part only
-    MPN_TRY(scc_dirty(c, act, Dn, De));
-    reset_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, c.mbits, 2);
-    MPN_LAUNCH_OK();
-    comp_size_list_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size);
-    MPN_LAUNCH_OK();
-  }
-  g_split_stats[1] = *rounds;
-  return MPN_OK;
-}
-
-// ------------------------------------------------------------------------------------------------
-// Batched graphs (n_graphs > 1): G block-diagonal graphs, nodes of a graph contiguous, edges (row, col)-sorted, so the active
-// entries of graph g are the contiguous slice [a_gptr[g], a_gptr[g+1]) of the active list.  CUT, the union-find SCC and the
-// canonical labels are graph-local as they stand (the reverse edge and every SCC lie inside one graph); what the kernels below add
-// is the per-graph camera bound and, for SPLITTING, sets keyed by (graph id, probability bits): the reference removes every edge
-// of ITS graph whose probability equals the dropped minimum (utils.py:96-98), so a value shared by two different graphs must
-// neither couple them nor count as a tie.
-// ------------------------------------------------------------------------------------------------
-constexpr unsigned long long HASH64_EMPTY = ~0ull;         // never a key: graph ids are < 2^31
-__device__ __forceinline__ unsigned long long graph_value_key(int g, unsigned int bits) {
-  return ((unsigned long long)(unsigned int)g << 32) | bits;
-}
-__device__ __forceinline__ unsigned int hash_u64(unsigned long long k) {
-  return hash_u32((unsigned int)k ^ hash_u32((unsigned int)(k >> 32) + 0x9e3779b9u));
-}
-__device__ __forceinline__ void set64_insert(unsigned long long* __restrict__ t, int cap, unsigned long long key) {
-  unsigned int slot = hash_u64(key) & (cap - 1);
-  for (;;) {
-    const unsigned long long old = atomicCAS(&t[slot], HASH64_EMPTY, key);
-    if (old == HASH64_EMPTY || old == key) return;
-    slot = (slot + 1) & (cap - 1);
-  }
-}
-__device__ __forceinline__ int set64_find(const unsigned long long* __restrict__ t, int cap, unsigned long long key) {
-  unsigned int slot = hash_u64(key) & (cap - 1);
-  for (;;) {
-    const unsigned long long v = t[slot];
-    if (v == key) return (int)slot;
-    if (v == HASH64_EMPTY) return -1;
-    slot = (slot + 1) & (cap - 1);
-  }
-}
-
-// a_gptr[g] = first active-list entry at or after the first edge of graph g (a_eid ascends); a_gptr[G] = A
-__global__ void active_graph_ptr_kernel(int G, const int* __restrict__ rowptr, const int* __restrict__ nptr, const int* __restrict__ a_eid,
-                                        int A, int* __restrict__ a_gptr) {
-  for (int g = blockIdx.x * blockDim.x + threadIdx.x; g <= G; g += gridDim.x * blockDim.x) {
-    const int e0 = rowptr[nptr[g]];
-    int lo = 0, hi = A;
-    while (lo < hi) {
-      const int mid = (lo + hi) >> 1;
-      if (a_eid[mid] < e0) lo = mid + 1; else hi = mid;
-    }
-    a_gptr[g] = lo;
-  }
-}
-// canonical graph-local labels (smallest node id of the SCC minus the graph's first node) and the number of SCCs per graph
-__global__ void graph_labels_kernel(int N, const int* __restrict__ label, const int* __restrict__ gid, const int* __restrict__ nptr,
-                                    int* __restrict__ local, int* __restrict__ roots) {
-  for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) {
-    const int g = gid[n], l = label[n];
-    if (local) local[n] = l - nptr[g];
-    if (l == n) atomicAdd(&roots[g], 1);
-  }
-}
-// skip (optional): graphs whose clusters are left out (they go through the reference order on the host)
-__global__ void mark_dirty_nodes_batched_kernel(int N, const int* __restrict__ label, const int* __restrict__ size, const int* __restrict__ gid,
-                                                const int* __restrict__ ncam, const int* __restrict__ skip, int* __restrict__ list,
-                                                int* __restrict__ count) {
-  for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) {
-    const int g = gid[n];
-    if ((skip == nullptr || !skip[g]) && size[label[n]] > ncam[g]) list[atomicAdd(count, 1)] = n;
-  }
-}
-__global__ void mark_dirty_edges_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src,
-                                                const int* __restrict__ a_dst, const uint8_t* __restrict__ act, const int* __restrict__ label,
-                                                const int* __restrict__ size, const int* __restrict__ gid, const int* __restrict__ ncam,
-                                                const int* __restrict__ skip, int* __restrict__ list, int* __restrict__ count) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
-    if (!act[a_eid[i]]) continue;
-    const int g = gid[a_src[i]];
-    if (skip != nullptr && skip[g]) continue;
-    const int limit = ncam[g];
-    if (size[label[a_src[i]]] > limit || size[label[a_dst[i]]] > limit) list[atomicAdd(count, 1)] = i;
-  }
-}
-__global__ void split_min_list_batched_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ a_eid,
-                                              const int* __restrict__ a_src, const int* __restrict__ a_dst, const uint8_t* __restrict__ act,
-                                              const float* __restrict__ prob, int pstride, const int* __restrict__ label,
-                                              const int* __restrict__ size, const int* __restrict__ gid, const int* __restrict__ ncam,
-                                              unsigned int* __restrict__ mbits) {
-  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
-    const int i = list[k];
-    const int e = a_eid[i];
-    if (!act[e]) continue;
-    const int lu = label[a_src[i]], lv = label[a_dst[i]];
-    const int limit = ncam[gid[a_src[i]]];
-    const unsigned int pb = __float_as_uint(prob[(size_t)e * pstride]);
-    if (size[lu] > limit) atomicMin(&mbits[lu], pb);
-    if (lv != lu && size[lv] > limit) atomicMin(&mbits[lv], pb);
-  }
-}
-__global__ void split_collect_list_batched_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ label,
-                                                  const int* __restrict__ size, const int* __restrict__ gid, const int* __restrict__ ncam,
-                                                  const unsigned int* __restrict__ mbits, unsigned long long* __restrict__ hash, int cap,
-                                                  int* __restrict__ n_big) {
-  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
-    const int n = list[k];
-    if (label[n] != n || size[n] <= ncam[gid[n]]) continue;
-    atomicAdd(n_big, 1);
-    const unsigned int bits = mbits[n];
-    if (bits == HASH_EMPTY) continue;
-    set64_insert(hash, cap, graph_value_key(gid[n], bits));
-  }
-}
-// every active edge of a graph whose probability equals one of that graph's dropped minima (utils.py:96-98)
-__global__ void split_remove_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ gid,
-                                            uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
-                                            const unsigned long long* __restrict__ hash, int cap) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
-    const int e = a_eid[i];
-    if (!act[e]) continue;
-    if (set64_find(hash, cap, graph_value_key(gid[a_src[i]], __float_as_uint(prob[(size_t)e * pstride]))) >= 0) act[e] = 0;
-  }
-}
-// ties per graph: the values of the dirty edges, how many active edges of the SAME graph carry each, the graphs that have one
-__global__ void tie_insert_batched_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ a_eid, const int* __restrict__ a_src,
-                                          const int* __restrict__ gid, const uint8_t* __restrict__ act, const float* __restrict__ prob,
-                                          int pstride, unsigned long long* __restrict__ keys, int cap) {
-  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) {
-    const int i = list[k];
-    const int e = a_eid[i];
-    if (!act[e]) continue;
-    set64_insert(keys, cap, graph_value_key(gid[a_src[i]], __float_as_uint(prob[(size_t)e * pstride])));
-  }
-}
-__global__ void tie_count_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ gid,
-                                         const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
-                                         const unsigned long long* __restrict__ keys, int* __restrict__ counts, int cap) {
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
-    const int e = a_eid[i];
-    if (!act[e]) continue;
-    const int slot = set64_find(keys, cap, graph_value_key(gid[a_src[i]], __float_as_uint(prob[(size_t)e * pstride])));
-    if (slot >= 0) atomicAdd(&counts[slot], 1);
-  }
-}
-__global__ void flag_wcc_ties_batched_kernel(int A, const int* __restrict__ a_eid, const int* __restrict__ a_src, const int* __restrict__ gid,
-                                             const uint8_t* __restrict__ act, const float* __restrict__ prob, int pstride,
-                                             const unsigned long long* __restrict__ keys, const int* __restrict__ counts, int cap,
-                                             const int* __restrict__ wcc, int* __restrict__ flag, uint8_t* __restrict__ tiedb,
-                                             int* __restrict__ gtied, int* __restrict__ n_tied_edges) {
-  int tied = 0;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < A; i += gridDim.x * blockDim.x) {
-    const int e = a_eid[i];
-    uint8_t t = 0;
-    if (act[e]) {
-      const int g = gid[a_src[i]];
-      const int slot = set64_find(keys, cap, graph_value_key(g, __float_as_uint(prob[(size_t)e * pstride])));
-      if (slot >= 0 && counts[slot] >= 2) { flag[wcc[a_src[i]]] = 1; gtied[g] = 1; ++tied; t = 1; }
-    }
-    tiedb[i] = t;
-  }
-  tied = __reduce_add_sync(0xffffffffu, tied);
-  if ((threadIdx.x & 31) == 0 && tied) atomicAdd(n_tied_edges, tied);
-}
-__global__ void flag_graphs_of_nodes_kernel(int n_list, const int* __restrict__ list, const int* __restrict__ gid, int* __restrict__ gflag) {
-  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_list; k += gridDim.x * blockDim.x) gflag[gid[list[k]]] = 1;
-}
-
-static int copy_graph_ptr(const PostCtx& c, std::vector<int>& nptr) {
-  nptr.resize((size_t)c.g.n_graphs + 1);
-  MPN_CUDA_OK(cudaMemcpyAsync(nptr.data(), c.g.graph_nptr, sizeof(int) * nptr.size(), cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  return MPN_OK;
-}
-
-// The reference order on the host for the graphs flagged in c.gflag (a probability tie among the values one of their oversized
-// clusters can drop): one split_exact_host_impl call per graph on its own slice of the active list, with graph-local node ids,
-// its own node count and camera bound — exactly the call a single-graph post-processing of that graph makes, so the engine's
-// numbering and its re-read of the integer label (utils.py:112) are the graph's own.  Graphs are independent: they run on a few
-// host threads, each writing its own slice, and the result depends neither on the thread count nor on the order of the seeds.
+// The reference order on the host for the graphs flagged in host_graph: one split_exact_host_impl call per graph on its own slice of
+// the active list, with graph-local node ids, its own node count and camera bound — exactly the call a single-graph
+// post-processing of that graph makes, so the engine's numbering and its re-read of the integer label (utils.py:112) are the
+// graph's own.  Graphs are independent: they run on a few host threads, each writing its own slice, and the result depends
+// neither on the thread count nor on the order of the seeds.
 static int split_host_graphs(PostCtx& c, uint8_t* act, const float* prob, int pstride, const std::vector<int>& ncam,
                              const std::vector<int>& nptr, const std::vector<int>& host_graph, int Dn, bool have_ties,
                              long long* steps, long long* off_lowest) {
-  const int A = c.n_active, G = c.g.n_graphs;
+  const int A = c.n_active, G = (int)ncam.size();
   gather_select_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, act, prob, pstride, c.wcc, c.wccflag, c.a_prob, c.sel);
   MPN_LAUNCH_OK();
-  active_graph_ptr_kernel<<<list_grid(G + 1), 256, 0, c.st>>>(G, c.g.rowptr, c.g.graph_nptr, c.a_eid, A, c.a_gptr);
-  MPN_LAUNCH_OK();
-  std::vector<int> agp((size_t)G + 1), seeds(Dn);
-  MPN_CUDA_OK(cudaMemcpyAsync(agp.data(), c.a_gptr, sizeof(int) * (G + 1), cudaMemcpyDeviceToHost, c.st));
+  std::vector<int> agp{0, A}, seeds(Dn);                // one graph: its slice is the whole active list
+  if (G > 1) {
+    agp.resize((size_t)G + 1);
+    active_graph_ptr_kernel<<<list_grid(G + 1), 256, 0, c.st>>>(G, c.g.rowptr, c.g.graph_nptr, c.a_eid, A, c.a_gptr);
+    MPN_LAUNCH_OK();
+    MPN_CUDA_OK(cudaMemcpyAsync(agp.data(), c.a_gptr, sizeof(int) * (G + 1), cudaMemcpyDeviceToHost, c.st));
+  }
   MPN_CUDA_OK(cudaMemcpyAsync(seeds.data(), c.dirty_nodes, sizeof(int) * Dn, cudaMemcpyDeviceToHost, c.st));
   MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  // runs of consecutive host-order graphs = contiguous ranges of the active list, packed back to back in pinned staging
+  // runs of consecutive host-order graphs = contiguous ranges of the active list, packed back to back in pinned staging (pageable
+  // destinations would be staged by the driver at a few GB/s)
   struct Run { int g0, g1; long long a0, a1, h0; };
   std::vector<Run> runs;
   long long staged = 0;
@@ -1178,9 +855,13 @@ static int split_host_graphs(PostCtx& c, uint8_t* act, const float* prob, int ps
   for (const Run& r : runs)
     for (int g = r.g0; g < r.g1; ++g) { graphs.push_back(g); h_of[g] = r.h0 + (agp[g] - r.a0); }
   std::vector<std::vector<int>> gseeds((size_t)G);
-  for (int v : seeds) {
-    const int g = (int)(std::upper_bound(nptr.begin(), nptr.end(), v) - nptr.begin()) - 1;
-    if (host_graph[g]) gseeds[g].push_back(v - nptr[g]);
+  if (G == 1) {
+    gseeds[0] = std::move(seeds);                  // one graph: every seed is its own, in its own ids
+  } else {
+    for (int v : seeds) {
+      const int g = (int)(std::upper_bound(nptr.begin(), nptr.end(), v) - nptr.begin()) - 1;
+      if (host_graph[g]) gseeds[g].push_back(v - nptr[g]);
+    }
   }
   std::vector<int64_t> gst(4 * (size_t)G, 0);
   std::vector<int> rc((size_t)G, MPN_OK);
@@ -1193,10 +874,15 @@ static int split_host_graphs(PostCtx& c, uint8_t* act, const float* prob, int ps
       const long long h = h_of[g], m = agp[g + 1] - agp[g];
       const int n0 = nptr[g];
       long long n_sel = 0;
-      ls.resize(m); ld.resize(m);
-      for (long long i = 0; i < m; ++i) { ls[i] = hs[h + i] - n0; ld[i] = hd[h + i] - n0; n_sel += hsel[h + i]; }
+      for (long long i = 0; i < m; ++i) n_sel += hsel[h + i];
       if (n_sel == 0) { memset(keep + h, 1, (size_t)m); continue; }
-      rc[g] = split_exact_host_impl(ls.data(), ld.data(), hp + h, m, nptr[g + 1] - n0, ncam[g], keep + h, &gst[4 * (size_t)g],
+      const int *s = hs + h, *d = hd + h;             // node ids are graph-local already when the graph starts at node 0
+      if (n0 != 0) {
+        ls.resize(m); ld.resize(m);
+        for (long long i = 0; i < m; ++i) { ls[i] = s[i] - n0; ld[i] = d[i] - n0; }
+        s = ls.data(); d = ld.data();
+      }
+      rc[g] = split_exact_host_impl(s, d, hp + h, m, nptr[g + 1] - n0, ncam[g], keep + h, &gst[4 * (size_t)g],
                                     have_ties ? htied + h : nullptr, gseeds[g].data(), (long long)gseeds[g].size(), hsel + h);
       if (rc[g] != MPN_OK) err[g] = mpn_last_error();
     }
@@ -1214,7 +900,7 @@ static int split_host_graphs(PostCtx& c, uint8_t* act, const float* prob, int ps
   *steps = *off_lowest = 0;
   for (int g : graphs) { *steps += gst[4 * (size_t)g]; *off_lowest += gst[4 * (size_t)g + 1]; }
   // write back: keep = 1 everywhere but in the slices the engine decided
-  MPN_CUDA_OK(cudaMemsetAsync(c.sel, 1, (size_t)A, c.st));
+  if (staged < A) MPN_CUDA_OK(cudaMemsetAsync(c.sel, 1, (size_t)A, c.st));
   for (const Run& r : runs)
     if (r.a1 > r.a0) MPN_CUDA_OK(cudaMemcpyAsync(c.sel + r.a0, keep + r.h0, (size_t)(r.a1 - r.a0), cudaMemcpyHostToDevice, c.st));
   apply_keep_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.sel, act);
@@ -1223,30 +909,33 @@ static int split_host_graphs(PostCtx& c, uint8_t* act, const float* prob, int ps
   return MPN_OK;
 }
 
-// SPLITTING of every graph of the batch.  The mode is chosen per graph: a graph with a tie among the values its oversized clusters
-// can drop (or every graph with an oversized cluster, when the tie table does not fit) goes through the reference order on the
-// host; the others drop their minima in parallel rounds on the device, restricted to their own dirty lists.  Graphs are
-// independent, so both modes run on one batch and the result is exact.
-static int split_stage_batched(PostCtx& c, uint8_t* act, const float* prob, int pstride, const int* ncam_dev,
-                               const std::vector<int>& ncam, const std::vector<int>& nptr) {
-  const int A = c.n_active, N = c.g.n_nodes, G = c.g.n_graphs;
-  const int* gid = c.g.node_gid;
+// SPLITTING of every graph; ncam / nptr: camera count and first node of each graph ({C} and {0, N} for one graph).  The mode is
+// chosen per graph: a graph with a tie among the values its oversized clusters can drop (or every graph with an oversized
+// cluster, when the tie table does not fit) goes through the reference order on the host; the others drop their minima in
+// parallel rounds on the device, restricted to their own dirty lists.  Graphs are independent, so both modes run on one batch and
+// the result is exact.
+static int split_stage(PostCtx& c, uint8_t* act, const float* prob, int pstride, const Graphs& graphs, const std::vector<int>& ncam,
+                       const std::vector<int>& nptr) {
+  const int A = c.n_active, N = c.g.n_nodes, G = (int)ncam.size();
   g_split_stats[0] = g_split_stats[1] = g_split_stats[2] = g_split_stats[3] = 0;
   if (A == 0) return MPN_OK;
+  // round 0 on the whole graph: components, sizes, dirty lists
   MPN_TRY(scc_stage(c, act, nullptr));
   MPN_CUDA_OK(cudaMemsetAsync(c.size, 0, sizeof(int) * N, c.st));
-  MPN_CUDA_OK(cudaMemsetAsync(c.counters + 5, 0, 4 * sizeof(int), c.st));
+  MPN_CUDA_OK(cudaMemsetAsync(c.counters + 5, 0, 2 * sizeof(int), c.st));
   comp_size_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size);
   MPN_LAUNCH_OK();
-  mark_dirty_nodes_batched_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size, gid, ncam_dev, nullptr, c.dirty_nodes, c.counters + 5);
+  mark_dirty_nodes_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size, graphs, nullptr, c.dirty_nodes, c.counters + 5);
   MPN_LAUNCH_OK();
-  mark_dirty_edges_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.label, c.size, gid, ncam_dev, nullptr,
-                                                                  c.dirty_edges, c.counters + 6);
+  mark_dirty_edges_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.label, c.size, graphs, nullptr,
+                                                         c.dirty_edges, c.counters + 6);
   MPN_LAUNCH_OK();
   int h[2] = {0, 0};
   MPN_CUDA_OK(cudaMemcpyAsync(h, c.counters + 5, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.st));
   MPN_CUDA_OK(cudaStreamSynchronize(c.st));
   int Dn = h[0], De = h[1];
+  static const bool dbg = getenv("MPN_POST_DEBUG") != nullptr;
+  if (dbg) fprintf(stderr, "[split] A=%d N=%d dirty nodes=%d dirty edges=%d\n", A, N, Dn, De);
   if (Dn == 0) return MPN_OK;
   // ---- which graphs have a tie among the values their oversized clusters can drop?
   iota_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.wcc);
@@ -1256,65 +945,71 @@ static int split_stage_batched(PostCtx& c, uint8_t* act, const float* prob, int 
   flatten_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.wcc, nullptr);
   MPN_LAUNCH_OK();
   MPN_CUDA_OK(cudaMemsetAsync(c.wccflag, 0, sizeof(int) * N, c.st));
-  MPN_CUDA_OK(cudaMemsetAsync(c.gflag, 0, sizeof(int) * G, c.st));
+  MPN_CUDA_OK(cudaMemsetAsync(c.gflag, 0, sizeof(int) * (G + 1), c.st));
   const bool table_fits = (long long)De * 5 <= (long long)c.tie_cap * 3;       // load factor <= 0.6
-  int n_tied = 0;
   if (table_fits) {
-    MPN_CUDA_OK(cudaMemsetAsync(c.tie_keys64, 0xFF, sizeof(unsigned long long) * c.tie_cap, c.st));
+    MPN_CUDA_OK(cudaMemsetAsync(c.tie_keys, 0xFF, sizeof(unsigned long long) * c.tie_cap, c.st));
     MPN_CUDA_OK(cudaMemsetAsync(c.tie_counts, 0, sizeof(int) * c.tie_cap, c.st));
     if (De > 0) {
-      tie_insert_batched_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, gid, act, prob, pstride, c.tie_keys64,
-                                                                 c.tie_cap);
+      tie_insert_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, graphs, act, prob, pstride, c.tie_keys,
+                                                         c.tie_cap);
       MPN_LAUNCH_OK();
     }
-    tie_count_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, gid, act, prob, pstride, c.tie_keys64, c.tie_counts,
-                                                             c.tie_cap);
+    tie_count_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, graphs, act, prob, pstride, c.tie_keys, c.tie_counts, c.tie_cap);
     MPN_LAUNCH_OK();
-    flag_wcc_ties_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, gid, act, prob, pstride, c.tie_keys64, c.tie_counts,
-                                                                 c.tie_cap, c.wcc, c.wccflag, c.tiedb, c.gflag, c.counters + 7);
-    MPN_LAUNCH_OK();
-    flag_wcc_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.wcc, c.wccflag);
+    flag_wcc_ties_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, graphs, act, prob, pstride, c.tie_keys, c.tie_counts,
+                                                         c.tie_cap, c.wcc, c.wccflag, c.tiedb, c.gflag, c.gflag + G);
     MPN_LAUNCH_OK();
   } else {
     MPN_CUDA_OK(cudaMemsetAsync(c.wccflag, 0x01, sizeof(int) * N, c.st));   // every component of the host-order graphs
-    flag_graphs_of_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, gid, c.gflag);
+    flag_graphs_of_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, graphs, c.gflag);
     MPN_LAUNCH_OK();
   }
-  std::vector<int> host_graph((size_t)G);
-  MPN_CUDA_OK(cudaMemcpyAsync(host_graph.data(), c.gflag, sizeof(int) * G, cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaMemcpyAsync(&n_tied, c.counters + 7, sizeof(int), cudaMemcpyDeviceToHost, c.st));
+  std::vector<int> host_graph((size_t)G + 1);
+  MPN_CUDA_OK(cudaMemcpyAsync(host_graph.data(), c.gflag, sizeof(int) * (G + 1), cudaMemcpyDeviceToHost, c.st));
   MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  const int n_tied = host_graph[G];
   long long n_host = 0, host_steps = 0, host_off_lowest = 0;
   for (int g = 0; g < G; ++g) n_host += host_graph[g] != 0;
   g_split_stats[0] = table_fits ? n_tied : -1;
+  if (dbg) fprintf(stderr, "[split] active edges carrying a tied value: %d%s; graphs in the reference order: %lld of %d\n", n_tied,
+                   table_fits ? "" : " (table too small: every graph with an oversized cluster goes to the host)", n_host, G);
   if (n_host > 0) {
+    if (table_fits) {                               // the components of the oversized clusters go to the host with their graph
+      flag_wcc_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.wcc, c.wccflag);
+      MPN_LAUNCH_OK();
+    }
     MPN_TRY(split_host_graphs(c, act, prob, pstride, ncam, nptr, host_graph, Dn, table_fits, &host_steps, &host_off_lowest));
-    // the device rounds below only see the other graphs
-    MPN_CUDA_OK(cudaMemsetAsync(c.counters + 5, 0, 2 * sizeof(int), c.st));
-    mark_dirty_nodes_batched_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size, gid, ncam_dev, c.gflag, c.dirty_nodes, c.counters + 5);
-    MPN_LAUNCH_OK();
-    mark_dirty_edges_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.label, c.size, gid, ncam_dev, c.gflag,
-                                                                    c.dirty_edges, c.counters + 6);
-    MPN_LAUNCH_OK();
-    MPN_CUDA_OK(cudaMemcpyAsync(h, c.counters + 5, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.st));
-    MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-    Dn = h[0];
-    De = h[1];
+    if (n_host == G) {
+      Dn = 0;                                       // no graph is left for the device rounds
+    } else {                                        // the device rounds below only see the other graphs
+      MPN_CUDA_OK(cudaMemsetAsync(c.counters + 5, 0, 2 * sizeof(int), c.st));
+      mark_dirty_nodes_kernel<<<list_grid(N), 256, 0, c.st>>>(N, c.label, c.size, graphs, c.gflag, c.dirty_nodes, c.counters + 5);
+      MPN_LAUNCH_OK();
+      mark_dirty_edges_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, c.a_dst, act, c.label, c.size, graphs, c.gflag,
+                                                             c.dirty_edges, c.counters + 6);
+      MPN_LAUNCH_OK();
+      MPN_CUDA_OK(cudaMemcpyAsync(h, c.counters + 5, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.st));
+      MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+      Dn = h[0];
+      De = h[1];
+    }
   }
   // ---- no tie inside any of the remaining graphs: every oversized cluster drops its minimum in the same round
   int rounds = 0;
   while (Dn > 0) {
+    // per-cluster minimum probability over the active edges touching each oversized cluster
     reset_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, c.mbits, 4);
     MPN_LAUNCH_OK();
-    MPN_CUDA_OK(cudaMemsetAsync(c.hash64, 0xFF, sizeof(unsigned long long) * c.hash_cap, c.st));
+    MPN_CUDA_OK(cudaMemsetAsync(c.hash, 0xFF, sizeof(unsigned long long) * c.hash_cap, c.st));
     MPN_CUDA_OK(cudaMemsetAsync(c.counters + 4, 0, sizeof(int), c.st));
     if (De > 0) {
-      split_min_list_batched_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, c.a_dst, act, prob, pstride,
-                                                                     c.label, c.size, gid, ncam_dev, c.mbits);
+      split_min_list_kernel<<<list_grid(De), 256, 0, c.st>>>(De, c.dirty_edges, c.a_eid, c.a_src, c.a_dst, act, prob, pstride, c.label,
+                                                           c.size, graphs, c.mbits);
       MPN_LAUNCH_OK();
     }
-    split_collect_list_batched_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, gid, ncam_dev, c.mbits, c.hash64,
-                                                                       c.hash_cap, c.counters + 4);
+    split_collect_list_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, graphs, c.mbits, c.hash, c.hash_cap,
+                                                              c.counters + 4);
     MPN_LAUNCH_OK();
     int n_big = 0;
     MPN_CUDA_OK(cudaMemcpyAsync(&n_big, c.counters + 4, sizeof(int), cudaMemcpyDeviceToHost, c.st));
@@ -1322,8 +1017,9 @@ static int split_stage_batched(PostCtx& c, uint8_t* act, const float* prob, int 
     if (n_big == 0) break;
     ++rounds;
     if (rounds > A + 1) { set_error("split did not converge"); return MPN_ERR_INVALID; }
-    split_remove_batched_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, gid, act, prob, pstride, c.hash64, c.hash_cap);
+    split_remove_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, graphs, act, prob, pstride, c.hash, c.hash_cap);
     MPN_LAUNCH_OK();
+    // recompute components and sizes of the dirty part only
     MPN_TRY(scc_dirty(c, act, Dn, De));
     reset_nodes_kernel<<<list_grid(Dn), 256, 0, c.st>>>(Dn, c.dirty_nodes, c.label, c.size, c.mbits, 2);
     MPN_LAUNCH_OK();
@@ -1349,6 +1045,13 @@ static int post_begin(PostCtx& c, const mpn_graph* g, const uint8_t* act, void* 
     return MPN_ERR_WORKSPACE;
   }
   return build_active_list(c, act);
+}
+
+static int copy_graph_ptr(const PostCtx& c, std::vector<int>& nptr) {
+  nptr.resize((size_t)c.g.n_graphs + 1);
+  MPN_CUDA_OK(cudaMemcpyAsync(nptr.data(), c.g.graph_nptr, sizeof(int) * nptr.size(), cudaMemcpyDeviceToHost, c.st));
+  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
+  return MPN_OK;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1507,7 +1210,7 @@ static int reference_keys(PostCtx& c, const uint8_t* act, RefKeys& k) {
     select_flagged_kernel<<<list_grid(A), 256, 0, c.st>>>(A, c.a_eid, c.a_src, act, c.wcc, c.wccflag, c.sel);
     MPN_LAUNCH_OK();
     const size_t A16 = ((size_t)A + 15) & ~(size_t)15;
-    char* pin = (char*)g_split_pin.get(9 * A16 + 64);          // pinned staging (see split_in_reference_order)
+    char* pin = (char*)g_split_pin.get(9 * A16 + 64);          // pinned staging (see split_host_graphs)
     MPN_REQUIRE(pin != nullptr, "reference numbering: out of pinned host memory");
     int *hs = (int*)pin, *hd = (int*)(pin + 4 * A16);
     uint8_t* hsel = (uint8_t*)(pin + 8 * A16);
@@ -1578,69 +1281,75 @@ static int roots_in_reference_order(const RefKeys& k, int A, std::vector<int>& o
   return MPN_OK;
 }
 
-static int labels_reference_parallel(PostCtx& c, const uint8_t* act, long long* labels_out, int* n_comp_out) {
-  const int N = c.g.n_nodes;
+// Reference numbering of each graph from 0 on its own; nptr = first node of each graph ({0, N} for one graph).  A DFS never leaves
+// its graph and the active list holds the graphs one after the other, so a component's (key, idx) orders it within its graph
+// exactly as numbering that graph alone does (keys shifted by the graph's first active entry); the order (size, key, idx) then
+// becomes (graph, size, key, idx) — a stable pass by graph over the whole order — and the nodes without an active edge follow
+// their own graph's components, in node order.
+static int labels_reference_per_graph(PostCtx& c, const uint8_t* act, const std::vector<int>& nptr, long long* labels_out,
+                                      int* n_comp_out) {
+  const int N = c.g.n_nodes, G = (int)nptr.size() - 1;
   RefKeys k;
   MPN_TRY(reference_keys(c, act, k));
   std::vector<int> order;
   MPN_TRY(roots_in_reference_order(k, c.n_active, order));
-  std::vector<int> rank(N, -1);
-  for (size_t i = 0; i < order.size(); ++i) rank[order[i]] = (int)i;
-  long long next = (long long)order.size();
-  for (int n = 0; n < N; ++n) labels_out[n] = (k.fa[n] != 0xFFFFFFFFu) ? rank[k.label[n]] : next++;
-  if (n_comp_out) *n_comp_out = (int)next;
-  return MPN_OK;
-}
-
-// Batched graphs: each graph numbered from 0 on its own.  A DFS never leaves its graph and the active list holds the graphs one
-// after the other, so a component's (key, idx) orders it within its graph exactly as the single-graph numbering does (keys shifted
-// by the graph's first active entry); the order (size, key, idx) then becomes (graph, size, key, idx) — a stable pass by graph
-// over the single-graph order — and the nodes without an active edge follow their own graph's components, in node order.
-static int labels_reference_batched(PostCtx& c, const uint8_t* act, const std::vector<int>& nptr, long long* labels_out,
-                                    int* n_comp_out) {
-  const int N = c.g.n_nodes, G = c.g.n_graphs;
-  RefKeys k;
-  MPN_TRY(reference_keys(c, act, k));
-  std::vector<int> order;
-  MPN_TRY(roots_in_reference_order(k, c.n_active, order));
-  std::vector<int> gid((size_t)N);
-  for (int g = 0; g < G; ++g)
-    for (int n = nptr[g]; n < nptr[g + 1]; ++n) gid[n] = g;
-  std::vector<int> start((size_t)G + 1, 0);             // components with an active edge per graph -> first position
-  for (int r : order) ++start[gid[r] + 1];
-  for (int g = 0; g < G; ++g) start[g + 1] += start[g];
-  std::vector<int> rank(N, -1);
-  {
-    std::vector<int> fill(start.begin(), start.end() - 1);
-    for (int r : order) { const int g = gid[r]; rank[r] = fill[g]++ - start[g]; }
+  std::vector<int> rank((size_t)N, -1), count((size_t)G, 0);      // rank[r]: the place of root r among its graph's SCCs
+  if (G == 1) {                                                    // one graph: its place in the order, no per-node graph ids
+    for (size_t i = 0; i < order.size(); ++i) rank[order[i]] = (int)i;
+    count[0] = (int)order.size();
+  } else {
+    // graph ids in an array of their own: reading them back from rank would chain each root on the previous root's store
+    std::vector<int> gid((size_t)N);
+    for (int g = 0; g < G; ++g) std::fill(gid.begin() + nptr[g], gid.begin() + nptr[g + 1], g);
+    for (int r : order) rank[r] = count[gid[r]]++;
   }
   for (int g = 0; g < G; ++g) {
-    long long next = start[g + 1] - start[g];
+    long long next = count[g];
     for (int n = nptr[g]; n < nptr[g + 1]; ++n) labels_out[n] = (k.fa[n] != 0xFFFFFFFFu) ? rank[k.label[n]] : next++;
     n_comp_out[g] = (int)next;
   }
   return MPN_OK;
 }
 
-// inference.post_processing (inference.py:70-169) on one graph: CUT, PRUNE, CUT, SPLIT, then the SCC labels
-static int post_processing_one_graph(PostCtx& c, uint8_t* act, const float* prob1, int pstride, int num_cameras, int flags, int32_t* labels,
-                                     int32_t* n_components, int32_t* prune_changed) {
+// canonical graph-local labels (smallest node id of the SCC minus the graph's first node) and the number of SCCs per graph
+__global__ void graph_labels_kernel(int N, const int* __restrict__ label, const Graphs graphs, const int* __restrict__ nptr,
+                                    int* __restrict__ local, int* __restrict__ roots) {
+  for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) {
+    const int g = graphs.graph_of(n), l = label[n];
+    if (local) local[n] = l - nptr[g];
+    if (l == n) atomicAdd(&roots[g], 1);
+  }
+}
+
+// inference.post_processing (inference.py:70-169) on every graph: CUT, PRUNE, CUT, SPLIT, then the SCC labels.  labels (optional,
+// device): canonical labels, graph-local in a batch; n_components (host): one count per graph; prune_changed (optional): whether
+// PRUNE removed an edge.
+static int post_pipeline(PostCtx& c, uint8_t* act, const float* prob1, int pstride, const Graphs& graphs, const std::vector<int>& ncam,
+                         const std::vector<int>& nptr, int flags, int32_t* labels, int32_t* n_components, int32_t* prune_changed) {
   int ch = 0, r = 0;
   if ((flags & MPN_POST_CUT) && c.n_active) {
     cut_kernel<<<list_grid(c.n_active), 256, 0, c.st>>>(c.n_active, c.a_eid, c.a_rev, act);
     MPN_LAUNCH_OK();
   }
-  if (flags & MPN_POST_PRUNE) MPN_TRY(prune_stage(c, act, prob1, pstride, num_cameras, &ch, &r));
+  if (flags & MPN_POST_PRUNE) MPN_TRY(prune_stage(c, act, prob1, pstride, graphs, &ch, &r));
   if ((flags & MPN_POST_CUT) && c.n_active) {
     cut_kernel<<<list_grid(c.n_active), 256, 0, c.st>>>(c.n_active, c.a_eid, c.a_rev, act);
     MPN_LAUNCH_OK();
   }
-  if (flags & MPN_POST_SPLIT) MPN_TRY(split_stage(c, act, prob1, pstride, num_cameras, &r));
+  if (flags & MPN_POST_SPLIT) MPN_TRY(split_stage(c, act, prob1, pstride, graphs, ncam, nptr));
   int nc = 0;
   MPN_TRY(scc_stage(c, act, &nc));
-  if (labels) MPN_CUDA_OK(cudaMemcpyAsync(labels, c.label, sizeof(int) * c.g.n_nodes, cudaMemcpyDeviceToDevice, c.st));
+  if (graphs.gid) {
+    const int G = (int)ncam.size();
+    MPN_CUDA_OK(cudaMemsetAsync(c.groots, 0, sizeof(int) * G, c.st));
+    graph_labels_kernel<<<list_grid(c.g.n_nodes), 256, 0, c.st>>>(c.g.n_nodes, c.label, graphs, c.g.graph_nptr, labels, c.groots);
+    MPN_LAUNCH_OK();
+    MPN_CUDA_OK(cudaMemcpyAsync(n_components, c.groots, sizeof(int) * G, cudaMemcpyDeviceToHost, c.st));
+  } else {
+    if (labels) MPN_CUDA_OK(cudaMemcpyAsync(labels, c.label, sizeof(int) * c.g.n_nodes, cudaMemcpyDeviceToDevice, c.st));
+    if (n_components) *n_components = nc;
+  }
   MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  if (n_components) *n_components = nc;
   if (prune_changed) *prune_changed = ch;
   return MPN_OK;
 }
@@ -1695,7 +1404,7 @@ int mpn_prune(const mpn_graph* g, uint8_t* act, const float* prob1, int32_t pstr
   MPN_REQUIRE(prob1 && pstride >= 1 && num_cameras >= 1, "prune: bad arguments");
   MPN_TRY(post_begin(c, g, act, ws, ws_bytes, stream));
   int ch = 0, r = 0;
-  MPN_TRY(prune_stage(c, act, prob1, pstride, num_cameras, &ch, &r));
+  MPN_TRY(prune_stage(c, act, prob1, pstride, one_graph(num_cameras), &ch, &r));
   MPN_CUDA_OK(cudaStreamSynchronize(c.st));
   if (changed) *changed = ch;
   if (rounds) *rounds = r;
@@ -1707,10 +1416,9 @@ int mpn_split(const mpn_graph* g, uint8_t* act, const float* prob1, int32_t pstr
   PostCtx c;
   MPN_REQUIRE(prob1 && pstride >= 1 && num_cameras >= 1, "split: bad arguments");
   MPN_TRY(post_begin(c, g, act, ws, ws_bytes, stream));
-  int r = 0;
-  MPN_TRY(split_stage(c, act, prob1, pstride, num_cameras, &r));
+  MPN_TRY(split_stage(c, act, prob1, pstride, one_graph(num_cameras), {num_cameras}, {0, g->n_nodes}));
   MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  if (rounds) *rounds = r;
+  if (rounds) *rounds = (int)g_split_stats[1];                 // device rounds, or the values the host order dropped
   return MPN_OK;
 }
 
@@ -1736,7 +1444,8 @@ int mpn_post_processing(const mpn_graph* g, uint8_t* act, const float* prob1, in
   PostCtx c;
   MPN_REQUIRE(prob1 && pstride >= 1 && num_cameras >= 1, "post_processing: bad arguments");
   MPN_TRY(post_begin(c, g, act, ws, ws_bytes, stream));
-  return post_processing_one_graph(c, act, prob1, pstride, num_cameras, flags, labels, n_components, prune_changed);
+  return post_pipeline(c, act, prob1, pstride, one_graph(num_cameras), {num_cameras}, {0, g->n_nodes}, flags, labels, n_components,
+                       prune_changed);
 }
 
 int mpn_post_processing_batched(const mpn_graph* g, uint8_t* act, const float* prob1, int32_t pstride, const int32_t* num_cameras_dev,
@@ -1749,28 +1458,14 @@ int mpn_post_processing_batched(const mpn_graph* g, uint8_t* act, const float* p
   MPN_CUDA_OK(cudaMemcpyAsync(ncam.data(), num_cameras_dev, sizeof(int) * G, cudaMemcpyDeviceToHost, c.st));
   MPN_CUDA_OK(cudaStreamSynchronize(c.st));
   for (int k = 0; k < G; ++k) MPN_REQUIRE(ncam[k] >= 1, "post_processing_batched: num_cameras[%d] = %d < 1", k, ncam[k]);
-  if (g->n_graphs <= 1) return post_processing_one_graph(c, act, prob1, pstride, ncam[0], flags, labels, n_components, nullptr);
-  MPN_REQUIRE(g->node_gid && g->graph_nptr, "post_processing_batched: batched graph without node_gid / graph_nptr");
-  std::vector<int> nptr;
-  MPN_TRY(copy_graph_ptr(c, nptr));
-  int ch = 0, r = 0;
-  if ((flags & MPN_POST_CUT) && c.n_active) {
-    cut_kernel<<<list_grid(c.n_active), 256, 0, c.st>>>(c.n_active, c.a_eid, c.a_rev, act);
-    MPN_LAUNCH_OK();
+  Graphs graphs = one_graph(ncam[0]);
+  std::vector<int> nptr{0, g->n_nodes};
+  if (g->n_graphs > 1) {
+    MPN_REQUIRE(g->node_gid && g->graph_nptr, "post_processing_batched: batched graph without node_gid / graph_nptr");
+    MPN_TRY(copy_graph_ptr(c, nptr));
+    graphs = Graphs{g->node_gid, num_cameras_dev, 0};
   }
-  if (flags & MPN_POST_PRUNE) MPN_TRY(prune_stage<true>(c, act, prob1, pstride, 0, &ch, &r, num_cameras_dev));
-  if ((flags & MPN_POST_CUT) && c.n_active) {
-    cut_kernel<<<list_grid(c.n_active), 256, 0, c.st>>>(c.n_active, c.a_eid, c.a_rev, act);
-    MPN_LAUNCH_OK();
-  }
-  if (flags & MPN_POST_SPLIT) MPN_TRY(split_stage_batched(c, act, prob1, pstride, num_cameras_dev, ncam, nptr));
-  MPN_TRY(scc_stage(c, act, nullptr));
-  MPN_CUDA_OK(cudaMemsetAsync(c.groots, 0, sizeof(int) * G, c.st));
-  graph_labels_kernel<<<list_grid(c.g.n_nodes), 256, 0, c.st>>>(c.g.n_nodes, c.label, c.g.node_gid, c.g.graph_nptr, labels, c.groots);
-  MPN_LAUNCH_OK();
-  MPN_CUDA_OK(cudaMemcpyAsync(n_components, c.groots, sizeof(int) * G, cudaMemcpyDeviceToHost, c.st));
-  MPN_CUDA_OK(cudaStreamSynchronize(c.st));
-  return MPN_OK;
+  return post_pipeline(c, act, prob1, pstride, graphs, ncam, nptr, flags, labels, n_components, nullptr);
 }
 
 int mpn_active_edges(const mpn_graph* g, const uint8_t* act, int32_t* src_out, int32_t* dst_out, int64_t capacity,
@@ -1854,7 +1549,7 @@ int mpn_labels_reference(const mpn_graph* g, const uint8_t* act, int64_t* labels
   MPN_TRY(post_begin(c, g, act, ws, ws_bytes, stream));
   MPN_REQUIRE((long long)c.n_active < (1ll << 30), "labels_reference: more than 2^30 active edges");
   int nc = 0;
-  MPN_TRY(labels_reference_parallel(c, act, (long long*)labels_out_host, &nc));
+  MPN_TRY(labels_reference_per_graph(c, act, {0, g->n_nodes}, (long long*)labels_out_host, &nc));
   if (n_components) *n_components = nc;
   return MPN_OK;
 }
@@ -1865,11 +1560,12 @@ int mpn_labels_reference_batched(const mpn_graph* g, const uint8_t* act, int64_t
   MPN_REQUIRE(labels_out_host && n_components_host, "labels_reference_batched: NULL output");
   MPN_TRY(post_begin(c, g, act, ws, ws_bytes, stream));
   MPN_REQUIRE((long long)c.n_active < (1ll << 30), "labels_reference_batched: more than 2^30 active edges");
-  if (g->n_graphs <= 1) return labels_reference_parallel(c, act, (long long*)labels_out_host, n_components_host);
-  MPN_REQUIRE(g->graph_nptr, "labels_reference_batched: batched graph without graph_nptr");
-  std::vector<int> nptr;
-  MPN_TRY(copy_graph_ptr(c, nptr));
-  return labels_reference_batched(c, act, nptr, (long long*)labels_out_host, n_components_host);
+  std::vector<int> nptr{0, g->n_nodes};
+  if (g->n_graphs > 1) {
+    MPN_REQUIRE(g->graph_nptr, "labels_reference_batched: batched graph without graph_nptr");
+    MPN_TRY(copy_graph_ptr(c, nptr));
+  }
+  return labels_reference_per_graph(c, act, nptr, (long long*)labels_out_host, n_components_host);
 }
 
 int mpn_labels_reference_host(const int32_t* src, const int32_t* dst, int64_t n_active, int32_t n_nodes, int64_t* labels_out,

@@ -20,6 +20,14 @@ def _as_bool(v):
     return bool(v)
 
 
+def _stage_flags(CONFIG):
+    """The CUT | PRUNE | SPLIT flag word of CONFIG, after the same in-place fix-up of its values as inference.py:75-91."""
+    for k in ('CUTTING', 'PRUNING', 'SPLITTING'):
+        CONFIG[k] = _as_bool(CONFIG[k])
+    return (_lib.POST_CUT if CONFIG['CUTTING'] else 0) | (_lib.POST_PRUNE if CONFIG['PRUNING'] else 0) | \
+        (_lib.POST_SPLIT if CONFIG['SPLITTING'] else 0)
+
+
 class _Post:
     """Shared plumbing: graph tables, uint8 activity flags and fp32 probabilities in the graph's edge order."""
 
@@ -212,10 +220,7 @@ def post_processing(num_cameras, ID_pred, predicted_active_edges, predictions, e
     round on the device, with one the components SPLITTING can touch follow the reference's own order (csrc/split_exact.cu).
     ``split_stats()`` tells which ran.
     """
-    for k in ('CUTTING', 'PRUNING', 'SPLITTING'):
-        CONFIG[k] = _as_bool(CONFIG[k])                       # same in-place fix-up as inference.py:75-91
-    flags = (_lib.POST_CUT if CONFIG['CUTTING'] else 0) | (_lib.POST_PRUNE if CONFIG['PRUNING'] else 0) | \
-            (_lib.POST_SPLIT if CONFIG['SPLITTING'] else 0)
+    flags = _stage_flags(CONFIG)
     if flags == 0:
         return ID_pred, predictions
     p = _Post(data, predictions, preds_prob)
@@ -295,10 +300,7 @@ def post_processing_batched(num_cameras, predictions, CONFIG, data, preds_prob, 
         raise ValueError("numbering must be 'reference' or 'canonical'")
     n_graphs = _graph_count(data)
     cams = _cameras_per_graph(num_cameras, n_graphs)
-    for k in ('CUTTING', 'PRUNING', 'SPLITTING'):
-        CONFIG[k] = _as_bool(CONFIG[k])                       # same in-place fix-up as inference.py:75-91
-    flags = (_lib.POST_CUT if CONFIG['CUTTING'] else 0) | (_lib.POST_PRUNE if CONFIG['PRUNING'] else 0) | \
-            (_lib.POST_SPLIT if CONFIG['SPLITTING'] else 0)
+    flags = _stage_flags(CONFIG)
     p = _Post(data, predictions, preds_prob)
     if p.g.n_graphs != n_graphs:
         raise ValueError("data.ptr describes %d graphs, its cached graph tables %d" % (n_graphs, p.g.n_graphs))

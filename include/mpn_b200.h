@@ -395,7 +395,8 @@ int mpn_post_processing(const mpn_graph* g, uint8_t* act_dev, const float* prob1
  * chosen per graph; mpn_split_last_stats then sums the counts over the graphs and out[3] is the number of graphs that took the
  * reference order.  labels_dev (optional): dev int32 [n_nodes], canonical graph-local labels (smallest node id of the SCC minus
  * the graph's first node); n_components_host: HOST int32 [n_graphs].  n_graphs <= 1: same as mpn_post_processing with
- * num_cameras_dev[0].  The workspace is mpn_post_workspace_bytes(g) (larger for n_graphs > 1).  Synchronises. */
+ * num_cameras_dev[0].  The workspace is mpn_post_workspace_bytes(g): the single-graph layout (whose SPLIT sets already hold
+ * (graph, value) keys) plus three int32 per graph.  Synchronises. */
 int mpn_post_processing_batched(const mpn_graph* g, uint8_t* act_dev, const float* prob1_dev, int32_t prob_stride,
                                 const int32_t* num_cameras_dev, int32_t flags, int32_t* labels_dev, int32_t* n_components_host,
                                 void* workspace_dev, size_t workspace_bytes, void* stream);

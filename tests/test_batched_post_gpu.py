@@ -149,6 +149,25 @@ def test_cross_graph_coupling_trap(m):
         check_per_graph(m, graphs, [TRAP_CAMERAS] * 2, flags, ID, P, nc, ptr, eptr)
 
 
+def test_single_graph_calls_take_a_batch_as_one_graph(m):
+    """post_processing, pruning and splitting handed a batch (data.ptr) process it as one disjoint-union graph: in the coupling
+    trap SPLITTING then drops graph B's edge that carries graph A's minimum, which the per-graph answer keeps."""
+    graphs = coupling_trap_case()
+    src, dst, prob, pred, n, _ = union_of(graphs)
+    union_act = pc.split_sequential(src, dst, pred, prob, TRAP_CAMERAS, n)
+    union_lab, _ = pc.scc_labels(src, dst, union_act, n)
+    data, pred_d, prob_d, _, _ = make_batch(graphs)
+    assert m.graph_for(data, data.edge_index, data.num_nodes).n_graphs == len(graphs)
+    for flags in ((False, False, True), (True, False, True)):
+        ID, P = m.post_processing(TRAP_CAMERAS, None, None, pred_d.clone(), None, cfg_of(flags), data, prob_d)
+        assert np.array_equal(P.cpu().numpy(), union_act) and np.array_equal(ID.numpy(), union_lab), flags
+    P = m.splitting(None, pred_d.clone(), prob_d, None, data, None, TRAP_CAMERAS)
+    assert np.array_equal(P.cpu().numpy(), union_act)
+    pruned, changed = pc.prune(src, dst, pred, prob, TRAP_CAMERAS, n)
+    P = m.pruning(data, pred_d.clone(), prob_d, None, TRAP_CAMERAS)
+    assert changed and np.array_equal(P.cpu().numpy(), pruned)
+
+
 def test_mixed_modes_in_one_batch(m):
     ties = [(s, d, p, a, n, C) for (_i, s, d, p, a, C, n, _ref) in _ties_cases()]
     clean = [load_golden(name) for name in ("post_n50_c4_clean", "post_n64_c4", "s02post_n300_c4")]
